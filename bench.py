@@ -1,7 +1,7 @@
 #!/usr/bin/env python
 """Benchmark of the ScrabbleGAN train step (BASELINE.json metric: train images/sec on 32 x 16*len word batches).
 
-    python bench.py [--gpus N] [--steps K] [--warmup W] [--dtype bf16|tf32|fp32] [--length L] [--batch B]
+    python bench.py [--gpus N] [--steps K] [--warmup W] [--dtype bf16|tf32|fp32] [--length L] [--batch B] [--dump-outputs DIR]
     python -m torch.distributed.run --nnodes=1 --nproc-per-node N ... bench.py --gpus N ...     (N > 1)
     python bench.py --impl reference ...      # the reference's own CPU path (torch-CPU restatement, see below)
 
@@ -18,6 +18,9 @@ One JSON line is printed by rank 0:
   roofline     the dominant kernel (tcgen05 implicit-GEMM conv) on its largest launch shape, timed live with CUDA
                events inside the timed region; `step` adds the whole-step algorithmic TFLOP/s
   cpu_baseline the reference's CPU path on this box's host cores (bounded sample), rank 0 only
+
+--dump-outputs DIR writes what the last timed step computed as DIR/*.npy (see dump_outputs); the inputs and initial
+weights are seeded, so two builds run with the same arguments can be compared file by file.
 
 The reference arm (--impl reference): TensorFlow / Keras / gin are not installable in this image (no network, not
 in the wheelhouse), so `baseline/_ref` cannot be produced; following the tier contract the arm times the torch-CPU
@@ -429,6 +432,27 @@ def dp_check(args, rt, mods, nets, world, rank):
         runtime.set_runtime(rt)
     return res
 
+
+DUMP_WEIGHT_SAMPLE = 1 << 20      # weights per network in --dump-outputs (G, D and R hold 16 M, 37 M and 5.6 M)
+
+
+def dump_outputs(out_dir, stats, nets):
+    """Writes what the last timed step computed: `train_step_stats.npy`, the 16 statistics train_step returns (in
+    data_utils.STAT_NAMES order), and for each of G, D, R the state the step leaves behind: `<net>_weights.npy`, a fixed
+    seeded sample of the trainable weights (the same indices on every run), and `<net>_bn_moving_stats.npy`, every BN
+    moving mean and variance.  All float32, about 12 MiB in all."""
+    import numpy as np
+    import torch
+    os.makedirs(out_dir, exist_ok=True)
+    np.save(os.path.join(out_dir, "train_step_stats.npy"), stats.detach().float().cpu().numpy())
+    for name, m in zip("GDR", nets):
+        w = torch.cat([v.data.reshape(-1) for v in m.store.vars if v.trainable])
+        idx = np.sort(np.random.default_rng(0).choice(w.numel(), min(DUMP_WEIGHT_SAMPLE, w.numel()), replace=False))
+        np.save(os.path.join(out_dir, name + "_weights.npy"), w[torch.from_numpy(idx).to(w.device)].cpu().numpy())
+        moving = [v.data.reshape(-1) for v in m.store.vars if not v.trainable]
+        if moving:
+            np.save(os.path.join(out_dir, name + "_bn_moving_stats.npy"), torch.cat(moving).cpu().numpy())
+
 # ----------------------------------------------------------------------------------------------------
 # our arm
 # ----------------------------------------------------------------------------------------------------
@@ -452,7 +476,12 @@ def main():
     ap.add_argument("--no-secondary", action="store_true", help="skip the secondary legs (L=10, random lengths, tf32, C2, C3, C5) and dp_check")
     ap.add_argument("--profile-range", action="store_true",
                     help="bracket the timed steps with cudaProfilerStart/Stop (for ncu --profile-from-start off)")
+    ap.add_argument("--dump-outputs", metavar="DIR", help="write what the last timed step computed to DIR/*.npy (rank 0)")
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
+    if args.dump_outputs and (args.impl != "b200" or args.workload != "step"):
+        ap.error("--dump-outputs applies to the train-step workload of --impl b200")
     args.warmup = max(args.warmup, 3)
 
     if args.impl == "reference":
@@ -577,7 +606,7 @@ def main():
         torch.cuda.profiler.start()
     e0.record()
     for i in range(args.steps):
-        step(i, dev, True)
+        last_stats = step(i, dev, True)
     e1.record()
     barrier()
     if args.profile_range:
@@ -585,6 +614,8 @@ def main():
     launches = rt.launch_count() - launches0
     clocks = sampler.stop() if rank == 0 else None
     ms_dev = e0.elapsed_time(e1)
+    if args.dump_outputs and rank == 0:       # before any later step: a replayed graph returns the same stats buffer
+        dump_outputs(args.dump_outputs, last_stats, (G, D, R))
 
     # ---- host-side enqueue cost of one step (queue empty before, no sync inside): tells whether the step is launch bound
     barrier()

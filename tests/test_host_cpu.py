@@ -106,6 +106,39 @@ def test_bench_flop_model_matches_the_survey():
     assert abs(bench.step_gflop_per_image(5, 5) - (79.714 - 9.938)) < 0.01
 
 
+def test_bench_dump_outputs_is_reproducible_and_bounded(tmp_path):
+    """bench.py --dump-outputs on host-side parameter stores: the same step output and weights give byte-identical files
+    (the weight sample is fixed), float32, every BN moving statistic in full, a large network sampled, 64 MB at most."""
+    import types
+    import numpy as np
+    import torch
+    import bench
+    params = importlib.import_module("scrabble-gan_b200.params")
+    nets = []
+    for name, n in (("G", 3 * bench.DUMP_WEIGHT_SAMPLE), ("D", 1000), ("R", 7)):
+        store = params.ParamStore(types.SimpleNamespace(device="cpu"), name, seed=len(nets))
+        store.add("conv.w", (n, 1), params.init_glorot_uniform)
+        if name != "D":
+            store.add("bn.moving_mean", (8,), params.init_zeros, trainable=False)
+            store.add("bn.moving_var", (8,), params.init_ones, trainable=False)
+        store.finalize()
+        nets.append(types.SimpleNamespace(store=store))
+    stats = torch.linspace(-1, 1, 16)
+    for d in ("a", "b"):
+        bench.dump_outputs(str(tmp_path / d), stats, nets)
+    files = sorted(p.name for p in (tmp_path / "a").iterdir())
+    assert files == ["D_weights.npy", "G_bn_moving_stats.npy", "G_weights.npy", "R_bn_moving_stats.npy", "R_weights.npy",
+                     "train_step_stats.npy"]
+    assert all((tmp_path / "a" / f).read_bytes() == (tmp_path / "b" / f).read_bytes() for f in files)
+    got = {f[:-4]: np.load(tmp_path / "a" / f) for f in files}
+    assert all(a.dtype == np.float32 for a in got.values())
+    assert np.array_equal(got["train_step_stats"], stats.numpy())
+    assert np.array_equal(got["G_bn_moving_stats"], np.r_[np.zeros(8), np.ones(8)])
+    assert got["G_weights"].shape == (bench.DUMP_WEIGHT_SAMPLE,) and np.isin(got["G_weights"], nets[0].store.w.numpy()).all()
+    assert np.array_equal(got["R_weights"], nets[2].store.by_name["conv.w"].numpy().ravel())
+    assert sum((tmp_path / "a" / f).stat().st_size for f in files) <= 64 << 20
+
+
 def test_synthetic_loaders_keep_the_reference_interfaces():
     du = importlib.import_module("scrabble-gan_b200.bigacgan.data_utils")
     char_vec = "abcdefghijklmnopqrstuvwxyzABCDEFGHIJKLMNOPQRSTUVWXYZ"
