@@ -288,6 +288,22 @@ int sg_ctc(sg_ctx* ctx, const float* logits, const int* labels, int b, int t, in
 int sg_ctc_ragged(sg_ctx* ctx, const float* logits, const int* labels, int b, int t_max, int c, int l_max,
                   const int* input_len, const int* label_len, float* loss, float* grad_logits);
 
+/* ---- reading words back with the recogniser (same conventions as sg_ctc: blank = c-1, [b, t_max, c] layout) -------------
+ * sg_softmax_rows: y = softmax(x) over rows of c fp32 values -- the reference's Dense(activation='softmax') output
+ * (net_architecture.py:55), i.e. what a Keras user feeds to K.ctc_decode. */
+int sg_softmax_rows(sg_ctx* ctx, const float* x, long long rows, int c, float* y);
+/* Replaces K.ctc_decode(greedy=True) / tf.nn.ctc_greedy_decoder(merge_repeated=True): per frame t < input_len[b] (NULL: all
+ * t_max frames; clamped to [0, t_max]) the most probable class (ties: lowest index), repeats merged, blanks dropped.
+ * decoded [b, t_max] int32 padded with -1, decoded_len [b], neg_sum_log[b] = -sum_t log(max_c probs[b,t,c] + 1e-7) (Keras'
+ * log_prob; [TF-SEMANTICS]).  Deterministic.  t_max <= 25600. */
+int sg_ctc_greedy_decode(sg_ctx* ctx, const float* probs, int b, int t_max, int c, const int* input_len,
+                         int* decoded, int* decoded_len, float* neg_sum_log);
+/* Replaces tf.edit_distance(normalize=False): exact Levenshtein distance dist[b] between hyp [b, hyp_stride] and
+ * ref [b, ref_stride] (int32, ref_stride <= 64).  A NULL length array means the run of leading non-negative entries
+ * (sg_label_lengths).  totals (NULL or long long[4], device) is ADDED to: {sum dist, sum ref length, exact matches, samples}. */
+int sg_edit_distance(sg_ctx* ctx, const int* hyp, const int* hyp_len, int hyp_stride, const int* ref, const int* ref_len,
+                     int ref_stride, int b, int* dist, long long* totals);
+
 /* ---- GAN losses + gradient balancing (K16, K17) -- net_loss.py:4-54; data_utils.py:418-442,476-490 --
  * sums is double[SG_LOSS_NSUMS]; all-reduce it across replicas between the two calls. */
 #define SG_LOSS_NSUMS 16

@@ -129,6 +129,9 @@ _PROTOS = {
     "sg_nonlocal_proj_bwd": (_I, [_P, _P, _P, _P, _P, _L, _P, _P, _P, _P, _P, _P, _P]),
     "sg_ctc": (_I, [_P, _P, _P, _I, _I, _I, _I, _P, _P]),
     "sg_ctc_ragged": (_I, [_P, _P, _P, _I, _I, _I, _I, _P, _P, _P, _P]),
+    "sg_softmax_rows": (_I, [_P, _P, _L, _I, _P]),
+    "sg_ctc_greedy_decode": (_I, [_P, _P, _I, _I, _I, _P, _P, _P, _P]),
+    "sg_edit_distance": (_I, [_P, _P, _P, _I, _P, _P, _I, _I, _P, _P]),
     "sg_loss_sums": (_I, [_P, _I, _I, _P, _P, _P, _P, _P, _P, _P, _I, _P]),
     "sg_loss_finish": (_I, [_P, _I, _I, _I, _F, _P, _P, _P, _P, _P, _P, _I, _P, _P, _P, _P, _P, _P, _P, _P, _P, _P]),
     "sg_loss_terms": (_I, [_P, _I, _P, _P, _P, _P, _P, _I, _P]),

@@ -339,14 +339,14 @@ class Recognizer(_Model):
         self.bn_training = False
         self.store.finalize(initialise)
 
-    def _bn_forward(self, rt, x, bn: BatchNormState, out_dt):
-        if self.bn_training:
+    def _bn_forward(self, rt, x, bn: BatchNormState, out_dt, training: bool):
+        if training:
             mean, rstd, count = batch_stats(rt, x, bn)
         else:
             mean, rstd = ops.bn_infer_prepare(rt, bn.moving_mean.data, bn.moving_var.data)
             count = 1
         y = ops.bn_apply(rt, x, mean, rstd, bn.gamma.data, bn.beta.data, False, False, out_dt)
-        return y, (mean, rstd, count, self.bn_training)
+        return y, (mean, rstd, count, training)
 
     def _bn_backward(self, rt, bn: BatchNormState, bc, dy, x, wgrad, out_dt, rows=None):
         """dy = grad of the BN output (fp32); x = BN input = relu(conv) (fp32).  Returns grad w.r.t. the conv
@@ -368,6 +368,12 @@ class Recognizer(_Model):
         (n,) int32: a RAGGED batch exactly as the reference model takes one (its inputs are [images, labels, input_length,
         label_length], net_architecture.py:66-75): words of different lengths padded to a common width, every sample's CTC
         recursion over its own 4*len-1 frames and len labels."""
+        logits, trunk = self._logits(rt, x, self.bn_training)
+        loss, glogits = ops.ctc(rt, logits, labels, want_grad, input_length, label_length)
+        return loss, trunk + (glogits,)
+
+    def _logits(self, rt, x, bn_training: bool):
+        """CRNN trunk + Dense pre-activations (n, W/4-1, classes) fp32, and the activations backward needs."""
         T = rt.op_dt
         cv = self.convs
         a1 = cv[0].forward(rt, x, relu=True, out_dt=T)
@@ -378,16 +384,24 @@ class Recognizer(_Model):
         a4 = cv[3].forward(rt, a3, relu=True, out_dt=T)
         p4 = ops.maxpool_fwd(rt, a4, 2, 1)
         a5 = cv[4].forward(rt, p4, relu=True, out_dt=SG_F32)
-        b5, bc5 = self._bn_forward(rt, a5, self.bn5, T)
+        b5, bc5 = self._bn_forward(rt, a5, self.bn5, T, bn_training)
         a6 = cv[5].forward(rt, b5, relu=True, out_dt=SG_F32)
-        b6, bc6 = self._bn_forward(rt, a6, self.bn6, T)
+        b6, bc6 = self._bn_forward(rt, a6, self.bn6, T, bn_training)
         p6 = ops.maxpool_fwd(rt, b6, 2, 1)
         a7 = cv[6].forward(rt, p6, relu=True, out_dt=SG_F32)           # (n, 1, W/4-1, 512)
         n, _, t, c = a7.shape
         logits = self.dense.forward(rt, a7, n * t).view(n, t, self.output_classes)
-        loss, glogits = ops.ctc(rt, logits, labels, want_grad, input_length, label_length)
-        cache = (x, a1, p1, a2, p2, a3, a4, p4, a5, b5, bc5, a6, b6, bc6, p6, a7, glogits)
-        return loss, cache
+        return logits, (x, a1, p1, a2, p2, a3, a4, p4, a5, b5, bc5, a6, b6, bc6, p6, a7)
+
+    def frame_probs(self, images) -> torch.Tensor:
+        """Per-frame class probabilities (B, W/4-1, classes) fp32 on the device: the output of the reference model's Dense
+        softmax layer (net_architecture.py:55), the input of K.ctc_decode.  BatchNorm always uses the moving statistics
+        (inference); `bn_training` and the moving statistics are neither read nor changed.  images: (B, 32, W[, 1]) host
+        buffer, device tensor or DLPack producer."""
+        x = _nhwc(to_device_f32(self.rt, images))
+        self.sn_forward(self.rt, update_u=False)
+        logits, _ = self._logits(self.rt, x, bn_training=False)
+        return ops.softmax_rows(self.rt, logits)
 
     @staticmethod
     def slice_cache(cache, a: int, b: int):

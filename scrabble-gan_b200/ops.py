@@ -601,6 +601,36 @@ def ctc(rt, logits, labels, want_grad=True, input_length=None, label_length=None
     return loss, grad
 
 
+def softmax_rows(rt, x):
+    """Softmax over the last dimension of an fp32 tensor (R's Dense activation)."""
+    c = x.shape[-1]
+    y = rt.empty(x.shape, SG_F32)
+    call.sg_softmax_rows(rt.ctx, _p(x), x.numel() // c, c, _p(y))
+    return y
+
+
+def ctc_greedy_decode(rt, probs, input_length=None):
+    """K.ctc_decode(greedy=True) on probs (B, T, C): decoded (B, T) int32 padded with -1, decoded_len (B,) int32,
+    neg_sum_log (B,) fp32.  input_length: (B,) int32 device tensor or None (all T frames)."""
+    b, t, c = probs.shape
+    decoded = torch.empty((b, t), device=rt.device, dtype=torch.int32)
+    dlen = torch.empty((b,), device=rt.device, dtype=torch.int32)
+    score = rt.empty((b,), SG_F32)
+    call.sg_ctc_greedy_decode(rt.ctx, _p(probs), b, t, c, _p(input_length), _p(decoded), _p(dlen), _p(score))
+    return decoded, dlen, score
+
+
+def edit_distance(rt, hyp, ref, hyp_length=None, ref_length=None, totals=None):
+    """Levenshtein distance (B,) int32 between the rows of hyp (B, Lh) and ref (B, Lr <= 64); without a length tensor a row
+    ends at its first negative entry.  totals: int64 (4,) device tensor that is ADDED to (sum dist, sum ref length, exact
+    matches, samples)."""
+    b = hyp.shape[0]
+    dist = torch.empty((b,), device=rt.device, dtype=torch.int32)
+    call.sg_edit_distance(rt.ctx, _p(hyp), _p(hyp_length), hyp.shape[1], _p(ref), _p(ref_length), ref.shape[1], b, _p(dist),
+                          _p(totals))
+    return dist
+
+
 def random_(rt, out, normal: bool = True, seed: Optional[int] = None):
     """Fill `out` (fp32) with N(0,1) (or U[-1,1)) numbers from the runtime's Philox stream; the stream position lives on the
     device (rt.rng_state), so the launch can be captured in a CUDA graph and still draw fresh numbers on every replay."""
