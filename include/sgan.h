@@ -47,12 +47,8 @@ long long sg_ctx_launch_count(sg_ctx* ctx);      /* kernels launched through thi
 int sg_ctx_set_speed_mode(sg_ctx* ctx, int on);
 /* tensor-core convolutions: when the last wave of output tiles of a launch would leave most SMs idle, the k-range of each of its
  * tiles is split over several CTAs, which exchange fp32 partial accumulators through the context's workspace and add them in a
- * fixed order (results stay bit-reproducible run to run).  On by default (SGAN_NO_SPLIT_TAIL=1 at context creation disables). */
+ * fixed order (results stay bit-reproducible run to run).  On by default. */
 int sg_ctx_set_conv_split_tail(sg_ctx* ctx, int on);
-/* size the grids of this context's kernels for at most `sms` SMs (persistent kernels launch min(units, sms) CTAs): a context
- * whose stream runs BESIDE another one (the side stream's filter gradients next to the main stream's input-gradient chain)
- * leaves the other SMs to it.  Clamped to the device's SM count, which is also the default. */
-int sg_ctx_set_sm_limit(sg_ctx* ctx, int sms);
 int sg_sizeof_conv_desc(void);                    /* sizeof(sg_conv_desc): layout guard for FFI mirrors */
 
 /* ---- convolution family (K1-K8) ------------------------------------------------------------------

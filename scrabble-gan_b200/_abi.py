@@ -54,7 +54,6 @@ _PROTOS = {
     "sg_zero": (_I, [_P, _P, _Z]),
     "sg_ctx_set_speed_mode": (_I, [_P, _I]),
     "sg_ctx_set_conv_split_tail": (_I, [_P, _I]),
-    "sg_ctx_set_sm_limit": (_I, [_P, _I]),
     "sg_sizeof_conv_desc": (_I, []),
     "sg_crc32c": (C.c_uint, [_P, _Z, C.c_uint]),
     "sg_random": (_I, [_P, _P, _L, C.c_ulonglong, C.c_ulonglong, _P, _I]),

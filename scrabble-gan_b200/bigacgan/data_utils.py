@@ -92,7 +92,7 @@ class _GraphedStep:
 
 def _graph_key(rt, generator, discriminator, recognizer, opts, b, l_r, l_f, kind, balance, update_g, balance_mode="reference"):
     return (id(generator), id(discriminator), id(recognizer), tuple(id(o) for o in opts), b, l_r, l_f, rt.mode, kind, bool(balance),
-            bool(update_g), bool(recognizer.trainable), os.environ.get("SGAN_NO_FUSED_BATCH", "0"), balance_mode,
+            bool(update_g), bool(recognizer.trainable), balance_mode,
             tuple(bool(getattr(m, "apply_sn", False)) for m in (generator, discriminator)))
 
 
@@ -191,7 +191,7 @@ def _capture(rt, gs, args, b, l_r, l_f, latent_dim):
             # forward pass since the last weight change (e.g. inference between two steps) would have left fresh entries,
             # the capture would skip the packs and every replay would then read filters from before its own Adam steps
             st.version += 1
-            if rt.mode == "bf16" and rt.use_direct:
+            if rt.mode == "bf16":
                 st.mirror(rt)                                   # fresh mirrors: no cast gets captured
         # optimizer state must exist BEFORE the capture: created inside it, the (m, v) slots would live in the graph's
         # private pool and their zero-fill would become a graph node (re-zeroing them on every replay)
@@ -232,7 +232,7 @@ def _replay(rt, gs, args, images, labels, fake_labels, noise):
     stores = [discriminator.store, recognizer.store, generator.store]
     for i, st in enumerate(stores):
         if st.version != gs.versions[i]:                        # weights changed outside the graph (load / assign)
-            if rt.mode == "bf16" and rt.use_direct:
+            if rt.mode == "bf16":
                 st.mirror(rt)
             gs.versions[i] = st.version
     x_s, yr_s, yf_s, z_s = gs.static
@@ -277,7 +277,7 @@ def _step_device(rt, args, x_real, y_real, y_fake, g_in, style_imgs):
     # [fake ; real] batch of 2B images (they have no cross-sample coupling: no batch-stat BN), which doubles the
     # GEMM M of every layer; G writes its tanh output straight into the first half, the real images are copied into
     # the second half.
-    fused = (l_r == l_f) and not recognizer.bn_training and os.environ.get("SGAN_NO_FUSED_BATCH", "0") != "1"
+    fused = (l_r == l_f) and not recognizer.bn_training
     if fused:
         xcat = rt.empty((2 * b, 32, 16 * l_r, 1))
         xcat[b:].copy_(x_real, non_blocking=True)
@@ -291,7 +291,7 @@ def _step_device(rt, args, x_real, y_real, y_fake, g_in, style_imgs):
     for m in nets:
         m.store.zero_grad()
         m.sn_forward(rt, update_u=True)             # apply_sn: refresh W / sigma(W) (one power-iteration step, persistent u)
-        if rt.use_tc and rt.batch_packs:
+        if rt.use_tc:
             m.prepack(rt)                           # all forward filters of the network that the last Adam step made stale: one launch
 
     # ---- forward passes (data_utils.py:398-415) -------------------------------------------------------------------
@@ -339,37 +339,19 @@ def _step_device(rt, args, x_real, y_real, y_fake, g_in, style_imgs):
     # Data parallel: each network's flat gradient bucket is SUM-all-reduced (not averaged: SURVEY Q7) as soon as its
     # filter gradients are complete, on NCCL's stream, overlapping with the backward passes that follow.
     pending = []
-    dimg_r_merged = dimg_d_merged = None
-    d_side = None
     discriminator.trainable = True
     recognizer.trainable = True
     br = rt.branch()                     # R's backward (side stream) next to D's two backward passes (main stream)
     if fused:
         with br:
-            if update_g and rt.merge_r_backward:
+            if update_g:
                 # ONE backward pass of R over the fused batch: filter gradients from the real half (R-loss, weight 1), image
                 # gradient of the fake half with the G-loss per-sample weights (different samples: nothing mixes)
-                recognizer.trainable = True
-                dimg_r_all = recognizer.backward(rt, rcc, up_r_fake_g, wgrad=True, want_dx=True, wgrad_rows=(b, 2 * b), up_rows=(0, b))
-                dimg_r_merged = dimg_r_all[:b]
+                dimg_r = recognizer.backward(rt, rcc, up_r_fake_g, wgrad=True, want_dx=True, wgrad_rows=(b, 2 * b), up_rows=(0, b))[:b]
             else:
                 recognizer.backward(rt, recognizer.slice_cache(rcc, b, 2 * b), None, wgrad=True, want_dx=False)
-                rfc = recognizer.slice_cache(rcc, 0, b)
             pending.append((id(recognizer), rt.allreduce_async_(recognizer.store.g, store=recognizer.store)))
-        if update_g and rt.merge_d_backward:
-            # ONE backward pass of D over the fused batch for both losses (Discriminator.backward_merged); its filter gradients
-            # run on the side stream next to the input-gradient chain and -- on one replica without spectral norm, where
-            # nothing reads D's bucket before D's optimizer launch (side stream too) -- next to G's backward pass as well
-            d_side = [] if (rt.concurrent_branches and rt.side_d_wgrads) else None
-            dimg_d_merged = discriminator.backward_merged(rt, dcc, ups[0:2].view(-1), b, up_d_fake_g, 1.0, side=d_side)
-            if d_side is not None and (rt.world_size > 1 or discriminator.store.sn is not None):
-                rt.branch().join()
-                d_side = None
-        else:
-            discriminator.backward(rt, dcc, ups[0:2].view(-1), wgrad=True, want_dx=False)
-        discriminator.sn_backward(rt)
-        pending.append((id(discriminator), rt.allreduce_async_(discriminator.store.g, store=discriminator.store)))
-        dfc = discriminator.slice_cache(dcc, 0, b)
+        d_cache, d_up = dcc, ups[0:2].view(-1)
     else:
         with br:
             recognizer.backward(rt, rrc, None, wgrad=True, want_dx=False)
@@ -377,18 +359,22 @@ def _step_device(rt, args, x_real, y_real, y_fake, g_in, style_imgs):
             if update_g:
                 # R's image gradient of the fake batch (frozen R, G loss) right away: D's filter gradients queue up behind it
                 # on the side stream, and G's backward pass must not wait for those
-                dimg_r_merged = recognizer.backward(rt, rfc, up_r_fake_g, wgrad=False, want_dx=True)
+                dimg_r = recognizer.backward(rt, rfc, up_r_fake_g, wgrad=False, want_dx=True)
         discriminator.backward(rt, drc, up_d_real, wgrad=True, want_dx=False)
-        if update_g and rt.merge_d_backward:
-            d_side = [] if (rt.concurrent_branches and rt.side_d_wgrads) else None
-            dimg_d_merged = discriminator.backward_merged(rt, dfc, up_d_fake_d, b, up_d_fake_g, 1.0, side=d_side)   # the whole batch is "fake"
-            if d_side is not None and (rt.world_size > 1 or discriminator.store.sn is not None):
-                rt.branch().join()
-                d_side = None
-        else:
-            discriminator.backward(rt, dfc, up_d_fake_d, wgrad=True, want_dx=False)
-        discriminator.sn_backward(rt)
-        pending.append((id(discriminator), rt.allreduce_async_(discriminator.store.g, store=discriminator.store)))
+        d_cache, d_up = dfc, up_d_fake_d             # unfused: the merged pass below sees only the fake batch
+    if update_g:
+        # ONE backward pass of D for both losses (Discriminator.backward_merged); its filter gradients run on the side stream
+        # next to the input-gradient chain and -- on one replica without spectral norm, where nothing reads D's bucket before
+        # D's optimizer launch (side stream too) -- next to G's backward pass as well
+        d_side = []
+        dimg = discriminator.backward_merged(rt, d_cache, d_up, b, up_d_fake_g, 1.0, side=d_side)
+        if rt.world_size > 1 or discriminator.store.sn is not None:
+            rt.branch().join()
+            d_side = None
+    else:
+        discriminator.backward(rt, d_cache, d_up, wgrad=True, want_dx=False)
+    discriminator.sn_backward(rt)
+    pending.append((id(discriminator), rt.allreduce_async_(discriminator.store.g, store=discriminator.store)))
     if use_w:
         style_promoter.trainable = True
         style_promoter.backward(rt, src_c, up_s_real, wgrad=True, want_dx=False)
@@ -405,15 +391,6 @@ def _step_device(rt, args, x_real, y_real, y_fake, g_in, style_imgs):
     if update_g:
         recognizer.trainable = False
         discriminator.trainable = False
-        if dimg_r_merged is None:
-            with br:
-                dimg_r = recognizer.backward(rt, rfc, up_r_fake_g, wgrad=False, want_dx=True)
-        else:
-            dimg_r = dimg_r_merged
-        if dimg_d_merged is not None:
-            dimg = dimg_d_merged
-        else:
-            dimg = discriminator.backward(rt, dfc, up_d_fake_g, wgrad=False, want_dx=True)
         br.join()
         if use_w:
             style_promoter.trainable = False

@@ -229,13 +229,6 @@ class _DownTrunk:
         feats = ops.gap_relu_fwd(rt, net)                     # relu -> GlobalAveragePooling2D
         return feats, (caches, net)
 
-    def slice_cache(self, cache, a: int, b: int):
-        caches, net = cache
-        out = []
-        for i, (c, ca) in enumerate(caches):
-            out.append((ResNetBlockDown.slice_cache(c, a, b), NonLocalBlock.slice_cache(ca, a, b) if ca is not None else None))
-        return (out, net[a:b])
-
     def backward(self, rt: Runtime, cache, dfeats, wgrad: bool, want_dx: bool, fake=None, side=None):
         """fake = (b, up, mult): merged backward (see ResNetBlockDown.backward); returns the image gradient of rows [0, b).
         side: list -- with `fake`, the blocks' filter gradients run on the side stream (their operands are collected here)."""
@@ -276,10 +269,6 @@ class Discriminator(_Model):
         logits = self.dense.forward(rt, feats, x.shape[0])
         return logits, (feats, c)
 
-    def slice_cache(self, cache, a: int, b: int):
-        feats, c = cache
-        return (feats[a:b], self.trunk.slice_cache(c, a, b))
-
     def backward(self, rt, cache, up, wgrad: bool = True, want_dx: bool = False):
         """up [n] = d(sum target)/d(logit).  Accumulates parameter gradients when wgrad; returns d/d(image) or None."""
         feats, c = cache
@@ -287,7 +276,7 @@ class Discriminator(_Model):
         dfeats = self.dense.backward(rt, feats, up, n, want_dx=True, wgrad=wgrad)
         return self.trunk.backward(rt, c, dfeats, wgrad, want_dx)
 
-    def backward_merged(self, rt, cache, up_all, b: int, up_fake_g, mult: float, side=None):
+    def backward_merged(self, rt, cache, up_all, b: int, up_fake_g, mult: float, side):
         """ONE backward pass over a [fake ; real] batch that serves both the D loss and the G loss (data_utils.py:449-468
         differentiates them separately; frozen weights make the second tape the same linear map).  Back-propagation is linear
         in a sample's upstream weight, so rows [0, b) -- the fake images -- travel with the constant weight 1 / mult; the
@@ -525,24 +514,18 @@ class Generator(_Model):
         zs = self.latent_dim
         net, ec = self.embed.forward(rt, z, zs, y)
         # all 12 CBN gamma / beta Dense layers (resnet_ops.py:18-26) in ONE launch: [n, sum of 2 C] with per-layer column blocks
-        gb = None
-        if rt.group_cbn_dense:
-            segs = self._cbn_segments()
-            gb_all = ops.cbn_dense_fwd(rt, z, zs, z.shape[0], [s[:3] for s in segs], self._cbn_wbase())
-            gb, col = [], 0
-            for c_, _, _, _ in segs:
-                gb.append(gb_all[:, col:])
-                col += c_
-            gb_stride = gb_all.shape[1]
+        segs = self._cbn_segments()
+        gb_all = ops.cbn_dense_fwd(rt, z, zs, z.shape[0], [s[:3] for s in segs], self._cbn_wbase())
+        gb, col = [], 0
+        for c_, _, _, _ in segs:
+            gb.append(gb_all[:, col:])
+            col += c_
+        gb_stride = gb_all.shape[1]
         caches = []
         for i, blk in enumerate(self.blocks):
-            zi = z[:, self.zchunk * (i + 1):]
-            kw = {}
-            if gb is not None:
-                kw = {"gb1": (gb[4 * i], gb[4 * i + 1], gb_stride), "gb2": (gb[4 * i + 2], gb[4 * i + 3], gb_stride)}
-            if lens is not None:
-                kw["ragged"] = (lens, net.shape[2] // y.shape[1])
-            net, c = blk.forward(rt, net, zi, zs, training, **kw)
+            ragged = (lens, net.shape[2] // y.shape[1]) if lens is not None else None
+            net, c = blk.forward(rt, net, training, (gb[4 * i], gb[4 * i + 1], gb_stride), (gb[4 * i + 2], gb[4 * i + 3], gb_stride),
+                                 ragged)
             ca = None
             if i in self.attn:
                 kv_cols = None
@@ -572,11 +555,8 @@ class Generator(_Model):
         n = net.shape[0]
         dpre = ops.tanh_bwd(rt, dimg, img)
         # filter gradients are off the input-gradient chain: on the side stream, next to the chain (ResNetBlockUp.backward)
-        side = [dpre] if (rt.concurrent_branches and rt.side_wgrads) else None
-        if side is not None:
-            with rt.branch():
-                self.out.wgrad(rt, act, dpre)
-        else:
+        side = [dpre]
+        with rt.branch():
             self.out.wgrad(rt, act, dpre)
         dact = self.out.dgrad(rt, dpre, (net.shape[1], net.shape[2]))
         s1, s2 = ops.bn_bwd_reduce(rt, dact, act, net, mean, rstd)
@@ -588,31 +568,27 @@ class Generator(_Model):
             rt.allreduce_small_(ab)
         d = ops.bn_bwd_apply(rt, dact, act, net, mean, rstd, self.bn.gamma.data, False, ab, count, training, False, SG_F32)
         dz = rt.zeros((n, self.latent_dim)) if want_dz else None
-        defer = [] if rt.group_cbn_dense else None
+        defer = []
         for i in reversed(range(self.num_blocks)):
             c, ca = caches[i]
             if ca is not None:
                 d = self.attn[i].backward(rt, ca, d, True)
-            d = self.blocks[i].backward(rt, c, d, dz[:, self.zchunk * (i + 1):] if want_dz else None, self.latent_dim, defer=defer,
-                                        side=side)
-        if defer:
-            # the 12 Dense filter gradients dW = z_block^T @ (d gamma | d beta) in ONE launch
-            by_layer = {id(cbn): (s1, s2) for cbn, s1, s2 in defer}
-            segs, ups = [], []
-            for (c_, zoff, woff, (cbn, which)) in self._cbn_segments(grad=True):
-                s1, s2 = by_layer[id(cbn)]
-                segs.append((c_, zoff, woff))
-                ups.append(s2 if which == "gamma" else s1)
-            ops.cbn_dense_wgrad(rt, z, self.latent_dim, n, segs, ups, self.store.g)
+            d = self.blocks[i].backward(rt, c, d, defer, side, dz[:, self.zchunk * (i + 1):] if want_dz else None, self.latent_dim)
+        # the 12 Dense filter gradients dW = z_block^T @ (d gamma | d beta) in ONE launch
+        by_layer = {id(cbn): (s1, s2) for cbn, s1, s2 in defer}
+        segs, ups = [], []
+        for (c_, zoff, woff, (cbn, which)) in self._cbn_segments(grad=True):
+            s1, s2 = by_layer[id(cbn)]
+            segs.append((c_, zoff, woff))
+            ups.append(s2 if which == "gamma" else s1)
+        ops.cbn_dense_wgrad(rt, z, self.latent_dim, n, segs, ups, self.store.g)
         self.embed.backward(rt, ec, d, dz, self.latent_dim)
         if want_dz:
             feats, tc = sc
             dfeats = self.style_dense.backward(rt, feats, dz, n, want_dx=True, wgrad=True)
             self.style.backward(rt, tc, dfeats, True, False)
-        if side is not None:
-            br = rt.branch()
-            br.join()                  # all filter gradients are in the bucket; only now may their operands be released
-            side.clear()
+        rt.branch().join()             # all filter gradients are in the bucket; only now may their operands be released
+        side.clear()
 
     def _cbn_segments(self, grad: bool = False):
         """(C, column offset of the block's z slice, offset of the Dense kernel in the flat store, (layer, which)) for the

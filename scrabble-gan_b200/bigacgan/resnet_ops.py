@@ -24,30 +24,24 @@ class ConditionalBatchNorm:
         self.beta = DenseLayer(store, name + ".beta", zdim, c)
         self.bn = BatchNormState(store, name, c, affine=False)
 
-    def forward(self, rt: Runtime, x, z, z_stride: int, training: bool, relu: bool, out_dt: int, gb=None):
+    def forward(self, rt: Runtime, x, gb, training: bool, relu: bool, out_dt: int):
         """gb = (gamma, beta, row stride): views into the grouped Dense output of the whole generator (one launch for all
-        CBN layers, ops.cbn_dense_fwd); without it the two Dense layers are launched here."""
-        n = x.shape[0]
+        CBN layers, ops.cbn_dense_fwd)."""
         if training:
             mean, rstd, count = batch_stats(rt, x, self.bn)
         else:
             mean, rstd = ops.bn_infer_prepare(rt, self.bn.moving_mean.data, self.bn.moving_var.data)
             count = 1
-        if gb is None:
-            g = self.gamma.forward(rt, z, n, ldx=z_stride)
-            b = self.beta.forward(rt, z, n, ldx=z_stride)
-            gs = None
-        else:
-            g, b, gs = gb
+        g, b, gs = gb
         y = ops.bn_apply(rt, x, mean, rstd, g, b, True, relu, out_dt, gb_stride=gs)
-        return y, (x, y if relu else None, z, z_stride, mean, rstd, g, count, training, gs)
+        return y, (x, y if relu else None, mean, rstd, g, count, training, gs)
 
-    def backward(self, rt: Runtime, cache, dy, out_dt: int = SG_F32, out=None, accumulate: bool = False, dz_out=None,
-                 dz_ld: int = 0, defer=None):
-        """dy: gradient w.r.t. the (post-ReLU) output.  Accumulates the Dense weight gradients -- or, with `defer` (a list),
-        only records (layer, d beta, d gamma) so that the caller computes all of them in one grouped launch -- and, when
-        dz_out is given, adds d/dz into dz_out (row stride dz_ld).  Returns dx."""
-        x, act, z, z_stride, mean, rstd, g, count, training, gs = cache
+    def backward(self, rt: Runtime, cache, dy, defer, out_dt: int = SG_F32, out=None, accumulate: bool = False, dz_out=None,
+                 dz_ld: int = 0):
+        """dy: gradient w.r.t. the (post-ReLU) output.  Records (layer, d beta, d gamma) in the list `defer`, so that the caller
+        computes the Dense weight gradients of all CBN layers in one grouped launch, and, when dz_out is given, adds d/dz into
+        dz_out (row stride dz_ld).  Returns dx."""
+        x, act, mean, rstd, g, count, training, gs = cache
         n = x.shape[0]
         s1, s2 = ops.bn_bwd_reduce(rt, dy, act, x, mean, rstd)          # s1 = d beta [n,c], s2 = d gamma [n,c]
         ab = None
@@ -56,11 +50,7 @@ class ConditionalBatchNorm:
             rt.allreduce_small_(ab)                                           # sync-BN backward statistics
         dx = ops.bn_bwd_apply(rt, dy, act, x, mean, rstd, g, True, ab, count, training, False, out_dt, out, int(accumulate),
                               gb_stride=gs)
-        if defer is not None:
-            defer.append((self, s1, s2))
-        else:
-            self.gamma.backward(rt, z, s2, n, ldx=z_stride, want_dx=False)
-            self.beta.backward(rt, z, s1, n, ldx=z_stride, want_dx=False)
+        defer.append((self, s1, s2))
         if dz_out is not None:
             ops.gemm(rt, s2, self.gamma.w.eff, n, self.gamma.cin, self.c, trans_b=True, out=dz_out, ldc=dz_ld, accumulate=1)
             ops.gemm(rt, s1, self.beta.w.eff, n, self.beta.cin, self.c, trans_b=True, out=dz_out, ldc=dz_ld, accumulate=1)
@@ -81,14 +71,15 @@ class ResNetBlockUp:
         self.conv = ConvLayer(store, name + ".conv", 3, 3, co, co)
         self.short = ConvTransposeLayer(store, name + ".short", 1, ci, co, self.stride)
 
-    def forward(self, rt: Runtime, x, z, z_stride: int, training: bool, gb1=None, gb2=None, ragged=None):
-        """ragged = (lens, columns per character of x): the inputs of both 3x3 convolutions are zeroed right of every word's
-        own width, so a short word of a padded batch sees the zero padding it would see alone (inference only)."""
-        a1, c1 = self.cbn1.forward(rt, x, z, z_stride, training, True, rt.op_dt, gb=gb1)
+    def forward(self, rt: Runtime, x, training: bool, gb1, gb2, ragged=None):
+        """gb1, gb2: (gamma, beta, row stride) of cbn1 / cbn2 (ConditionalBatchNorm.forward).  ragged = (lens, columns per
+        character of x): the inputs of both 3x3 convolutions are zeroed right of every word's own width, so a short word of a
+        padded batch sees the zero padding it would see alone (inference only)."""
+        a1, c1 = self.cbn1.forward(rt, x, gb1, training, True, rt.op_dt)
         if ragged is not None:
             ops.mask_width_(rt, a1, ragged[0], ragged[1])
         u = self.up.forward(rt, a1)
-        a2, c2 = self.cbn2.forward(rt, u, z, z_stride, training, True, rt.op_dt, gb=gb2)
+        a2, c2 = self.cbn2.forward(rt, u, gb2, training, True, rt.op_dt)
         if ragged is not None:
             ops.mask_width_(rt, a2, ragged[0], ragged[1] * self.stride[1])
         bsum = ops.axpby(rt, 1.0, self.conv.b.data, 1.0, self.short.b.data)      # conv bias + shortcut bias (everywhere)
@@ -97,28 +88,26 @@ class ResNetBlockUp:
         self.short.forward(rt, xs, out=h, accumulate=True, bias=None)
         return h, (c1, c2, a1, a2, xs, x.shape)
 
-    def backward(self, rt: Runtime, cache, dh, dz_out=None, dz_ld: int = 0, defer=None, side=None):
-        """side: a list -- the three filter gradients of the block are not on the input-gradient chain, so they are enqueued on
-        the runtime's side stream (rt.branch) and run next to the chain's (small, latency-bound) kernels; the list collects
-        the temporaries they read, which the caller keeps alive until it has joined the side stream."""
+    def backward(self, rt: Runtime, cache, dh, defer, side, dz_out=None, dz_ld: int = 0):
+        """defer: list of the CBN layers' Dense gradient operands (ConditionalBatchNorm.backward).  side: a list -- the three
+        filter gradients of the block are not on the input-gradient chain, so they are enqueued on the runtime's side stream
+        (rt.branch) and run next to the chain's (small, latency-bound) kernels; the list collects the temporaries they read,
+        which the caller keeps alive until it has joined the side stream."""
         c1, c2, a1, a2, xs, xshape = cache
         n, hh, ww, _ = xshape
         dh_op = ops.cast(rt, dh, rt.op_dt)
 
         def off_chain(fn, *keep):
-            if side is None:
-                fn()
-                return
             side.extend(keep)
             with rt.branch():
                 fn()
         # main branch, back to front
         off_chain(lambda: self.conv.wgrad(rt, a2, dh_op, also_bias=self.short.b.grad), dh_op)   # the shortcut bias sees the same upstream gradient
         da2 = self.conv.dgrad(rt, dh_op, (hh * self.stride[0], ww * self.stride[1]))
-        du = self.cbn2.backward(rt, c2, da2, out_dt=rt.op_dt, dz_out=dz_out, dz_ld=dz_ld, defer=defer)
+        du = self.cbn2.backward(rt, c2, da2, defer, out_dt=rt.op_dt, dz_out=dz_out, dz_ld=dz_ld)
         off_chain(lambda: self.up.wgrad(rt, a1, du), du)
         da1 = self.up.dgrad(rt, du)
-        dx = self.cbn1.backward(rt, c1, da1, out_dt=SG_F32, dz_out=dz_out, dz_ld=dz_ld, defer=defer)
+        dx = self.cbn1.backward(rt, c1, da1, defer, out_dt=SG_F32, dz_out=dz_out, dz_ld=dz_ld)
         # shortcut branch
         off_chain(lambda: self.short.wgrad(rt, xs, dh_op, bias_grad=False), dh_op)
         self.short.dgrad(rt, dh_op, out=dx, accumulate=True)
@@ -146,11 +135,11 @@ class ResNetBlockDown:
             xs = x
         h1 = self.conv1.forward(rt, xr, relu=True, out_dt=rt.op_dt)
         h2 = None
-        if not narrow and rt.use_tc and rt.fuse_shortcut:
+        if not narrow and rt.use_tc:
             # conv2 and the 1x1 shortcut in ONE launch: the shortcut's k-blocks land in the same TMEM accumulator
             bsum = ops.axpby(rt, 1.0, self.conv2.b.data, 1.0, self.short.b.data)
             h2 = self.conv2.forward_with_shortcut(rt, h1, self.short, xs, bsum)
-        if h2 is None and narrow and rt.use_tc and rt.fuse_shortcut and self.ci == 1:
+        if h2 is None and narrow and rt.use_tc and self.ci == 1:
             # one-channel input (the image): the 1x1 shortcut is an outer product, added in conv2's epilogue
             bsum = ops.axpby(rt, 1.0, self.conv2.b.data, 1.0, self.short.b.data)
             h2 = self.conv2.forward_with_rank1_shortcut(rt, h1, self.short, xs, bsum)
@@ -159,12 +148,6 @@ class ResNetBlockDown:
             self.short.forward(rt, xs, out=h2, accumulate=True)
         out = h2 if self.is_last else ops.avgpool2_fwd(rt, h2)
         return out, (xr, xs, h1, (h, w))
-
-    @staticmethod
-    def slice_cache(cache, a: int, b: int):
-        """Cache of the sub-batch [a, b) of a forward pass (views, no copies)."""
-        xr, xs, h1, hw = cache
-        return (xr[a:b], xs[a:b], h1[a:b], hw)
 
     def backward(self, rt: Runtime, cache, dout, wgrad: bool = True, want_dx: bool = True, fake=None, side=None):
         """fake = (b, up, mult) -- the merged discriminator backward (Discriminator.backward_merged): rows [0, b) of the batch
@@ -196,7 +179,10 @@ class ResNetBlockDown:
             dx = self.conv1.dgrad(rt, dh1[rows], (h, w), mask=xr[rows])
             self.short.dgrad(rt, dpre[rows], (h, w), out=dx, accumulate=True)
         if wgrad:
-            def filter_grads():
+            # off the input-gradient chain: the rescale and the three filter gradients go to the side stream (everything
+            # the chain reads from these tensors has been enqueued above); the caller keeps the tensors alive until it joins
+            side.extend((dpre, dh1, dout))
+            with rt.branch():
                 seen = set()
                 for t in (dpre, dh1, dout):
                     if t.data_ptr() not in seen:             # last block in fp32 mode: dpre IS dout (no cast, no pooling)
@@ -205,12 +191,4 @@ class ResNetBlockDown:
                 self.conv2.wgrad(rt, h1, dpre, also_bias=self.short.b.grad, bias_src=dout)
                 self.short.wgrad(rt, xs, dpre, bias_grad=False)
                 self.conv1.wgrad(rt, xr, dh1)
-            if side is None:
-                filter_grads()
-            else:
-                # off the input-gradient chain: the rescale and the three filter gradients go to the side stream (everything
-                # the chain reads from these tensors has been enqueued above); the caller keeps the tensors alive until it joins
-                side.extend((dpre, dh1, dout))
-                with rt.branch():
-                    filter_grads()
         return dx

@@ -18,7 +18,6 @@ __global__ void __launch_bounds__(AT_THREADS) k_attn_fwd(const float* __restrict
                                                           const float* __restrict__ g, int Q, int KV,
                                                           float* __restrict__ o, float* __restrict__ lse, int kv_w,
                                                           const int* __restrict__ kv_cols) {
-  sg_pdl_prologue();
   // ragged batches: kv_cols[n] (may be NULL) = number of valid key COLUMNS of image n; key j sits in column j % kv_w
   __shared__ __align__(16) float ks[128 * AT_DK];
   __shared__ __align__(16) float vs[128 * AT_DV];
@@ -102,7 +101,6 @@ __global__ void __launch_bounds__(AT_THREADS) k_attn_bwd_q(const float* __restri
                                                             const float* __restrict__ g, const float* __restrict__ o,
                                                             const float* __restrict__ lse, const float* __restrict__ d_o,
                                                             int Q, int KV, float* __restrict__ dtheta) {
-  sg_pdl_prologue();
   __shared__ __align__(16) float ks[128 * AT_DK];
   __shared__ __align__(16) float vs[128 * AT_DV];
   const int n = blockIdx.y;
@@ -166,7 +164,6 @@ __global__ void __launch_bounds__(AT_THREADS) k_attn_bwd_kv(const float* __restr
                                                              const float* __restrict__ lse, const float* __restrict__ d_o,
                                                              int Q, int KV, int q_per_split, float* __restrict__ dphi,
                                                              float* __restrict__ dg, unsigned int* __restrict__ sems) {
-  sg_pdl_prologue();
   __shared__ __align__(16) float qs[AT_QT * AT_DK];
   __shared__ __align__(16) float dos[AT_QT * AT_DV];
   __shared__ float ls[AT_QT], Ds[AT_QT];

@@ -60,7 +60,6 @@ static inline int atc_pad(int n) { return (n + 63) / 64 * 64 + 8; }
 // D[row] = sum_j dO[row,j] * O[row,j]   (32 columns); 8 threads per row
 __global__ void __launch_bounds__(256) k_attn_rowdot(const float* __restrict__ d_o, const float* __restrict__ o, long long rows,
                                                       float* __restrict__ D) {
-  sg_pdl_prologue();
   long long i = (long long)blockIdx.x * 256 + threadIdx.x;
   long long row = i >> 3;
   int sub = (int)(i & 7);
@@ -82,7 +81,6 @@ __global__ void __launch_bounds__(ATC_THREADS) k_attn_fwd_tc(const float* __rest
                                                               const float* __restrict__ gv, int Q, int KV, int KVp,
                                                               float* __restrict__ o, float* __restrict__ lse, int kv_w,
                                                               const int* __restrict__ kv_cols) {
-  sg_pdl_prologue();
   // ragged batches: kv_cols[n] (may be NULL) = valid key COLUMNS of image n; key j sits in column j % kv_w
   extern __shared__ __align__(16) uint8_t smem[];
   uint32_t* Kt = reinterpret_cast<uint32_t*>(smem);                         // [8][KVp]  tf32
@@ -200,7 +198,6 @@ __global__ void __launch_bounds__(ATC_THREADS) k_attn_bwd_q_tc(const float* __re
                                                                 const float* __restrict__ gv, const float* __restrict__ lse,
                                                                 const float* __restrict__ d_o, const float* __restrict__ Dv, int Q,
                                                                 int KV, int KVp, float* __restrict__ dtheta) {
-  sg_pdl_prologue();
   extern __shared__ __align__(16) uint8_t smem[];
   uint32_t* Kt = reinterpret_cast<uint32_t*>(smem);                               // [8][KVp] tf32
   __nv_bfloat16* Ktb = reinterpret_cast<__nv_bfloat16*>(Kt + ATC_DK * KVp);       // [8][KVp] bf16
@@ -286,7 +283,6 @@ __global__ void __launch_bounds__(ATC_THREADS) k_attn_bwd_kv_tc(const float* __r
                                                                  const float* __restrict__ gv, const float* __restrict__ lse,
                                                                  const float* __restrict__ d_o, const float* __restrict__ Dv, int Q,
                                                                  int KV, float* __restrict__ dphi, float* __restrict__ dg) {
-  sg_pdl_prologue();
   __shared__ uint32_t Qt[ATC_DK * ATC_QP];
   __shared__ __align__(16) __nv_bfloat16 Qtb[ATC_DK * ATC_QP];
   __shared__ __align__(16) __nv_bfloat16 dOs[ATC_QC * ATC_VROW];

@@ -19,7 +19,6 @@ static inline BnLayout bn_layout(int c) {
 
 __global__ void k_bn_stats(const float* __restrict__ x, long long rows, int c, int tc, int lanes,
                            long long rows_per_block, float* __restrict__ partial) {
-  sg_pdl_prologue();
   extern __shared__ float sm[];     // [lanes][2*c]
   int q = threadIdx.x % tc, lane = threadIdx.x / tc;
   long long r0 = (long long)blockIdx.x * rows_per_block;
@@ -48,7 +47,6 @@ __global__ void k_bn_stats(const float* __restrict__ x, long long rows, int c, i
 // slices combined through shared memory -- the serial chain per thread is nblocks/16 loads instead of nblocks.
 __global__ void __launch_bounds__(512) k_bn_stats_reduce(const float* __restrict__ partial, int nblocks, int c2,
                                                           float* __restrict__ sums) {
-  sg_pdl_prologue();
   __shared__ double sm[16][33];
   const int jx = threadIdx.x & 31, sl = threadIdx.x >> 5;
   const int j = blockIdx.x * 32 + jx;
@@ -67,7 +65,6 @@ __global__ void __launch_bounds__(512) k_bn_stats_reduce(const float* __restrict
 __global__ void k_bn_finalize(const float* __restrict__ sums, double count, int c, float eps, float momentum,
                               float* __restrict__ mean, float* __restrict__ rstd, float* __restrict__ mm,
                               float* __restrict__ mv) {
-  sg_pdl_prologue();
   int j = blockIdx.x * blockDim.x + threadIdx.x;
   if (j >= c) return;
   double m = (double)sums[j] / count;
@@ -84,7 +81,6 @@ __global__ void k_bn_finalize(const float* __restrict__ sums, double count, int 
 
 __global__ void k_bn_infer_prepare(const float* __restrict__ mm, const float* __restrict__ mv, int c, float eps,
                                    float* __restrict__ mean, float* __restrict__ rstd) {
-  sg_pdl_prologue();
   int j = blockIdx.x * blockDim.x + threadIdx.x;
   if (j >= c) return;
   mean[j] = mm[j];
@@ -96,7 +92,6 @@ __global__ void k_bn_apply(const float* __restrict__ x, long long total4, long l
                            const float* __restrict__ mean, const float* __restrict__ rstd,
                            const float* __restrict__ gamma, const float* __restrict__ beta, long long gb_stride,
                            int relu, TO* __restrict__ out) {
-  sg_pdl_prologue();
   long long stride = (long long)gridDim.x * blockDim.x;
   for (long long i = (long long)blockIdx.x * blockDim.x + threadIdx.x; i < total4; i += stride) {
     int q = (int)(i % c4);
@@ -117,7 +112,6 @@ __global__ void k_bn_bwd_reduce(const float* __restrict__ dy, const TA* __restri
                                 const float* __restrict__ mean, const float* __restrict__ rstd,
                                 float* __restrict__ s1, float* __restrict__ s2, float* __restrict__ scratch,
                                 unsigned int* __restrict__ tickets) {
-  sg_pdl_prologue();
   extern __shared__ float sm[];     // [lanes][2*c]
   int ni = blockIdx.y;
   int q = threadIdx.x % tc, lane = threadIdx.x / tc;
@@ -168,7 +162,6 @@ __global__ void k_bn_bwd_reduce(const float* __restrict__ dy, const TA* __restri
 __global__ void __launch_bounds__(256) k_bn_bwd_combine(const float* __restrict__ s1, const float* __restrict__ s2,
                                                          const float* __restrict__ gamma, long long gb_stride, int n, int c,
                                                          float* __restrict__ ab) {
-  sg_pdl_prologue();
   __shared__ float sa[8][33], sb[8][33];
   const int jx = threadIdx.x & 31, sl = threadIdx.x >> 5;
   const int j = blockIdx.x * 32 + jx;
@@ -196,7 +189,6 @@ __global__ void k_bn_bwd_apply(const float* __restrict__ dy, const TA* __restric
                                const float* __restrict__ rstd, const float* __restrict__ gamma, long long gb_stride,
                                const float* __restrict__ ab, float inv_count, int use_batch, int mask_by_x,
                                TO* __restrict__ dx, int accumulate) {
-  sg_pdl_prologue();
   long long stride = (long long)gridDim.x * blockDim.x;
   int c = 4 * c4;
   for (long long i = (long long)blockIdx.x * blockDim.x + threadIdx.x; i < total4; i += stride) {

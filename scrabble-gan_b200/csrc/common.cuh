@@ -19,14 +19,12 @@ struct sg_ctx {
   // fixed workspace of the deterministic cross-block reductions (allocated once by sg_ctx_create, see sg_det_* below):
   float* det_scratch;        // SG_DET_SCRATCH_BYTES of per-block partial sums
   unsigned int* det_tickets; // SG_DET_TICKETS arrival counters / turn semaphores, all zero between launches
-  int conv_split_tail;       // k_conv_tc: split the k-range of the tiles of a partial last wave (SGAN_NO_SPLIT_TAIL=1 disables)
+  int conv_split_tail;       // k_conv_tc: split the k-range of the tiles of a partial last wave (sg_ctx_set_conv_split_tail)
   // auxiliary streams of the copy-engine gradient-bucket all-reduce (peer.cu): one peer pull per stream, so that the pulls
   // from different peers run on different copy engines at the same time; created on first use
   cudaStream_t aux_stream[8];
   cudaEvent_t aux_fork, aux_join[8];
   int n_aux;
-  int edge_q4;               // edge-layer convs (Cin = 1 / Cout = 1, C = 64): the 4-pixels-per-thread kernels (SGAN_NO_EDGE_Q4=1 disables)
-  int pdl;                   // launch kernels with programmatic stream serialization (SGAN_PDL=1 enables; off: measured slower), see sg_launch
 };
 #define SG_DET_SCRATCH_BYTES (48u << 20)
 #define SG_DET_TICKETS 16384
@@ -60,22 +58,9 @@ void sg_set_error(const char* fmt, ...);
 static inline int sg_div_up(long long a, long long b) { return (int)((a + b - 1) / b); }
 
 // ---------------------------------------------------------------------------------------------------
-// Kernel launches.  A train step is ~300 dependent launches on one stream, most of them a few microseconds long, so the
-// boundary between two kernels is a visible share of the step.  Every libsgan kernel starts with sg_pdl_prologue() --
-// griddepcontrol.wait: block until the preceding kernel has completed and its writes are visible; then
-// griddepcontrol.launch_dependents: let the NEXT kernel's CTAs be scheduled as soon as resources free up -- so that it MAY be
-// launched with programmatic stream serialization (SGAN_PDL=1): its CTAs are then resident and past their launch latency when
-// the predecessor's last CTA retires.  No kernel touches global memory before its prologue, so the data flow is exactly that of
-// fully serialised launches.  OFF by default: measured on B200 inside the captured step graph (bench.py, 296 launches) the
-// programmatic edges cost 1.5 % (9.82 ms vs 9.67 ms per step) -- graph kernel->kernel edges are already cheap, and the early
-// resident CTAs of the successor buy nothing while they wait.  Without the attribute both instructions are no-ops.
+// Kernel launches
 // ---------------------------------------------------------------------------------------------------
 #ifdef __CUDACC__
-__device__ __forceinline__ void sg_pdl_prologue() {
-  asm volatile("griddepcontrol.wait;" ::: "memory");
-  asm volatile("griddepcontrol.launch_dependents;" ::: "memory");
-}
-
 template <typename... P, typename... A>
 static inline cudaError_t sg_launch_ex(sg_ctx* ctx, bool cooperative, void (*kern)(P...), dim3 grid, dim3 block, size_t smem, A&&... args) {
   cudaLaunchConfig_t cfg;
@@ -86,15 +71,10 @@ static inline cudaError_t sg_launch_ex(sg_ctx* ctx, bool cooperative, void (*ker
   cfg.stream = ctx->stream;
   cudaLaunchAttribute attr[1];
   memset(attr, 0, sizeof(attr));
-  if (cooperative) {              // grid-wide barrier inside: the runtime guarantees (or refuses) co-residency
-    attr[0].id = cudaLaunchAttributeCooperative;
-    attr[0].val.cooperative = 1;
-  } else {
-    attr[0].id = cudaLaunchAttributeProgrammaticStreamSerialization;
-    attr[0].val.programmaticStreamSerializationAllowed = 1;
-  }
+  attr[0].id = cudaLaunchAttributeCooperative;   // grid-wide barrier inside: the runtime guarantees (or refuses) co-residency
+  attr[0].val.cooperative = 1;
   cfg.attrs = attr;
-  cfg.numAttrs = (cooperative || ctx->pdl) ? 1 : 0;
+  cfg.numAttrs = cooperative ? 1 : 0;
   return cudaLaunchKernelEx(&cfg, kern, static_cast<P>(args)...);
 }
 // errors surface through the SG_POST_LAUNCH that follows every launch (cudaGetLastError)

@@ -26,7 +26,6 @@ template <int TN, int RN>
 __global__ void __launch_bounds__(256) k_conv_fwd_simt(sg_conv_desc d, const void* __restrict__ in,
                                                         const float* __restrict__ w, const float* __restrict__ bias,
                                                         const void* __restrict__ mask, void* __restrict__ out) {
-  sg_pdl_prologue();
   __shared__ float As[CS_TK][CS_TM + 4];
   __shared__ float Bs[CS_TK][TN + 4];
   constexpr int TX = TN / RN;                  // threads along N (16)
@@ -134,7 +133,6 @@ __global__ void __launch_bounds__(256) k_conv_fwd_simt(sg_conv_desc d, const voi
 __global__ void __launch_bounds__(256) k_conv_wgrad_simt(sg_conv_desc d, const void* __restrict__ in,
                                                           const void* __restrict__ dy, float* __restrict__ dw,
                                                           long long pos_per_split, unsigned int* __restrict__ sems) {
-  sg_pdl_prologue();
   __shared__ float As[CS_TK][CS_TM + 4];   // [pos][kflat]
   __shared__ float Bs[CS_TK][64 + 4];      // [pos][co]
   const int tid = threadIdx.x;
@@ -255,7 +253,6 @@ template <bool NARROW_IN>
 __global__ void __launch_bounds__(256) k_wgrad_narrow(sg_conv_desc d, const void* __restrict__ in, const void* __restrict__ dy,
                                                        float* __restrict__ dw, long long pos_per_block, float* __restrict__ scratch,
                                                        unsigned int* __restrict__ ticket) {
-  sg_pdl_prologue();
   extern __shared__ float red[];                       // [lanes][ntaps][wide]
   const int wide = NARROW_IN ? d.c_out : d.c_in;
   const int lanes = 256 / wide;
@@ -318,7 +315,6 @@ template <typename TIn>
 __global__ void __launch_bounds__(256, 4) k_conv_fwd_cout1(sg_conv_desc d, const TIn* __restrict__ in, const float* __restrict__ w,
                                                             const float* __restrict__ bias, const void* __restrict__ mask,
                                                             void* __restrict__ out) {
-  sg_pdl_prologue();
   // the ntaps x c_in filter lives in shared memory (2 broadcast LDS.128 per tap) instead of 72 registers per thread:
   // 4 blocks per SM instead of 2, which is what hides the load latency of this streaming kernel
   __shared__ __align__(16) float ws[9][256];
@@ -387,7 +383,6 @@ __global__ void __launch_bounds__(192) k_wgrad_narrow64(const TW* __restrict__ w
                                                          int n, int H, int W, int nH, int nW, int ntaps, sg_conv_desc d,
                                                          int sign, float* __restrict__ dw, long long chunks_per_block,
                                                          int narrow_in, float* __restrict__ scratch, unsigned int* __restrict__ ticket) {
-  sg_pdl_prologue();
   __shared__ float Bs[WN_PIX][64];
   __shared__ __align__(16) float As[9][WN_PIX];
   const int tid = threadIdx.x;
@@ -455,7 +450,6 @@ __global__ void __launch_bounds__(192) k_wgrad_narrow64(const TW* __restrict__ w
 template <typename TOut, int CH>
 __global__ void __launch_bounds__(256, 4) k_conv_fwd_cin1(sg_conv_desc d, const float* __restrict__ in, const float* __restrict__ w,
                                                            const float* __restrict__ bias, TOut* __restrict__ out) {
-  sg_pdl_prologue();
   // CH output channels per thread: the 3x3 input patch is loaded ONCE per (pixel, CH channels) and reused for CH/8 chunks
   // of 8 channels (this kernel is instruction bound: with CH = 8 the nine patch loads and their bounds checks were
   // repeated for every 8 channels)
@@ -566,7 +560,6 @@ template <typename TIn>
 __global__ void __launch_bounds__(256, 3) k_conv_fwd_cout1_q4(sg_conv_desc d, EdgeTaps tp, const TIn* __restrict__ in, const float* __restrict__ w,
                                                                const float* __restrict__ bias, const void* __restrict__ mask,
                                                                void* __restrict__ out) {
-  sg_pdl_prologue();
   __shared__ __align__(16) float ws[9][64];               // dense 3 x 3 slots (zero where the conv has no tap)
   for (int i = threadIdx.x; i < 9 * 64; i += 256) {
     int sl = i / 64, ci = i - sl * 64;
@@ -635,7 +628,6 @@ __global__ void __launch_bounds__(256, 3) k_conv_fwd_cout1_q4(sg_conv_desc d, Ed
 template <typename TOut>
 __global__ void __launch_bounds__(256, 3) k_conv_fwd_cin1_q4(sg_conv_desc d, EdgeTaps tp, const float* __restrict__ in, const float* __restrict__ w,
                                                               const float* __restrict__ bias, TOut* __restrict__ out) {
-  sg_pdl_prologue();
   __shared__ __align__(16) float ws[10][64];              // dense 3 x 3 slots + bias row
   for (int i = threadIdx.x; i < 10 * 64; i += 256) {
     int sl = i / 64, co = i - sl * 64;
@@ -719,7 +711,6 @@ template <typename TW>
 __global__ void __launch_bounds__(256, 2) k_wgrad_edge_q4(const TW* __restrict__ wide, const void* __restrict__ narrow, int narrow_dt, int n, int H,
                                                            int W, EdgeTaps tp, sg_conv_desc d, float* __restrict__ dw, int narrow_in,
                                                            float* __restrict__ scratch, unsigned int* __restrict__ ticket) {
-  sg_pdl_prologue();
   __shared__ float red[8][576];
   const int oct = threadIdx.x & 7;
   const int quads_x = W >> 2;
@@ -832,7 +823,7 @@ int sg_conv_fwd_simt(sg_ctx* ctx, const sg_conv_desc* d, const void* in, const f
   if (M == 0) return SG_OK;
   {
     EdgeTaps tp;
-    const bool q4 = ctx->edge_q4 && M < (1LL << 40) && edge_taps(d, &tp);
+    const bool q4 = M < (1LL << 40) && edge_taps(d, &tp);
     if (q4 && d->c_out == 1 && d->c_in == 64 && ((uintptr_t)in & 15) == 0) {
       long long need = (M / 4 + 31) / 32, cap = (long long)ctx->num_sms * 12;
       int grid = (int)(need < cap ? need : cap);
@@ -917,7 +908,7 @@ int sg_conv_wgrad_simt(sg_ctx* ctx, const sg_conv_desc* d, const void* in, const
           ((uintptr_t)wide & 15) == 0) {
         long long Pw = (long long)d->n * H * W;
         EdgeTaps tp0, tp;
-        if (ctx->edge_q4 && nH == H && nW == W && edge_taps(d, &tp0) && ((uintptr_t)nar & 15) == 0) {
+        if (nH == H && nW == W && edge_taps(d, &tp0) && ((uintptr_t)nar & 15) == 0) {
           // patch position of tap t in the narrow tensor: +tap for c_in == 1 (narrow = input), -tap for c_out == 1 (narrow = dy)
           for (int i = 0; i < 9; ++i) tp.slot[i] = narrow_in ? tp0.slot[i] : tp0.slot[8 - i];
           long long need = (Pw / 4 + 31) / 32, cap = (long long)ctx->num_sms * 2;

@@ -246,7 +246,6 @@ __global__ void __launch_bounds__(TC_THREADS, 1) k_conv_tc(const __grid_constant
   tc_fence_before();
   __syncthreads();
   tc_fence_after();
-  sg_pdl_prologue();        // barriers, descriptors and TMEM are set up while the preceding kernel drains; global memory from here on
   const uint32_t tmem_base = tmem_slot;
 
   if (warp == 0) {
@@ -601,7 +600,6 @@ __global__ void __launch_bounds__(TC_THREADS, 1) k_wgrad_tc(const __grid_constan
   tc_fence_before();
   __syncthreads();
   tc_fence_after();
-  sg_pdl_prologue();        // barriers, descriptors and TMEM are set up while the preceding kernel drains; global memory from here on
   const uint32_t tmem_base = tmem_slot;
 
   const int ptiles = p.tiles_x * p.tiles_y * p.tiles_n;
@@ -768,7 +766,7 @@ __global__ void __launch_bounds__(TC_THREADS, 1) k_wgrad_tc(const __grid_constan
         // Ordered turns (common.cuh, scheme A): the few pixel splits of one filter tile add their partial tiles in split
         // order.  Unit (tile, sp) only waits on unit (tile, sp - 1), which has a lower unit index: it was taken earlier by
         // its CTA (static round-robin, every CTA walks its units in increasing order), so the wait always ends.
-        if (p.det_mode == 1) {              // (det_mode 3, diagnostics only: unordered atomics as in round 1)
+        if (p.det_mode == 1) {
           if (threadIdx.x == 64) sg_turn_wait(p.sems + tile, (unsigned int)sp);
           asm volatile("bar.sync 1, 128;" ::: "memory");
         }
@@ -860,7 +858,6 @@ __global__ void __launch_bounds__(TC_THREADS, 1) k_wgrad_tc(const __grid_constan
 // ---------------------------------------------------------------------------------------------------
 template <typename TO>
 __global__ void k_pack_weights(sg_conv_desc d, const float* __restrict__ w, TO* __restrict__ out) {
-  sg_pdl_prologue();
   const long long ktot = (long long)d.ntaps * d.c_in;
   const long long total = ktot * d.c_out;
   long long stride = (long long)gridDim.x * blockDim.x;
@@ -876,7 +873,6 @@ __global__ void k_pack_weights(sg_conv_desc d, const float* __restrict__ w, TO* 
 // two float4 loads -> one 16/32-byte store
 template <typename TO>
 __global__ void __launch_bounds__(256) k_pack_weights_v8(sg_conv_desc d, const float* __restrict__ w, TO* __restrict__ out) {
-  sg_pdl_prologue();
   const int c8 = d.c_in / 8;
   const long long total8 = (long long)d.c_out * d.ntaps * c8;
   long long stride = (long long)gridDim.x * blockDim.x;
@@ -898,7 +894,6 @@ __global__ void __launch_bounds__(256) k_pack_weights_v8(sg_conv_desc d, const f
 // coalesced.  grid = (ci tiles, co tiles, taps), block = 32 x 8.
 template <typename TO>
 __global__ void __launch_bounds__(256) k_pack_weights_t(sg_conv_desc d, const float* __restrict__ w, TO* __restrict__ out) {
-  sg_pdl_prologue();
   __shared__ float tile[32][33];
   const int t = blockIdx.z;
   const int ci0 = blockIdx.x * 32, co0 = blockIdx.y * 32;
@@ -968,7 +963,6 @@ __device__ __forceinline__ void pack_tile_v8(const PackJob& j, int tile) {
   sg_st4(dst + 4, b);
 }
 __global__ void __launch_bounds__(256) k_pack_weights_multi(const __grid_constant__ PackJobs jobs) {
-  sg_pdl_prologue();
   __shared__ float smt[32][33];
   int ji = 0;
   while (ji + 1 < jobs.njobs && (int)blockIdx.x >= jobs.job[ji + 1].tile0) ++ji;
@@ -1590,17 +1584,9 @@ static int conv_wgrad_tc_impl(sg_ctx* ctx, const sg_conv_desc* d, const void* in
   p.ptiles_per_split = sg_div_up(ptiles, splits);
   p.splits = sg_div_up(ptiles, p.ptiles_per_split);
   p.partial = ctx->det_scratch;
-  // measured per layer (tools/bench_conv.py, SGAN_WGRAD_DET=turns|scratch): ordered turns cost ~one epilogue per split on the
-  // critical path, which only long main loops hide; the scratch + grid-barrier combine costs ~5-15 us flat
+  // measured per layer (tools/bench_conv.py): ordered turns cost ~one epilogue per split on the critical path, which only long
+  // main loops hide; the scratch + grid-barrier combine costs ~5-15 us flat
   p.det_mode = p.splits == 1 ? 0 : ((p.splits <= 4 && p.ptiles_per_split >= 64) ? 1 : 2);
-  {
-    const char* ov = getenv("SGAN_WGRAD_DET");          // A/B diagnostics: "legacy" = unordered atomics, "turns" = ordered turns only
-    if (ov && p.splits > 1) {
-      if (!strcmp(ov, "legacy")) p.det_mode = 3;
-      else if (!strcmp(ov, "turns")) p.det_mode = 1;
-      else if (!strcmp(ov, "scratch")) p.det_mode = 2;
-    }
-  }
   if (p.det_mode == 2 && (long long)base_units * p.splits * 128 * p.BN * (long long)sizeof(float) > (long long)SG_DET_SCRATCH_BYTES - (1 << 20)) {
     // the partial tiles would not fit the context's scratch: fall back to 4 ordered splits
     p.ptiles_per_split = sg_div_up(ptiles, 4);

@@ -31,7 +31,6 @@ __device__ __forceinline__ float lse3(float a, float b, float c) {
 __global__ void k_ctc(const float* __restrict__ logits, const int* __restrict__ labels, int Tmax, int C, int Lmax,
                       const int* __restrict__ input_len, const int* __restrict__ label_len, float* __restrict__ loss,
                       float* __restrict__ grad) {
-  sg_pdl_prologue();
   extern __shared__ float sm[];
   const int b = blockIdx.x;
   int T = input_len ? input_len[b] : Tmax, L = label_len ? label_len[b] : Lmax;
@@ -189,7 +188,6 @@ extern "C" int sg_ctc_ragged(sg_ctx* ctx, const float* logits, const int* labels
 // y = softmax(x) over rows of C fp32 values (the reference's Dense(activation='softmax'), net_architecture.py:55); one warp
 // per row, max-subtracted exp and an fp32 sum -- the first stage of k_ctc
 __global__ void k_softmax_rows(const float* __restrict__ x, long long rows, int C, float* __restrict__ y) {
-  sg_pdl_prologue();
   const int lane = threadIdx.x & 31;
   const long long r = (long long)blockIdx.x * SOFTMAX_ROWS_PER_BLOCK + (threadIdx.x >> 5);
   if (r >= rows) return;
@@ -211,7 +209,6 @@ __global__ void k_softmax_rows(const float* __restrict__ x, long long rows, int 
 __global__ void __launch_bounds__(DECODE_THREADS) k_ctc_greedy_decode(const float* __restrict__ probs, int Tmax, int C,
                                                                       const int* __restrict__ input_len, int* __restrict__ decoded,
                                                                       int* __restrict__ decoded_len, float* __restrict__ neg_sum_log) {
-  sg_pdl_prologue();
   extern __shared__ float sm[];
   int* best = reinterpret_cast<int*>(sm);
   float* logmax = sm + Tmax;
@@ -296,7 +293,6 @@ __global__ void __launch_bounds__(EDIT_THREADS) k_edit_distance(const int* __res
                                                                 int hyp_stride, const int* __restrict__ ref,
                                                                 const int* __restrict__ ref_len, int ref_stride, int nb,
                                                                 int* __restrict__ dist, long long* __restrict__ totals) {
-  sg_pdl_prologue();
   __shared__ long long s_tot[EDIT_THREADS / 32][4];
   const int lane = threadIdx.x & 31, warp = threadIdx.x >> 5;
   const int b = blockIdx.x * (EDIT_THREADS / 32) + warp;

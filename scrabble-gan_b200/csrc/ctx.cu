@@ -37,14 +37,7 @@ int sg_ctx_create(int device, void* cuda_stream, sg_ctx** out) {
   c->num_sms = prop.multiProcessorCount;
   c->encode_tiled = nullptr;
   c->launches = 0;
-  {
-    const char* e = getenv("SGAN_NO_SPLIT_TAIL");
-    c->conv_split_tail = !(e && e[0] == '1');
-    e = getenv("SGAN_NO_EDGE_Q4");
-    c->edge_q4 = !(e && e[0] == '1');
-    e = getenv("SGAN_PDL");
-    c->pdl = e && e[0] == '1';
-  }
+  c->conv_split_tail = 1;
   // the ONE device allocation libsgan makes: the fixed workspace of the deterministic reductions (common.cuh)
   cudaError_t e1 = cudaMalloc((void**)&c->det_scratch, SG_DET_SCRATCH_BYTES);
   cudaError_t e2 = e1 == cudaSuccess ? cudaMalloc((void**)&c->det_tickets, SG_DET_TICKETS * sizeof(unsigned int)) : e1;
@@ -98,14 +91,6 @@ int sg_zero(sg_ctx* ctx, void* ptr, size_t bytes) {
 int sg_ctx_set_speed_mode(sg_ctx* ctx, int on) {
   SG_REQUIRE(ctx != nullptr, "ctx is NULL");
   ctx->speed_mode = on ? 1 : 0;
-  return SG_OK;
-}
-
-int sg_ctx_set_sm_limit(sg_ctx* ctx, int sms) {
-  SG_REQUIRE(ctx != nullptr && sms >= 1, "sg_ctx_set_sm_limit: bad args");
-  cudaDeviceProp prop;
-  SG_CHECK_CUDA(cudaGetDeviceProperties(&prop, ctx->device));
-  ctx->num_sms = sms < prop.multiProcessorCount ? sms : prop.multiProcessorCount;
   return SG_OK;
 }
 

@@ -13,7 +13,6 @@ static inline int ew_grid(sg_ctx* ctx, long long work_items, int threads) {
 template <typename TO>
 __global__ void k_act_prep(const float* __restrict__ x, long long n4, long long n, TO* __restrict__ relu_out,
                            TO* __restrict__ copy_out) {
-  sg_pdl_prologue();
   long long stride = (long long)gridDim.x * blockDim.x;
   for (long long i = (long long)blockIdx.x * blockDim.x + threadIdx.x; i < n4; i += stride) {
     float4 v = sg_ld4(x + 4 * i);
@@ -31,7 +30,6 @@ __global__ void k_act_prep(const float* __restrict__ x, long long n4, long long 
 template <typename TA, typename TO>
 __global__ void k_mask_mul(const float* __restrict__ dy, const TA* __restrict__ act, TO* __restrict__ out,
                            long long n4, long long n, int accumulate) {
-  sg_pdl_prologue();
   long long stride = (long long)gridDim.x * blockDim.x;
   for (long long i = (long long)blockIdx.x * blockDim.x + threadIdx.x; i < n4; i += stride) {
     float4 d = sg_ld4(dy + 4 * i);
@@ -52,7 +50,6 @@ __global__ void k_mask_mul(const float* __restrict__ dy, const TA* __restrict__ 
 
 __global__ void k_axpby(float a, const float* __restrict__ x, float b, const float* __restrict__ y,
                         float* __restrict__ out, long long n4, long long n) {
-  sg_pdl_prologue();
   long long stride = (long long)gridDim.x * blockDim.x;
   for (long long i = (long long)blockIdx.x * blockDim.x + threadIdx.x; i < n4; i += stride) {
     float4 v = sg_ld4(x + 4 * i);
@@ -72,7 +69,6 @@ __global__ void k_axpby(float a, const float* __restrict__ x, float b, const flo
 
 __global__ void k_scale_add(const float* __restrict__ sigma, const float* __restrict__ a,
                             const float* __restrict__ x, float* __restrict__ out, long long n4, long long n) {
-  sg_pdl_prologue();
   const float s = *sigma;
   long long stride = (long long)gridDim.x * blockDim.x;
   for (long long i = (long long)blockIdx.x * blockDim.x + threadIdx.x; i < n4; i += stride) {
@@ -84,13 +80,11 @@ __global__ void k_scale_add(const float* __restrict__ sigma, const float* __rest
 }
 
 __global__ void k_tanh_fwd(const float* __restrict__ x, float* __restrict__ y, long long n) {
-  sg_pdl_prologue();
   long long stride = (long long)gridDim.x * blockDim.x;
   for (long long i = (long long)blockIdx.x * blockDim.x + threadIdx.x; i < n; i += stride) y[i] = tanhf(x[i]);
 }
 __global__ void k_tanh_bwd(const float* __restrict__ dy, const float* __restrict__ y, float* __restrict__ dx,
                            long long n) {
-  sg_pdl_prologue();
   long long stride = (long long)gridDim.x * blockDim.x;
   for (long long i = (long long)blockIdx.x * blockDim.x + threadIdx.x; i < n; i += stride) {
     float t = y[i];
@@ -98,7 +92,6 @@ __global__ void k_tanh_bwd(const float* __restrict__ dy, const float* __restrict
   }
 }
 __global__ void k_scale_rows(float* __restrict__ x, const float* __restrict__ w, int rows, long long cols) {
-  sg_pdl_prologue();
   long long n = (long long)rows * cols;
   long long stride = (long long)gridDim.x * blockDim.x;
   for (long long i = (long long)blockIdx.x * blockDim.x + threadIdx.x; i < n; i += stride) x[i] *= w[i / cols];
@@ -110,7 +103,6 @@ __global__ void k_scale_rows(float* __restrict__ x, const float* __restrict__ w,
 // grid: (blocks per sample, samples)
 template <typename T>
 __global__ void __launch_bounds__(256) k_scale_samples(T* __restrict__ x, long long per_sample8, const float* __restrict__ up, float mult) {
-  sg_pdl_prologue();
   const float f = up[blockIdx.y] * mult;
   if (f == 1.0f) return;
   T* xs = x + (long long)blockIdx.y * per_sample8 * 8;
@@ -128,7 +120,6 @@ __global__ void __launch_bounds__(256) k_scale_samples(T* __restrict__ x, long l
 // deterministic: per-block partials, summed in block order by the block that arrives last (common.cuh, scheme B)
 __global__ void k_dot(const float* __restrict__ a, const float* __restrict__ b, long long n, float* out, int accumulate,
                       float* __restrict__ scratch, unsigned int* ticket) {
-  sg_pdl_prologue();
   __shared__ float sm[32];
   float acc = 0.f;
   long long stride = (long long)gridDim.x * blockDim.x;
@@ -149,7 +140,6 @@ template <typename T, int NT>
 __global__ void __launch_bounds__(NT) k_colsum_v4(const T* __restrict__ x, long long rows, int cols, long long rows_per_block,
                                                     float* __restrict__ out, int accumulate, float* __restrict__ scratch,
                                                     unsigned int* ticket) {
-  sg_pdl_prologue();
   __shared__ float4 sm[NT];
   const int cgs = cols >> 2;                          // column groups of 4
   const int cg_per_pass = cgs < NT ? cgs : NT;
@@ -202,7 +192,6 @@ __global__ void __launch_bounds__(NT) k_colsum_v4(const T* __restrict__ x, long 
 template <typename T>
 __global__ void k_colsum(const T* __restrict__ x, long long rows, int cols, long long rows_per_block,
                          float* __restrict__ out, int accumulate, float* __restrict__ scratch, unsigned int* ticket) {
-  sg_pdl_prologue();
   long long r0 = (long long)blockIdx.x * rows_per_block;
   long long r1 = r0 + rows_per_block;
   if (r1 > rows) r1 = rows;
@@ -217,7 +206,6 @@ __global__ void k_colsum(const T* __restrict__ x, long long rows, int cols, long
 
 template <typename TO>
 __global__ void k_cast(const float* __restrict__ x, TO* __restrict__ out, long long n) {
-  sg_pdl_prologue();
   long long stride = (long long)gridDim.x * blockDim.x;
   for (long long i = (long long)blockIdx.x * blockDim.x + threadIdx.x; i < n; i += stride) sg_st(out + i, x[i]);
 }
@@ -226,7 +214,6 @@ __global__ void k_cast(const float* __restrict__ x, TO* __restrict__ out, long l
 // pooling (NHWC, c % 4 == 0)
 // ---------------------------------------------------------------------------------------------------
 __global__ void k_avgpool2_fwd(const float* __restrict__ x, int n, int h, int w, int c4, float* __restrict__ out) {
-  sg_pdl_prologue();
   int ho = h / 2, wo = w / 2;
   long long total = (long long)n * ho * wo * c4;
   long long stride = (long long)gridDim.x * blockDim.x;
@@ -249,7 +236,6 @@ __global__ void k_avgpool2_fwd(const float* __restrict__ x, int n, int h, int w,
 // math: one division chain per 4 stores instead of per store)
 template <typename TO>
 __global__ void k_avgpool2_bwd(const float* __restrict__ dout, int n, int h, int w, int c4, TO* __restrict__ dx) {
-  sg_pdl_prologue();
   const int ho = h / 2, wo = w / 2;
   const long long total = (long long)n * ho * wo * c4;
   const long long stride = (long long)gridDim.x * blockDim.x;
@@ -272,7 +258,6 @@ __global__ void k_avgpool2_bwd(const float* __restrict__ dout, int n, int h, int
 template <typename T>
 __global__ void k_maxpool_fwd(const T* __restrict__ x, int n, int h, int w, int c, int ph, int pw,
                               T* __restrict__ out) {
-  sg_pdl_prologue();
   int ho = h / ph, wo = w / pw;
   long long total = (long long)n * ho * wo * c;
   long long stride = (long long)gridDim.x * blockDim.x;
@@ -294,7 +279,6 @@ __global__ void k_maxpool_fwd(const T* __restrict__ x, int n, int h, int w, int 
 // 4 channels per thread (c % 4 == 0): 8/16-byte loads and stores
 template <typename T>
 __global__ void k_maxpool_fwd_v4(const T* __restrict__ x, int n, int h, int w, int c4, int ph, int pw, T* __restrict__ out) {
-  sg_pdl_prologue();
   int ho = h / ph, wo = w / pw;
   long long total = (long long)n * ho * wo * c4;
   long long stride = (long long)gridDim.x * blockDim.x;
@@ -318,7 +302,6 @@ __global__ void k_maxpool_fwd_v4(const T* __restrict__ x, int n, int h, int w, i
 template <typename TX, typename TO>
 __global__ void k_maxpool_bwd_v4(const float* __restrict__ dout, const TX* __restrict__ x, int n, int h, int w, int c4,
                                  int ph, int pw, int relu_mask, TO* __restrict__ dx) {
-  sg_pdl_prologue();
   int ho = h / ph, wo = w / pw;
   long long total = (long long)n * ho * wo * c4;
   long long stride = (long long)gridDim.x * blockDim.x;
@@ -359,7 +342,6 @@ __global__ void k_maxpool_bwd_v4(const float* __restrict__ dout, const TX* __res
 template <typename TX, typename TO>
 __global__ void k_maxpool_bwd(const float* __restrict__ dout, const TX* __restrict__ x, int n, int h, int w, int c,
                               int ph, int pw, int relu_mask, TO* __restrict__ dx) {
-  sg_pdl_prologue();
   int ho = h / ph, wo = w / pw;
   long long total = (long long)n * ho * wo * c;
   long long stride = (long long)gridDim.x * blockDim.x;
@@ -387,7 +369,6 @@ __global__ void k_maxpool_bwd(const float* __restrict__ dout, const TX* __restri
 
 // global average pool of relu(x): one block per (image, 128-channel slab); threads split (pixel-slices x channels)
 __global__ void k_gap_relu_fwd(const float* __restrict__ x, long long hw, int c, float* __restrict__ out) {
-  sg_pdl_prologue();
   __shared__ float sm[8][128];
   int ni = blockIdx.y;
   int c0 = blockIdx.x * 128;
@@ -408,7 +389,6 @@ __global__ void k_gap_relu_fwd(const float* __restrict__ x, long long hw, int c,
 
 __global__ void k_gap_relu_bwd(const float* __restrict__ dfeat, const float* __restrict__ x, long long hw, int c,
                                long long total, float* __restrict__ dx) {
-  sg_pdl_prologue();
   long long stride = (long long)gridDim.x * blockDim.x;
   float inv = 1.f / (float)hw;
   for (long long i = (long long)blockIdx.x * blockDim.x + threadIdx.x; i < total; i += stride) {
@@ -438,7 +418,6 @@ __device__ __forceinline__ void philox4x32_10(uint32_t c0, uint32_t c1, uint32_t
 }
 __global__ void k_philox(float* __restrict__ out, long long n, unsigned long long seed, unsigned long long offset,
                          const unsigned long long* __restrict__ offset_dev, int normal) {
-  sg_pdl_prologue();
   const unsigned long long base = offset + (offset_dev ? *offset_dev : 0ull);
   const long long groups = (n + 3) / 4, stride = (long long)gridDim.x * blockDim.x;
   for (long long g = (long long)blockIdx.x * blockDim.x + threadIdx.x; g < groups; g += stride) {
@@ -467,7 +446,6 @@ __global__ void k_philox(float* __restrict__ out, long long n, unsigned long lon
   }
 }
 __global__ void k_philox_advance(unsigned long long* offset_dev, unsigned long long by) {
-  sg_pdl_prologue();
   if (blockIdx.x == 0 && threadIdx.x == 0) *offset_dev += by;
 }
 
@@ -475,7 +453,6 @@ __global__ void k_philox_advance(unsigned long long* offset_dev, unsigned long l
 // ragged batches (several word lengths in one launch): zero everything right of a word's own width
 template <typename T>
 __global__ void k_mask_width(T* __restrict__ x, long long total4, int h, int w, int c4, const int* __restrict__ lens, int cols_per_char) {
-  sg_pdl_prologue();
   const long long stride = (long long)gridDim.x * blockDim.x;
   for (long long i = (long long)blockIdx.x * blockDim.x + threadIdx.x; i < total4; i += stride) {
     const long long pix = i / c4;
@@ -485,7 +462,6 @@ __global__ void k_mask_width(T* __restrict__ x, long long total4, int h, int w, 
   }
 }
 __global__ void k_label_lengths(const int* __restrict__ labels, int b, int l, int* __restrict__ lens) {
-  sg_pdl_prologue();
   int i = blockIdx.x * blockDim.x + threadIdx.x;
   if (i >= b) return;
   int n = 0;

@@ -17,7 +17,6 @@ __device__ __forceinline__ long long fb_out_index(int b, int l, int L, int k) {
 __global__ void __launch_bounds__(256) k_fb_fwd(const float* __restrict__ z, int z_stride, const int* __restrict__ y,
                                                  int L, int vocab, const float* __restrict__ bank,
                                                  float* __restrict__ out) {
-  sg_pdl_prologue();
   __shared__ float zs[FB_J];
   int p = blockIdx.y, b = p / L, l = p % L;
   int v = y[p];
@@ -38,7 +37,6 @@ __global__ void __launch_bounds__(256) k_fb_fwd(const float* __restrict__ z, int
 __global__ void __launch_bounds__(128) k_fb_bwd_bank(const float* __restrict__ dout, const float* __restrict__ z,
                                                       int z_stride, const int* __restrict__ y, int B, int L,
                                                       float* __restrict__ dbank) {
-  sg_pdl_prologue();
   __shared__ float zs[FB_J];
   int v = blockIdx.y;
   int k = blockIdx.x * 128 + threadIdx.x;
@@ -65,7 +63,6 @@ __global__ void __launch_bounds__(128) k_fb_bwd_bank(const float* __restrict__ d
 __global__ void __launch_bounds__(256) k_fb_bwd_z(const float* __restrict__ dout, const int* __restrict__ y, int L,
                                                    int vocab, const float* __restrict__ bank, float* __restrict__ dz0,
                                                    int dz_stride) {
-  sg_pdl_prologue();
   __shared__ float sm[32];
   int j = blockIdx.x, b = blockIdx.y;
   float acc = 0.f;

@@ -14,7 +14,6 @@ template <int GT_K>
 __global__ void __launch_bounds__(256) k_gemm(int ta, int tb, int M, int N, int K, const float* __restrict__ A, int lda,
                                                const float* __restrict__ B, int ldb, float* __restrict__ C, int ldc,
                                                const float* __restrict__ bias, int accumulate, int k_per_split, float* __restrict__ scratch, unsigned int* __restrict__ tickets) {
-  sg_pdl_prologue();
   __shared__ float As[GT_K][GT_M + 4];
   __shared__ float Bs[GT_K][GT_N + 4];
   const int tid = threadIdx.x;
@@ -154,7 +153,6 @@ struct CbnSegs {
 // out[r, col] = sum_k z[r, z_off(seg) + k] * W_seg[k, col - col0(seg)],  k < 32
 __global__ void __launch_bounds__(256) k_cbn_dense_fwd(const float* __restrict__ z, int z_stride, int n, CbnSegs t,
                                                        const float* __restrict__ w, float* __restrict__ out) {
-  sg_pdl_prologue();
   const long long total = (long long)n * t.total;
   for (long long i = (long long)blockIdx.x * blockDim.x + threadIdx.x; i < total; i += (long long)gridDim.x * blockDim.x) {
     const int col = (int)(i % t.total), r = (int)(i / t.total);
@@ -172,7 +170,6 @@ __global__ void __launch_bounds__(256) k_cbn_dense_fwd(const float* __restrict__
 // dW_seg[k, cl] += sum_r z[r, z_off + k] * s_seg[r, cl]     (one thread per output: no atomics, fixed order over r)
 __global__ void __launch_bounds__(256) k_cbn_dense_wgrad(const float* __restrict__ z, int z_stride, int n, CbnSegs t,
                                                          float* __restrict__ dw) {
-  sg_pdl_prologue();
   const long long total = 32LL * t.total;
   for (long long i = (long long)blockIdx.x * blockDim.x + threadIdx.x; i < total; i += (long long)gridDim.x * blockDim.x) {
     const int col = (int)(i % t.total), k = (int)(i / t.total);

@@ -34,7 +34,6 @@ __device__ double block_sum_d(double v, double* sm) {
 __global__ void k_loss_sums(int kind, int use_w, const float* d_real, const float* d_fake, const float* s_real,
                             const float* s_fake, const float* s5, const float* r_fake, const float* r_real, int b,
                             double* sums) {
-  sg_pdl_prologue();
   __shared__ double sm[32];
   double acc[SUM_N];
   for (int j = 0; j < SUM_N; ++j) acc[j] = 0.0;
@@ -73,7 +72,6 @@ __global__ void k_loss_finish(int kind, int use_w, int balance, float alpha, con
                               const double* sums, float* up_d_real, float* up_d_fake_d, float* up_s_real,
                               float* up_s_fake_w, float* up_s_slot5, float* up_d_fake_g, float* up_s_fake_g,
                               float* up_r_fake_g, float* stats) {
-  sg_pdl_prologue();
   const double N = sums[SUM_N];
   const double mean_g = sums[SUM_G] / N, mean_r = sums[SUM_R] / N;
   double var_g = sums[SUM_G2] / N - mean_g * mean_g, var_r = sums[SUM_R2] / N - mean_r * mean_r;
@@ -179,7 +177,6 @@ int sg_loss_finish(sg_ctx* ctx, int kind, int use_w, int balance, float alpha, c
 // terms[7][b]: d_loss, d_loss_real, d_loss_fake, g_loss, s_loss, s_loss_1, s_loss_2   (net_loss.py return order)
 __global__ void k_loss_terms(int kind, const float* d_real, const float* d_fake, const float* s_a, const float* s_b,
                              const float* s_c, int b, float* terms) {
-  sg_pdl_prologue();
   for (int i = blockIdx.x * blockDim.x + threadIdx.x; i < b; i += gridDim.x * blockDim.x) {
     float dr = d_real[i], df = d_fake[i], sa = s_a[i], sb = s_b[i], sc = s_c ? s_c[i] : 0.f;
     float dlr, dlf, g, s1, s2;
@@ -199,7 +196,6 @@ __global__ void k_loss_terms(int kind, const float* d_real, const float* d_fake,
 
 // g_bal = g + alpha (sd_g / sd_r) r ; r_bal = alpha (sd_g / sd_r) r ; stds = {sd_r, sd_g}   (single CTA)
 __global__ void k_grad_balance(const float* r, const float* g, int b, float alpha, float* g_bal, float* r_bal, float* stds) {
-  sg_pdl_prologue();
   __shared__ double sm[32];
   double sr = 0, sr2 = 0, sg = 0, sg2 = 0;
   for (int i = threadIdx.x; i < b; i += blockDim.x) {
@@ -249,7 +245,6 @@ int sg_grad_balance(sg_ctx* ctx, const float* r_fake, const float* g_loss, int b
 // ---------------------------------------------------------------------------------------------------
 __global__ void __launch_bounds__(256) k_imgbal_sums(const float* __restrict__ gd, const float* __restrict__ gr, long long n,
                                                       double* __restrict__ sums, double* __restrict__ scratch, unsigned int* ticket) {
-  sg_pdl_prologue();
   __shared__ double sm[32];
   double a[4] = {0.0, 0.0, 0.0, 0.0};
   const long long stride = (long long)gridDim.x * blockDim.x;
@@ -277,7 +272,6 @@ __global__ void __launch_bounds__(256) k_imgbal_sums(const float* __restrict__ g
 // g_loss_balanced = g_loss_final = g_loss + r_loss_balanced, alpha, r_loss_fake_std := sd_r, g_loss_std := sd_d
 __global__ void k_imgbal_apply(const float* __restrict__ gd, const float* __restrict__ gr, long long n, float alpha,
                                const double* __restrict__ sums, float* __restrict__ out, float* __restrict__ stats) {
-  sg_pdl_prologue();
   const double N = sums[4];
   const double md = sums[0] / N, mr = sums[2] / N;
   double vd = sums[1] / N - md * md, vr = sums[3] / N - mr * mr;

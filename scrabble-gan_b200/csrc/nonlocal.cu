@@ -39,7 +39,6 @@ template <int K, int N, bool TRANS_W>
 __global__ void __launch_bounds__(256) k_nl_rowgemm(long long rows, SegMat A, SegMat W, SegMat C, const float* __restrict__ alpha_p,
                                                      int accumulate, const float* __restrict__ resid_scale_p,
                                                      const float* __restrict__ resid_x, float* __restrict__ resid_out) {
-  sg_pdl_prologue();
   using T = NlTile<K, N>;
   __shared__ __align__(16) float As[K][T::TRP];     // transposed: As[k][row]
   __shared__ __align__(16) float Ws[K][N];
@@ -133,7 +132,6 @@ template <int KA, int KB>
 __global__ void __launch_bounds__(NLW_SUB * (KA / 4) * (KB / 4)) k_nl_wgrad(long long rows, long long rows_per_block, SegMat A, SegMat B,
                                                                              SegMat DW, const float* __restrict__ alpha_p,
                                                                              float* __restrict__ scratch, unsigned int* __restrict__ ticket) {
-  sg_pdl_prologue();
   constexpr int TA = KA / 4, TB = KB / 4, NT = TA * TB;
   extern __shared__ __align__(16) float nlw_smem[];
   const int sub = threadIdx.x / NT, tid = threadIdx.x % NT;
@@ -239,7 +237,6 @@ template <int K, int N, bool TRANS_W>
 __global__ void __launch_bounds__(256) k_nl_rowgemm_mma(long long rows, SegMat A, SegMat W, SegMat C, const float* __restrict__ alpha_p,
                                                          int accumulate, const float* __restrict__ resid_scale_p,
                                                          const float* __restrict__ resid_x, float* __restrict__ resid_out) {
-  sg_pdl_prologue();
   constexpr int KP = K + 8;                                  // padded row (bf16): conflict-free 32-bit fragment reads
   __shared__ __align__(16) __nv_bfloat16 Wt[N * KP];         // Wt[n][k] = Wlogical[k][n]
   for (int i = threadIdx.x; i < K * N; i += 256) {
@@ -308,7 +305,6 @@ template <int KA, int KB>
 __global__ void __launch_bounds__(256, 1) k_nl_wgrad_mma(long long rows, long long rows_per_block, SegMat A, SegMat B, SegMat DW,
                                                           const float* __restrict__ alpha_p, float* __restrict__ scratch,
                                                           unsigned int* __restrict__ ticket) {
-  sg_pdl_prologue();
   constexpr int MT = KA / 16, NT = KB / 8;
   __shared__ float red[KA * KB];
   for (int i = threadIdx.x; i < KA * KB; i += 256) red[i] = 0.f;

@@ -11,7 +11,6 @@
 __global__ void k_adam(float* __restrict__ w, const float* __restrict__ g, float* __restrict__ m, float* __restrict__ v,
                        long long n4, long long n, float lr_t, float b1, float b2, float eps, __nv_bfloat16* __restrict__ wb,
                        const float* __restrict__ lr_dev) {
-  sg_pdl_prologue();
   if (lr_dev) lr_t = *lr_dev;          // step size from device memory (CUDA-graph replays: see k_adam_prepare)
   long long stride = (long long)gridDim.x * blockDim.x;
   const float c1 = 1.f - b1, c2 = 1.f - b2;
@@ -42,7 +41,6 @@ __global__ void k_adam(float* __restrict__ w, const float* __restrict__ g, float
 template <bool kNoM, bool kClear>
 __global__ void k_adam_fused(float* __restrict__ w, float* __restrict__ g, float* __restrict__ m, float* __restrict__ v, long long n4,
                              long long n, float b1, float b2, float eps, __nv_bfloat16* __restrict__ wb, const float* __restrict__ lr_dev) {
-  sg_pdl_prologue();
   const float lr_t = *lr_dev;
   long long stride = (long long)gridDim.x * blockDim.x;
   const float c1 = 1.f - b1, c2 = 1.f - b2;
@@ -76,7 +74,6 @@ __global__ void k_adam_fused(float* __restrict__ w, float* __restrict__ g, float
 // Device-side step counter and Keras step size  lr_t = lr sqrt(1 - b2^t) / (1 - b1^t):  t_set >= 0 sets the counter (eager
 // calls pass the host iteration count), t_set < 0 increments it (captured launches: every graph replay advances by one).
 __global__ void k_adam_prepare(int* __restrict__ step, float* __restrict__ lr_dev, int t_set, float lr, float b1, float b2) {
-  sg_pdl_prologue();
   if (blockIdx.x == 0 && threadIdx.x == 0) {
     int t = t_set >= 0 ? t_set : *step + 1;
     *step = t;
@@ -87,7 +84,6 @@ __global__ void k_adam_prepare(int* __restrict__ step, float* __restrict__ lr_de
 
 __global__ void k_rmsprop(float* __restrict__ w, const float* __restrict__ g, float* __restrict__ ms, long long n,
                           float lr, float rho, float eps) {
-  sg_pdl_prologue();
   long long stride = (long long)gridDim.x * blockDim.x;
   for (long long i = (long long)blockIdx.x * blockDim.x + threadIdx.x; i < n; i += stride) {
     float gi = g[i];
@@ -101,7 +97,6 @@ __global__ void k_rmsprop(float* __restrict__ w, const float* __restrict__ g, fl
 // v_raw[r] = sum_c u[c] W[r,c]  (one warp per row)
 __global__ void k_sn_rowdot(const float* __restrict__ w, int rows, int cols, const float* __restrict__ u,
                             const float* __restrict__ u_scale, float* __restrict__ v) {
-  sg_pdl_prologue();
   int r = blockIdx.x * (blockDim.x >> 5) + (threadIdx.x >> 5);
   if (r >= rows) return;
   int lane = threadIdx.x & 31;
@@ -115,7 +110,6 @@ __global__ void k_sn_rowdot(const float* __restrict__ w, int rows, int cols, con
 __global__ void k_sn_coldot(const float* __restrict__ w, int rows, int cols, const float* __restrict__ v,
                             const float* __restrict__ v_scale, int rows_per_block, float* __restrict__ t,
                             float* __restrict__ scratch, unsigned int* __restrict__ tickets) {
-  sg_pdl_prologue();
   int c = blockIdx.x * blockDim.x + threadIdx.x;
   int r0 = blockIdx.y * rows_per_block, r1 = r0 + rows_per_block;
   if (r1 > rows) r1 = rows;
@@ -132,7 +126,6 @@ __global__ void k_sn_coldot(const float* __restrict__ w, int rows, int cols, con
 }
 // out[0] = rsqrt(max(sum x^2, 1e-12))   (tf.nn.l2_normalize scale), out[1] = sum x^2
 __global__ void k_sn_invnorm(const float* __restrict__ x, int n, float* __restrict__ out) {
-  sg_pdl_prologue();
   __shared__ float sm[32];
   float acc = 0.f;
   for (int i = threadIdx.x; i < n; i += blockDim.x) acc += x[i] * x[i];
@@ -142,7 +135,6 @@ __global__ void k_sn_invnorm(const float* __restrict__ x, int n, float* __restri
 // sigma = (v W) . u_hat = sum_c t[c] * (t[c]*inv_t) ; u_out = t*inv_t
 __global__ void k_sn_sigma(const float* __restrict__ t, int cols, const float* __restrict__ inv_t, float* __restrict__ u_out,
                            float* __restrict__ sigma) {
-  sg_pdl_prologue();
   __shared__ float sm[32];
   float s = *inv_t, acc = 0.f;
   for (int i = threadIdx.x; i < cols; i += blockDim.x) {
@@ -154,7 +146,6 @@ __global__ void k_sn_sigma(const float* __restrict__ t, int cols, const float* _
   if (threadIdx.x == 0) *sigma = r;
 }
 __global__ void k_sn_scale(const float* __restrict__ w, long long n, const float* __restrict__ sigma, float* __restrict__ out) {
-  sg_pdl_prologue();
   float inv = 1.f / *sigma;
   long long stride = (long long)gridDim.x * blockDim.x;
   for (long long i = (long long)blockIdx.x * blockDim.x + threadIdx.x; i < n; i += stride) out[i] = w[i] * inv;
@@ -290,7 +281,6 @@ int sg_spectral_norm(sg_ctx* ctx, const float* w, int rows, int cols, const floa
 __global__ void k_sn_bwd(float* __restrict__ g, const float* __restrict__ dot, const float* __restrict__ v_raw,
                          const float* __restrict__ inv_v, const float* __restrict__ u_hat, const float* __restrict__ sigma, int rows,
                          int cols) {
-  sg_pdl_prologue();
   const float d = *dot, iv = *inv_v, is = 1.f / *sigma;
   const long long n = (long long)rows * cols, stride = (long long)gridDim.x * blockDim.x;
   for (long long i = (long long)blockIdx.x * blockDim.x + threadIdx.x; i < n; i += stride) {

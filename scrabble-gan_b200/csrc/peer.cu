@@ -70,7 +70,6 @@ __device__ __forceinline__ void peer_publish_and_wait(const PeerTable& pt) {
 
 template <typename T>
 __global__ void __launch_bounds__(512) k_peer_allreduce(T* __restrict__ data, int n, PeerTable pt) {
-  sg_pdl_prologue();
   pt.seq = peer_next_seq(pt);
   const size_t slot = (size_t)(pt.seq & 1u) * SG_PEER_SLOT_BYTES;
   T* mine = reinterpret_cast<T*>(pt.buf[pt.rank] + slot);
@@ -97,7 +96,6 @@ __global__ void __launch_bounds__(1024) k_bn_finalize_peer(const float* __restri
                                                             float eps, float momentum, float* __restrict__ sums_out,
                                                             float* __restrict__ mean, float* __restrict__ rstd,
                                                             float* __restrict__ mm, float* __restrict__ mv, PeerTable pt) {
-  sg_pdl_prologue();
   __shared__ double red[1024];
   pt.seq = peer_next_seq(pt);
   const int c2 = 2 * c;
@@ -152,7 +150,6 @@ __global__ void __launch_bounds__(1024) k_bn_finalize_peer(const float* __restri
 
 // barrier only: publish my next sequence number to every peer, wait for theirs
 __global__ void __launch_bounds__(32) k_peer_barrier(PeerTable pt) {
-  sg_pdl_prologue();
   pt.seq = peer_next_seq(pt);
   peer_publish_and_wait(pt);
   peer_commit_seq(pt);
@@ -162,7 +159,6 @@ __global__ void __launch_bounds__(32) k_peer_barrier(PeerTable pt) {
 // staging slots the copy engines filled): the same additions in the same order whichever rank owns the shard
 __global__ void __launch_bounds__(256) k_bucket_reduce(float* __restrict__ g, const float* __restrict__ staging, long long len,
                                                         long long slot_stride, int world, int rank) {
-  sg_pdl_prologue();
   const long long n4 = len / 4, stride = (long long)gridDim.x * blockDim.x;
   for (long long i = (long long)blockIdx.x * blockDim.x + threadIdx.x; i < n4; i += stride) {
     float4 acc = make_float4(0.f, 0.f, 0.f, 0.f);
@@ -186,7 +182,6 @@ __global__ void __launch_bounds__(256) k_bucket_reduce(float* __restrict__ g, co
 struct BucketPtrs { unsigned long long g[SG_PEER_MAX_WORLD]; };
 
 __global__ void __launch_bounds__(256) k_bucket_pull_reduce(BucketPtrs bp, long long lo, long long len, int world, int rank) {
-  sg_pdl_prologue();
   float* mine = reinterpret_cast<float*>(bp.g[rank]) + lo;
   const long long n4 = len / 4, stride = (long long)gridDim.x * blockDim.x;
   for (long long i = (long long)blockIdx.x * blockDim.x + threadIdx.x; i < n4; i += stride) {
@@ -211,7 +206,6 @@ __global__ void __launch_bounds__(256) k_bucket_pull_reduce(BucketPtrs bp, long 
 
 // all-gather: blockIdx.y = peer index (skipping myself); copy that peer's reduced shard into my bucket
 __global__ void __launch_bounds__(256) k_bucket_gather(BucketPtrs bp, long long shard, long long n, int world, int rank) {
-  sg_pdl_prologue();
   const int r = (int)blockIdx.y < rank ? (int)blockIdx.y : (int)blockIdx.y + 1;
   long long lo = (long long)r * shard, hi = lo + shard;
   if (lo > n) lo = n;

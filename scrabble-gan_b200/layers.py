@@ -204,7 +204,7 @@ class ConvTransposeLayer:
                                          int(accumulate))
                 self._descs[key] = d
             descs.append(d)
-        if rt.merge_phases and len(descs) > 1 and all(ops.direct_ok(rt, d) for d in descs):
+        if len(descs) > 1 and all(ops.direct_ok(rt, d) for d in descs):
             ops.conv_run_phases(rt, descs, x, self.w.mirror(rt), b, out)       # every phase in ONE launch
             return out
         for (py, px), d in zip(self.phases, descs):

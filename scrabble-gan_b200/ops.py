@@ -147,10 +147,10 @@ def direct_ok(rt: Runtime, d: ConvDesc, force: bool = False) -> bool:
     """True when the tensor-core launch should read the filter in place from the store's bf16 mirror (no packing pass).
     By default only roles for which the master layout is already K-major (dgrads of Conv2D, phases of Conv2DTranspose):
     reading an HWIO filter in place makes it an N-major UMMA operand, which measured ~20% slower on the big forward
-    convs than the packed K-major copy (profiles/), more than the packing pass costs.  SGAN_DIRECT_NMAJOR=1 enables it."""
-    if not (rt.use_direct and rt.mode == "bf16" and _abi.load().sg_conv_tc_direct_supported(C.byref(d))):
+    convs than the packed K-major copy (profiles/), more than the packing pass costs."""
+    if not (rt.mode == "bf16" and _abi.load().sg_conv_tc_direct_supported(C.byref(d))):
         return False
-    return force or d.w_ci_stride == 1 or rt.direct_nmajor
+    return force or d.w_ci_stride == 1
 
 
 class _Traced:
@@ -241,9 +241,9 @@ def _conv_wgrad(rt: Runtime, d: ConvDesc, x, dy, dw_master, force_simt: bool = F
     db (and db2): bias gradient(s) to accumulate the column sums of dy into IN THE SAME LAUNCH; returns True when that was
     done (tensor-core path of a plain Conv2D whose extra bias units fit into the idle slots of the launch's last wave --
     sg_conv_wgrad_tc_bias_fits; force_bias skips that test), False when the caller still has to sum dy itself."""
-    tc_dt = SG_BF16 if rt.mode == "bf16" else (SG_F32 if (rt.mode == "tf32" and rt.tf32_wgrad_tc) else None)
+    tc_dt = SG_BF16 if rt.mode == "bf16" else (SG_F32 if rt.mode == "tf32" else None)
     if not force_simt and tc_dt is not None and d.in_dt == tc_dt and d.out_dt == tc_dt and tc_ok(rt, d):
-        if db is not None and rt.fuse_bias_grad and d.out_sy == 1 and d.out_sx == 1 and d.grid_h == d.out_h and d.grid_w == d.out_w and \
+        if db is not None and d.out_sy == 1 and d.out_sx == 1 and d.grid_h == d.out_h and d.grid_w == d.out_w and \
                 (force_bias or _abi.load().sg_conv_wgrad_tc_bias_fits(rt.ctx, C.byref(d))):
             call.sg_conv_wgrad_tc_bias(rt.ctx, C.byref(d), _p(x), _p(dy), _p(dw_master), _p(db), _p(db2))
             return True

@@ -42,13 +42,6 @@ class Runtime:
         # discriminator's inside a train step): created on first use by branch()
         self.side_stream = None
         self._side_ctx = None
-        self.concurrent_branches = os.environ.get("SGAN_NO_BRANCHES", "0") != "1"
-        # D's filter gradients (merged backward) on the side stream, next to D's input-gradient chain and G's backward pass;
-        # side_sms > 0 sizes the side stream's grids for that many SMs, leaving the rest to the main stream's chain
-        self.side_d_wgrads = os.environ.get("SGAN_NO_SIDE_D_WGRADS", "0") != "1"
-        self.side_sms = int(os.environ.get("SGAN_SIDE_SMS", "0"))
-        # G's filter gradients on the side stream, next to its input-gradient chain
-        self.side_wgrads = os.environ.get("SGAN_NO_SIDE_WGRADS", "0") != "1"
         self.num_sms = torch.cuda.get_device_properties(device).multi_processor_count
         self.set_mode(mode)
         # data-parallel state (see dp.py)
@@ -74,27 +67,10 @@ class Runtime:
         self.use_tc = mode in ("bf16", "tf32")
         self.op_dt = SG_BF16 if mode == "bf16" else SG_F32
         self.op_torch = torch.bfloat16 if mode == "bf16" else torch.float32
-        # bf16 mode: tensor-core convs read their filters in place from a bf16 mirror of the flat parameter buffer
-        self.use_direct = os.environ.get("SGAN_NO_DIRECT", "0") != "1"
-        self.direct_nmajor = os.environ.get("SGAN_DIRECT_NMAJOR", "0") == "1"
-        self.fuse_shortcut = os.environ.get("SGAN_NO_FUSED_SHORTCUT", "0") != "1"
-        self.merge_r_backward = os.environ.get("SGAN_NO_MERGED_R_BWD", "0") != "1"
-        # D's two backward passes of a step (D loss: filter gradients; G loss: image gradient through the frozen D) as one
-        self.merge_d_backward = os.environ.get("SGAN_NO_MERGED_D_BWD", "0") != "1"
-        # "tf32" mode: filter gradients on the tensor cores too (fp32 operands read as tf32, MN-major 32-byte-atom swizzle)
-        self.tf32_wgrad_tc = os.environ.get("SGAN_TF32_WGRAD_SIMT", "0") != "1"
-        # bias gradients of tensor-core convs come out of the filter-gradient launch (dy^T . 1 on the tensor cores)
-        self.fuse_bias_grad = os.environ.get("SGAN_NO_FUSED_BIAS_GRAD", "0") != "1"
-        # the generator's 12 conditional-batch-norm Dense layers (and their filter gradients) as one grouped launch each
-        self.group_cbn_dense = os.environ.get("SGAN_NO_GROUPED_CBN", "0") != "1"
         self.trace = None                       # diagnostics: a list makes ops.conv_* record (role, shape, events) per launch
-        # all output phases of a transposed conv in one tensor-core launch
-        self.merge_phases = os.environ.get("SGAN_NO_MERGED_PHASES", "0") != "1"
-        # one packing launch per network and step instead of one per layer
-        self.batch_packs = os.environ.get("SGAN_NO_BATCHED_PACKS", "0") != "1"
         for c in (self._main_ctx, self._side_ctx):
             if c is not None:
-                call.sg_ctx_set_speed_mode(c, int(mode == "bf16" and os.environ.get("SGAN_NO_NL_TC", "0") != "1"))
+                call.sg_ctx_set_speed_mode(c, int(mode == "bf16"))
 
     # ---- memory helpers (torch = allocator only) ------------------------------------------------------
     def empty(self, shape, dt: int = SG_F32) -> torch.Tensor:
@@ -166,7 +142,7 @@ class Runtime:
             br.join()                 # the main stream waits for the branch
 
         The side context owns its own workspace (deterministic-reduction scratch, tickets), so kernels of the two streams
-        never share one.  With concurrent_branches off the branch degenerates to the main stream (same results)."""
+        never share one."""
         return Branch(self)
 
 
@@ -217,46 +193,38 @@ class Runtime:
 class Branch:
     def __init__(self, rt: Runtime):
         self.rt = rt
-        self.active = rt.concurrent_branches
         self._ctxmgr = None
         self._done = None               # event recorded on the side stream at the end of the last `with` block of this branch
-        if not self.active:
-            return
         if rt.side_stream is None:
             rt.side_stream = torch.cuda.Stream(device=rt.device)
             handle = C.c_void_p()
             call.sg_ctx_create(rt.device_index, C.c_void_p(rt.side_stream.cuda_stream), C.byref(handle))
             rt._side_ctx = handle
-            call.sg_ctx_set_speed_mode(handle, int(rt.mode == "bf16" and os.environ.get("SGAN_NO_NL_TC", "0") != "1"))
-            if rt.side_sms > 0:
-                call.sg_ctx_set_sm_limit(handle, rt.side_sms)
+            call.sg_ctx_set_speed_mode(handle, int(rt.mode == "bf16"))
         self.main = torch.cuda.current_stream(rt.device)
         rt.side_stream.wait_stream(self.main)
 
     def __enter__(self):
-        if self.active:
-            self.rt.ctx = self.rt._side_ctx
-            self._ctxmgr = torch.cuda.stream(self.rt.side_stream)
-            self._ctxmgr.__enter__()
+        self.rt.ctx = self.rt._side_ctx
+        self._ctxmgr = torch.cuda.stream(self.rt.side_stream)
+        self._ctxmgr.__enter__()
         return self
 
     def __exit__(self, *exc):
-        if self.active:
-            self._done = torch.cuda.Event()
-            self._done.record(self.rt.side_stream)
-            self._ctxmgr.__exit__(*exc)
-            self.rt.ctx = self.rt._main_ctx
+        self._done = torch.cuda.Event()
+        self._done.record(self.rt.side_stream)
+        self._ctxmgr.__exit__(*exc)
+        self.rt.ctx = self.rt._main_ctx
         return False
 
     def join(self) -> None:
         """The current stream waits for what THIS branch enqueued (its `with` blocks) -- not for work other branches put on
         the side stream afterwards; a branch without a `with` block joins the whole side stream."""
-        if self.active:
-            cur = torch.cuda.current_stream(self.rt.device)
-            if self._done is not None:
-                cur.wait_event(self._done)
-            else:
-                cur.wait_stream(self.rt.side_stream)
+        cur = torch.cuda.current_stream(self.rt.device)
+        if self._done is not None:
+            cur.wait_event(self._done)
+        else:
+            cur.wait_stream(self.rt.side_stream)
 
 
 _default: Optional[Runtime] = None

@@ -179,7 +179,7 @@ def _train_step_case(rt, mode, use_w, loss_name, balance, tol_out, tol_grad, b=3
     """`rounding`: operand-rounding mode of the oracle ("bf16" / "tf32", sgan_oracle.set_operand_rounding) so that the
     reduced-precision modes are compared against an oracle that rounds where the CUDA path rounds."""
     rt.set_mode(mode)
-    O.set_operand_rounding(rounding, wgrad=(rounding == "bf16" or bool(getattr(rt, "tf32_wgrad_tc", False))))
+    O.set_operand_rounding(rounding)
     try:
         return _train_step_case_impl(rt, mode, use_w, loss_name, balance, tol_out, tol_grad, b, l_r, l_f, style_encoder, seed, calibrate)
     finally:

@@ -86,16 +86,12 @@ def _g_backward_with_oracle_image_gradient(rt, soft, P, inputs, extra, g_exp, tw
     assert_grads(G.store.grad_dict(), g_exp, tw, tt, "{}: G gradients from the oracle's image gradient (G's backward operator)".format(what), soft=soft)
 
 
-def _oracle_step(P, images, labels, fake_labels, z, mode, tf32_wgrad=False, **kw):
-    O.set_operand_rounding({"fp32": None, "tf32": "tf32", "bf16": "bf16"}[mode], wgrad=(mode == "bf16" or tf32_wgrad))
+def _oracle_step(P, images, labels, fake_labels, z, mode, **kw):
+    O.set_operand_rounding({"fp32": None, "tf32": "tf32", "bf16": "bf16"}[mode])
     try:
         return O.train_step(P, {}, images, labels, fake_labels, z, return_grads=True, **kw)
     finally:
         O.set_operand_rounding(None)
-
-
-def _tf32_wgrad_on_tc(rt):
-    return bool(getattr(rt, "tf32_wgrad_tc", False))
 
 
 # ----------------------------------------------------------------------------------------------------
@@ -104,23 +100,22 @@ def _tf32_wgrad_on_tc(rt):
 _FUSED_ORACLE = {}
 
 
-def _fused_case(mode, tf32_wgrad):
+def _fused_case(mode):
     """B = 16, L = 3 (fp64 oracle with operand rounding: ~20 s once per mode)."""
-    key = (mode, tf32_wgrad)
-    if key not in _FUSED_ORACLE:
+    if mode not in _FUSED_ORACLE:
         dt = torch.float64
         b, l = 16, 3
         P = make_params(40, dt)
         inputs = make_inputs(41, b, l, l, dt)
-        stats, newp, _, grads, extra = _oracle_step(P, *inputs, mode, tf32_wgrad)
-        _FUSED_ORACLE[key] = (P, inputs, stats, grads, extra)
-    return _FUSED_ORACLE[key]
+        stats, newp, _, grads, extra = _oracle_step(P, *inputs, mode)
+        _FUSED_ORACLE[mode] = (P, inputs, stats, grads, extra)
+    return _FUSED_ORACLE[mode]
 
 
 @pytest.mark.parametrize("graph", [False, True], ids=["eager", "graph-replay"])
 @pytest.mark.parametrize("mode", ["bf16", "tf32"])
 def test_fused_path_matches_rounded_oracle(rt, mode, graph):
-    """`test_bf16_matches_quantised_oracle`: l_r == l_f (fused 2B batch), merge_r_backward on, eager and replayed from a
+    """`test_bf16_matches_quantised_oracle`: l_r == l_f (fused 2B batch), eager and replayed from a
     CUDA graph; gradients of all three networks against the fp64 oracle with operand rounding."""
     rt.set_mode(mode)
     old = (du.GRAPH_ENABLED, du.GRAPH_WARMUP)
@@ -128,8 +123,7 @@ def test_fused_path_matches_rounded_oracle(rt, mode, graph):
     try:
         du._graph_cache.clear()
         du.GRAPH_ENABLED, du.GRAPH_WARMUP = graph, 0
-        assert rt.merge_r_backward
-        P, (images, labels, fake_labels, z), stats, grads, extra = _fused_case(mode, _tf32_wgrad_on_tc(rt))
+        P, (images, labels, fake_labels, z), stats, grads, extra = _fused_case(mode)
         if graph:
             # every kernel of the step is launched once eagerly first (on throw-away models): CUDA loads a kernel's module
             # at its first launch, which must not happen inside a stream capture
@@ -180,12 +174,11 @@ class _FullCase:
         self.inputs = make_inputs(61, self.B, self.L, self.L, dt)
         self._oracle = {}
 
-    def oracle(self, mode, tf32_wgrad=False):
-        key = (mode, tf32_wgrad)
-        if key not in self._oracle:
-            stats, newp, _, grads, extra = _oracle_step(self.P, *self.inputs, mode, tf32_wgrad)
-            self._oracle[key] = (stats, grads, extra)
-        return self._oracle[key]
+    def oracle(self, mode):
+        if mode not in self._oracle:
+            stats, newp, _, grads, extra = _oracle_step(self.P, *self.inputs, mode)
+            self._oracle[mode] = (stats, grads, extra)
+        return self._oracle[mode]
 
 
 @pytest.fixture(scope="module")
@@ -207,7 +200,7 @@ def test_train_step_at_baseline_size(rt, full_case, mode):
         du.GRAPH_ENABLED = False
         fc = full_case
         images, labels, fake_labels, z = fc.inputs
-        stats, grads, extra = fc.oracle(mode, _tf32_wgrad_on_tc(rt))
+        stats, grads, extra = fc.oracle(mode)
         G, D, R, _ = build_models(rt, fc.P)
         tol = TOL_OUT[mode]
 
@@ -295,7 +288,7 @@ def test_recognizer_ctc_at_config3_size(rt, mode):
         x = torch.rand(b, 32, 16 * l, 1, generator=g) * 2 - 1
         y = torch.randint(0, classes - 1, (b, l), generator=g)
         leaf = {k: v.clone().requires_grad_(not k.endswith(O.NON_TRAINABLE_SUFFIXES)) for k, v in P.items()}
-        O.set_operand_rounding({"fp32": None, "tf32": "tf32", "bf16": "bf16"}[mode], wgrad=(mode == "bf16" or _tf32_wgrad_on_tc(rt)))
+        O.set_operand_rounding({"fp32": None, "tf32": "tf32", "bf16": "bf16"}[mode])
         try:
             loss = O.recognizer(x, y, torch.full((b, 1), 4 * l - 1), torch.full((b, 1), l), leaf)
             loss.sum().backward()

@@ -143,6 +143,11 @@ def g_isolation(rt, mode, sigma):
     table("G grads", G.store.grad_dict(), {k: v.grad for k, v in leaf.items() if v.requires_grad})
 
 
+def cbn_gb(rt, cbn, z):
+    """(gamma, beta, row stride) of one conditional BN layer from its own Dense layers; z: a block's slice of the latent."""
+    return cbn.gamma.forward(rt, z, z.shape[0], ldx=128), cbn.beta.forward(rt, z, z.shape[0], ldx=128), None
+
+
 def g_stages(rt, mode, sigma=0.0):
     """stage-by-stage forward of G against the (rounded) oracle"""
     rt.set_mode(mode)
@@ -178,7 +183,8 @@ def g_stages(rt, mode, sigma=0.0):
     net, _ = G.embed.forward(rt, zd, 128, yd)
     print("  bank : {:.3e}".format(rel_max(net, exp["bank"])))
     for i, blk in enumerate(G.blocks):
-        net, _ = blk.forward(rt, net, zd[:, 32 * (i + 1):], 128, True)
+        zi = zd[:, 32 * (i + 1):]
+        net, _ = blk.forward(rt, net, True, cbn_gb(rt, blk.cbn1, zi), cbn_gb(rt, blk.cbn2, zi))
         print("  B{}   : {:.3e}".format(i + 1, rel_max(net, exp["B%d" % (i + 1)])))
         if i in G.attn:
             net, _ = G.attn[i].forward(rt, net)
@@ -201,11 +207,11 @@ def g_stages(rt, mode, sigma=0.0):
     finally:
         O.set_operand_rounding(None)
     zi = zd[:, 32:]
-    a1, _ = blk.cbn1.forward(rt, x0, zi, 128, True, True, rt.op_dt)
+    a1, _ = blk.cbn1.forward(rt, x0, cbn_gb(rt, blk.cbn1, zi), True, True, rt.op_dt)
     print("  B1.a1: {:.3e}".format(rel_max(a1.float(), e_a1)))
     u = blk.up.forward(rt, a1)
     print("  B1.u : {:.3e}".format(rel_max(u, e_u)))
-    a2, _ = blk.cbn2.forward(rt, u, zi, 128, True, True, rt.op_dt)
+    a2, _ = blk.cbn2.forward(rt, u, cbn_gb(rt, blk.cbn2, zi), True, True, rt.op_dt)
     print("  B1.a2: {:.3e}".format(rel_max(a2.float(), e_a2)))
     h = blk.conv.forward(rt, a2)
     print("  B1.h : {:.3e}".format(rel_max(h, e_h)))
