@@ -294,6 +294,17 @@ int sg_softmax_rows(sg_ctx* ctx, const float* x, long long rows, int c, float* y
  * log_prob; [TF-SEMANTICS]).  Deterministic.  t_max <= 25600. */
 int sg_ctc_greedy_decode(sg_ctx* ctx, const float* probs, int b, int t_max, int c, const int* input_len,
                          int* decoded, int* decoded_len, float* neg_sum_log);
+/* Replaces K.ctc_decode(greedy=False) / tf.nn.ctc_beam_search_decoder(merge_repeated) with the default scorer: CTC prefix beam
+ * search over frames t < input_len[b] (NULL: all t_max; clamped to [0, t_max]) of x = log-softmax(log(probs + 1e-7))
+ * [TF-SEMANTICS], beam_width in [1, 128] kept prefixes (ties: lower candidate index), 2 <= c <= 128, 1 <= top_paths <=
+ * beam_width.  Path k is the beam of rank k: decoded [top_paths, b, t_max] int32 padded with -1 (merge_repeated: consecutive
+ * equal symbols merged [TF-SEMANTICS]), decoded_len [top_paths, b], log_prob [b, top_paths] = the beam's log probability
+ * (-inf and length 0 beyond the live beams; 0 for the empty word of a sample without frames).  Deterministic.  scratch holds
+ * the back-pointers: at least sg_ctc_beam_decode_scratch_bytes(b, t_max, beam_width) bytes. */
+size_t sg_ctc_beam_decode_scratch_bytes(int b, int t_max, int beam_width);
+int sg_ctc_beam_decode(sg_ctx* ctx, const float* probs, int b, int t_max, int c, const int* input_len, int beam_width,
+                       int top_paths, int merge_repeated, int* decoded, int* decoded_len, float* log_prob, void* scratch,
+                       size_t scratch_bytes);
 /* Replaces tf.edit_distance(normalize=False): exact Levenshtein distance dist[b] between hyp [b, hyp_stride] and
  * ref [b, ref_stride] (int32, ref_stride <= 64).  A NULL length array means the run of leading non-negative entries
  * (sg_label_lengths).  totals (NULL or long long[4], device) is ADDED to: {sum dist, sum ref length, exact matches, samples}. */

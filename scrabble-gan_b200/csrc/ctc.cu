@@ -4,6 +4,8 @@
 // => effective per-frame distribution q = (p + eps) / (1 + C eps), blank = C-1, repeats merged.
 // One CTA per sample; thread s owns extended-label state s (S = 2L+1); log-space alpha/beta in shared memory.
 // dL/du (u = log(p+eps)) = q - occupancy/P  [tf.nn.ctc_loss gradient], chained through log and softmax to z.
+#include <atomic>
+
 #include "common.cuh"
 
 #define CTC_EPS 1e-7f
@@ -378,6 +380,309 @@ extern "C" int sg_edit_distance(sg_ctx* ctx, const int* hyp, const int* hyp_len,
   if (b == 0) return SG_OK;
   sg_launch(ctx, k_edit_distance, sg_div_up(b, EDIT_THREADS / 32), EDIT_THREADS, 0, hyp, hyp_len, hyp_stride, ref, ref_len,
             ref_stride, b, dist, totals);
+  SG_POST_LAUNCH(ctx);
+  return SG_OK;
+}
+
+// ---------------------------------------------------------------------------------------------------
+// CTC prefix beam search (K.ctc_decode(greedy=False) / tf.nn.ctc_beam_search_decoder with the default scorer), one sample
+// per CTA, the beam state in shared memory.
+//   x_t = log-softmax(log(p_t + 1e-7)) over the C classes [TF-SEMANTICS: Keras feeds log(y_pred + 1e-7) to the decoder, which
+//   treats its input as logits], i.e. log((p + eps) / (1 + C eps)) as in k_ctc.
+//   A beam is a prefix: (log P_blank, log P_label), their total, its parent (the kept beam one symbol shorter, or -1) and its
+//   last symbol.  At frame t every kept beam b of rank r offers its continuation (candidate index r C + C - 1) and its
+//   extensions by c < C - 1 (index r C + c) whose prefix is not already kept -- a kept prefix b + c is a kept beam with parent
+//   b and last symbol c, found in a W x C child table.  The beam_width largest totals are kept, ties to the lower index;
+//   candidates of total -inf are never kept.  The selection is a radix select on orderable 64-bit (total, ~index) keys with
+//   8-bit digits (integer histogram counters only), the kept candidates are ranked by counting; fp32 sums in a fixed order,
+//   so the result is bit-reproducible.
+//   Back-pointers (old rank << 8 | emitted symbol or 0xFF) go to the caller's scratch [b, Tmax, W]; path k is the beam of
+//   rank k, read back from the last frame.  merge_repeated merges consecutive equal symbols of the written path [TF-SEMANTICS].
+// dynamic smem: cand[W * C] (float) | child[W * C] (int8)
+// ---------------------------------------------------------------------------------------------------
+#define BEAM_THREADS 256
+#define BEAM_MAX_W 128
+#define BEAM_MAX_C 128
+#define BEAM_NO_SYMBOL 0xFF
+
+__device__ __forceinline__ unsigned long long beam_key(float s, int pos) {
+  const unsigned int u = __float_as_uint(s);
+  const unsigned int ord = (u & 0x80000000u) ? ~u : (u | 0x80000000u);          // larger float -> larger unsigned
+  return ((unsigned long long)ord << 32) | (unsigned long long)(0xFFFFFFFFu - (unsigned int)pos);   // then lower index
+}
+
+__global__ void __launch_bounds__(BEAM_THREADS) k_ctc_beam_decode(const float* __restrict__ probs, int Tmax, int C,
+                                                                  const int* __restrict__ input_len, int W, int top_paths,
+                                                                  int merge_repeated, int* __restrict__ decoded,
+                                                                  int* __restrict__ decoded_len, float* __restrict__ log_prob,
+                                                                  unsigned short* bp) {
+  extern __shared__ float sm[];
+  float* cand = sm;
+  signed char* child = reinterpret_cast<signed char*>(sm + W * C);
+  __shared__ float s_x[BEAM_MAX_C];
+  __shared__ float s_pb[2][BEAM_MAX_W], s_pl[2][BEAM_MAX_W], s_tot[2][BEAM_MAX_W];
+  __shared__ int s_last[2][BEAM_MAX_W], s_par[2][BEAM_MAX_W];
+  __shared__ float s_npb[BEAM_MAX_W], s_npl[BEAM_MAX_W];
+  __shared__ int s_contrank[BEAM_MAX_W], s_sel[BEAM_MAX_W], s_order[BEAM_MAX_W], s_len[BEAM_MAX_W];
+  __shared__ unsigned long long s_selkey[BEAM_MAX_W];
+  __shared__ int s_hist[256];
+  __shared__ int s_nsel, s_digit, s_above, s_count, s_total;
+  const int b = blockIdx.x, tid = threadIdx.x, lane = tid & 31, warp = tid >> 5;
+  int T = input_len ? input_len[b] : Tmax;
+  T = T < 0 ? 0 : (T > Tmax ? Tmax : T);
+  const float* p = probs + (long long)b * Tmax * C;
+  unsigned short* bpb = bp + (long long)b * Tmax * W;
+  const int blank = C - 1;
+
+  for (int i = tid; i < W * C; i += BEAM_THREADS) child[i] = -1;
+  if (tid == 0) {                                     // t = 0: the empty prefix, P_blank = 1, P_label = 0
+    s_pb[0][0] = 0.f; s_pl[0][0] = NEG_INF; s_tot[0][0] = 0.f; s_last[0][0] = -1; s_par[0][0] = -1;
+  }
+  int nb = 1, cur = 0;
+  __syncthreads();
+
+  for (int t = 0; t < T; ++t) {
+    const int nxt = cur ^ 1;
+    if (warp == 0) {                                  // the frame's log-probabilities, one warp (C <= 128)
+      float lp[BEAM_MAX_C / 32];
+      float m = NEG_INF;
+#pragma unroll
+      for (int j = 0; j < BEAM_MAX_C / 32; ++j) {
+        const int k = lane + 32 * j;
+        lp[j] = k < C ? logf(p[(long long)t * C + k] + CTC_EPS) : NEG_INF;
+        m = fmaxf(m, lp[j]);
+      }
+      m = sg_warp_max(m);
+      float s = 0.f;
+#pragma unroll
+      for (int j = 0; j < BEAM_MAX_C / 32; ++j)
+        if (lane + 32 * j < C) s += expf(lp[j] - m);
+      const float ls = logf(sg_warp_sum(s));
+#pragma unroll
+      for (int j = 0; j < BEAM_MAX_C / 32; ++j)
+        if (lane + 32 * j < C) s_x[lane + 32 * j] = (lp[j] - m) - ls;
+    }
+    __syncthreads();
+
+    // candidates: cand[r C + c] = total of the extension of beam r by c, or of r's continuation at c = blank
+    const int n = nb * C;
+    for (int i = tid; i < n; i += BEAM_THREADS) {
+      const int r = i / C, c = i - r * C;
+      float v;
+      if (c == blank) {
+        const int last = s_last[cur][r], par = s_par[cur][r];
+        const float npb = s_tot[cur][r] + s_x[blank];
+        float npl = NEG_INF;
+        if (last >= 0) {
+          const float xl = s_x[last];
+          npl = s_pl[cur][r] + xl;
+          if (par >= 0) {                             // the parent's mass moves into this prefix by emitting `last`
+            const float prev = last == s_last[cur][par] ? s_pb[cur][par] : s_tot[cur][par];
+            npl = lse2(npl, prev + xl);
+          }
+        }
+        s_npb[r] = npb;
+        s_npl[r] = npl;
+        v = lse2(npb, npl);
+      } else if (child[i] >= 0) {
+        v = NEG_INF;                                  // prefix already kept: its continuation accounts for it
+      } else {
+        v = s_x[c] + (c == s_last[cur][r] ? s_pb[cur][r] : s_tot[cur][r]);
+      }
+      cand[i] = v;
+    }
+    __syncthreads();
+
+    // radix select of the W largest keys: digits of the total (4 passes), then of the index (bits 31..16 of ~index are all
+    // ones as n <= 2^14); stops as soon as every key with the chosen prefix is kept.  kept <=> key >= prefix.
+    unsigned long long prefix = 0ull, mask = 0ull;
+    int need = W;
+    bool keep_all = false;
+    for (int pass = 0; pass < 6; ++pass) {
+      const int sh = pass < 4 ? 56 - 8 * pass : 8 * (5 - pass);
+      if (pass == 4) {
+        prefix |= 0xFFFF0000ull;
+        mask |= 0xFFFF0000ull;
+      }
+      for (int i = tid; i < 256; i += BEAM_THREADS) s_hist[i] = 0;
+      __syncthreads();
+      for (int i = tid; i < n; i += BEAM_THREADS) {
+        const float v = cand[i];
+        if (v == NEG_INF) continue;
+        const unsigned long long key = beam_key(v, i);
+        if ((key & mask) == prefix) atomicAdd(&s_hist[(int)((key >> sh) & 0xFFull)], 1);
+      }
+      __syncthreads();
+      if (warp == 0) {                                // lane l owns bins 255 - 8l .. 248 - 8l, scanned from the top
+        int cnt[8], sum = 0;
+#pragma unroll
+        for (int j = 0; j < 8; ++j) {
+          cnt[j] = s_hist[255 - 8 * lane - j];
+          sum += cnt[j];
+        }
+        int inc = sum;
+#pragma unroll
+        for (int o = 1; o < 32; o <<= 1) {
+          const int v = __shfl_up_sync(0xffffffffu, inc, o);
+          if (lane >= o) inc += v;
+        }
+        const int exc = inc - sum;
+        const unsigned int hit = __ballot_sync(0xffffffffu, exc < need && need <= inc);
+        if (hit && lane == __ffs(hit) - 1) {
+          int above = exc, sel = -1, count = 0;
+#pragma unroll
+          for (int j = 0; j < 8; ++j) {               // unrolled: cnt stays in registers
+            if (sel >= 0) continue;
+            if (above + cnt[j] >= need) {
+              sel = j;
+              count = cnt[j];
+            } else {
+              above += cnt[j];
+            }
+          }
+          s_digit = 255 - 8 * lane - sel;
+          s_above = above;
+          s_count = count;
+        }
+        if (lane == 31) s_total = inc;
+      }
+      __syncthreads();
+      if (pass == 0 && s_total <= need) {             // W or fewer live candidates: all kept
+        keep_all = true;
+        break;
+      }
+      need -= s_above;
+      prefix |= (unsigned long long)s_digit << sh;
+      mask |= 0xFFull << sh;
+      if (s_count == need) break;
+    }
+
+    if (tid == 0) s_nsel = 0;
+    __syncthreads();
+    for (int i = tid; i < n; i += BEAM_THREADS) {     // gather (any order: the rank below does not depend on it)
+      const float v = cand[i];
+      if (v == NEG_INF) continue;
+      const unsigned long long key = beam_key(v, i);
+      if (keep_all || key >= prefix) {
+        const int slot = atomicAdd(&s_nsel, 1);
+        s_sel[slot] = i;
+        s_selkey[slot] = key;
+      }
+    }
+    __syncthreads();
+    const int nk = s_nsel;
+    for (int i = tid; i < nk; i += BEAM_THREADS) {    // rank = number of larger keys (keys are distinct)
+      const unsigned long long k = s_selkey[i];
+      int rank = 0;
+      for (int j = 0; j < nk; ++j) rank += s_selkey[j] > k;
+      s_order[rank] = s_sel[i];
+    }
+    for (int i = tid; i < nb; i += BEAM_THREADS) s_contrank[i] = -1;
+    __syncthreads();
+    for (int k = tid; k < nk; k += BEAM_THREADS) {
+      const int pos = s_order[k];
+      if (pos % C == blank) s_contrank[pos / C] = k;  // new rank of old beam r's continuation
+    }
+    for (int j = tid; j < nb; j += BEAM_THREADS)      // forget the old child table
+      if (s_par[cur][j] >= 0) child[s_par[cur][j] * C + s_last[cur][j]] = -1;
+    __syncthreads();
+    for (int k = tid; k < nk; k += BEAM_THREADS) {    // the new beams, in rank order
+      const int pos = s_order[k], r = pos / C, c = pos - r * C;
+      const float v = cand[pos];
+      int par, last;
+      if (c == blank) {
+        const int op = s_par[cur][r];
+        s_pb[nxt][k] = s_npb[r];
+        s_pl[nxt][k] = s_npl[r];
+        last = s_last[cur][r];
+        par = op >= 0 ? s_contrank[op] : -1;
+      } else {
+        s_pb[nxt][k] = NEG_INF;
+        s_pl[nxt][k] = v;
+        last = c;
+        par = s_contrank[r];
+      }
+      s_tot[nxt][k] = v;
+      s_last[nxt][k] = last;
+      s_par[nxt][k] = par;
+      if (par >= 0) child[par * C + last] = (signed char)k;
+      bpb[(long long)t * W + k] = (unsigned short)((r << 8) | (c == blank ? BEAM_NO_SYMBOL : c));
+    }
+    __syncthreads();
+    nb = nk;
+    cur = nxt;
+  }
+
+  // path k = beam of rank k, walked back from the last frame: once to count, once to write
+  for (int k = tid; k < top_paths; k += BEAM_THREADS) {
+    int len = 0;
+    if (k < nb) {
+      int r = k, after = -1;
+      for (int t = T - 1; t >= 0; --t) {
+        const unsigned int e = bpb[(long long)t * W + r];
+        const int sym = (int)(e & 0xFFu);
+        if (sym != BEAM_NO_SYMBOL) {
+          if (!merge_repeated || sym != after) ++len;
+          after = sym;
+        }
+        r = (int)(e >> 8);
+      }
+      int* out = decoded + ((long long)k * gridDim.x + b) * Tmax;
+      int j = len;
+      r = k;
+      after = -1;
+      for (int t = T - 1; t >= 0; --t) {
+        const unsigned int e = bpb[(long long)t * W + r];
+        const int sym = (int)(e & 0xFFu);
+        if (sym != BEAM_NO_SYMBOL) {
+          if (!merge_repeated || sym != after) out[--j] = sym;
+          after = sym;
+        }
+        r = (int)(e >> 8);
+      }
+    }
+    s_len[k] = len;
+    decoded_len[(long long)k * gridDim.x + b] = len;
+    log_prob[(long long)b * top_paths + k] = k < nb ? s_tot[cur][k] : NEG_INF;
+  }
+  __syncthreads();
+  for (int k = 0; k < top_paths; ++k) {
+    int* out = decoded + ((long long)k * gridDim.x + b) * Tmax;
+    for (int i = s_len[k] + tid; i < Tmax; i += BEAM_THREADS) out[i] = -1;
+  }
+}
+
+extern "C" size_t sg_ctc_beam_decode_scratch_bytes(int b, int t_max, int beam_width) {
+  if (b <= 0 || t_max <= 0 || beam_width <= 0) return 0;
+  return (size_t)b * (size_t)t_max * (size_t)beam_width * sizeof(unsigned short);
+}
+
+extern "C" int sg_ctc_beam_decode(sg_ctx* ctx, const float* probs, int b, int t_max, int c, const int* input_len, int beam_width,
+                                  int top_paths, int merge_repeated, int* decoded, int* decoded_len, float* log_prob,
+                                  void* scratch, size_t scratch_bytes) {
+  SG_REQUIRE(ctx && probs && decoded && decoded_len && log_prob, "sg_ctc_beam_decode: NULL");
+  SG_REQUIRE(b >= 0 && t_max >= 1 && c >= 2 && c <= BEAM_MAX_C, "sg_ctc_beam_decode: bad sizes (b %d, t_max %d, c %d <= %d)", b,
+             t_max, c, BEAM_MAX_C);
+  SG_REQUIRE(beam_width >= 1 && beam_width <= BEAM_MAX_W, "sg_ctc_beam_decode: beam_width %d not in [1, %d]", beam_width,
+             BEAM_MAX_W);
+  SG_REQUIRE(top_paths >= 1 && top_paths <= beam_width, "sg_ctc_beam_decode: top_paths %d not in [1, beam_width %d]", top_paths,
+             beam_width);
+  if (b == 0) return SG_OK;
+  const size_t need = sg_ctc_beam_decode_scratch_bytes(b, t_max, beam_width);
+  SG_REQUIRE(scratch && scratch_bytes >= need, "sg_ctc_beam_decode: scratch of %zu bytes for %d x %d back-pointers, got %zu", need,
+             b, t_max, scratch_bytes);
+  const size_t smem = (size_t)beam_width * c * (sizeof(float) + 1);
+  // the kernel's ~11 KB of static shared memory counts against the 48 KB default too: allow the largest dynamic size once per
+  // device (the attribute is a cap, the launch asks for what it uses), not on every launch
+  static std::atomic<unsigned long long> attr_set{0};
+  const unsigned long long bit = ctx->device < 64 ? 1ull << ctx->device : 0ull;     // 0: no cache, set every time
+  if (!bit || !(attr_set.load() & bit)) {
+    SG_CHECK_CUDA(cudaFuncSetAttribute(k_ctc_beam_decode, cudaFuncAttributeMaxDynamicSharedMemorySize,
+                                       (int)((size_t)BEAM_MAX_W * BEAM_MAX_C * (sizeof(float) + 1))));
+    attr_set.fetch_or(bit);
+  }
+  sg_launch(ctx, k_ctc_beam_decode, b, BEAM_THREADS, smem, probs, t_max, c, input_len, beam_width, top_paths, merge_repeated,
+            decoded, decoded_len, log_prob, (unsigned short*)scratch);
   SG_POST_LAUNCH(ctx);
   return SG_OK;
 }

@@ -620,6 +620,20 @@ def ctc_greedy_decode(rt, probs, input_length=None):
     return decoded, dlen, score
 
 
+def ctc_beam_decode(rt, probs, input_length=None, beam_width=100, top_paths=1, merge_repeated=True):
+    """K.ctc_decode(greedy=False) on probs (B, T, C): decoded (top_paths, B, T) int32 padded with -1, decoded_len
+    (top_paths, B) int32, log_prob (B, top_paths) fp32.  input_length: (B,) int32 device tensor or None (all T frames)."""
+    b, t, c = probs.shape
+    decoded = torch.empty((top_paths, b, t), device=rt.device, dtype=torch.int32)
+    dlen = torch.empty((top_paths, b), device=rt.device, dtype=torch.int32)
+    log_prob = rt.empty((b, top_paths), SG_F32)
+    nbytes = _abi.load().sg_ctc_beam_decode_scratch_bytes(b, t, beam_width)
+    scratch = rt.empty(((nbytes + 3) // 4,), SG_F32)            # back-pointers
+    call.sg_ctc_beam_decode(rt.ctx, _p(probs), b, t, c, _p(input_length), int(beam_width), int(top_paths), int(bool(merge_repeated)),
+                            _p(decoded), _p(dlen), _p(log_prob), _p(scratch), nbytes)
+    return decoded, dlen, log_prob
+
+
 def edit_distance(rt, hyp, ref, hyp_length=None, ref_length=None, totals=None):
     """Levenshtein distance (B,) int32 between the rows of hyp (B, Lh) and ref (B, Lr <= 64); without a length tensor a row
     ends at its first negative entry.  totals: int64 (4,) device tensor that is ADDED to (sum dist, sum ref length, exact
