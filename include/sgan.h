@@ -305,6 +305,20 @@ size_t sg_ctc_beam_decode_scratch_bytes(int b, int t_max, int beam_width);
 int sg_ctc_beam_decode(sg_ctx* ctx, const float* probs, int b, int t_max, int c, const int* input_len, int beam_width,
                        int top_paths, int merge_repeated, int* decoded, int* decoded_len, float* log_prob, void* scratch,
                        size_t scratch_bytes);
+/* Replaces K.ctc_batch_cost over every (sample, word) pair of a lexicon: scores [b, v] = log p(lexicon[v] | x_b), minus the
+ * CTC loss of the pair, with x = log-softmax(log(probs + 1e-7)) over frames t < input_len[b] (NULL: all t_max; clamped to
+ * [0, t_max]) [TF-SEMANTICS].  lexicon [v, l_max] int32 padded with -1, lex_len [v] word lengths (clamped to [0, l_max]).
+ * A word that cannot fit in its sample's frames (length + adjacent repeats > frames) or holds a symbol outside [0, c - 1)
+ * scores -inf; over 0 frames the empty word scores 0.  Limits: l_max <= 31, 2 <= c <= 128, t_max * c * 4 <= 200 KB.
+ * Deterministic. */
+int sg_ctc_lexicon_scores(sg_ctx* ctx, const float* probs, int b, int t_max, int c, const int* input_len, const int* lexicon,
+                          const int* lex_len, int v, int l_max, float* scores);
+/* Replaces the arg-max / top-k over the lexicon of those scores: per sample (row of scores [b, v]) the top_paths largest
+ * scores, exact, equal scores to the lower word index, -inf ranked like any other score; 1 <= top_paths <= min(v, 128).
+ * Path k: decoded [top_paths, b, l_max] int32 (the word, padded with -1), decoded_len [top_paths, b], log_prob [b, top_paths]
+ * (its score), index [b, top_paths] (its row in the lexicon).  Deterministic. */
+int sg_ctc_lexicon_topk(sg_ctx* ctx, const float* scores, int b, int v, const int* lexicon, const int* lex_len, int l_max,
+                        int top_paths, int* decoded, int* decoded_len, float* log_prob, int* index);
 /* Replaces tf.edit_distance(normalize=False): exact Levenshtein distance dist[b] between hyp [b, hyp_stride] and
  * ref [b, ref_stride] (int32, ref_stride <= 64).  A NULL length array means the run of leading non-negative entries
  * (sg_label_lengths).  totals (NULL or long long[4], device) is ADDED to: {sum dist, sum ref length, exact matches, samples}. */

@@ -132,6 +132,8 @@ _PROTOS = {
     "sg_ctc_greedy_decode": (_I, [_P, _P, _I, _I, _I, _P, _P, _P, _P]),
     "sg_ctc_beam_decode_scratch_bytes": (_Z, [_I, _I, _I]),
     "sg_ctc_beam_decode": (_I, [_P, _P, _I, _I, _I, _P, _I, _I, _I, _P, _P, _P, _P, _Z]),
+    "sg_ctc_lexicon_scores": (_I, [_P, _P, _I, _I, _I, _P, _P, _P, _I, _I, _P]),
+    "sg_ctc_lexicon_topk": (_I, [_P, _P, _I, _I, _P, _P, _I, _I, _P, _P, _P, _P]),
     "sg_edit_distance": (_I, [_P, _P, _P, _I, _P, _P, _I, _I, _P, _P]),
     "sg_loss_sums": (_I, [_P, _I, _I, _P, _P, _P, _P, _P, _P, _P, _I, _P]),
     "sg_loss_finish": (_I, [_P, _I, _I, _I, _F, _P, _P, _P, _P, _P, _P, _I, _P, _P, _P, _P, _P, _P, _P, _P, _P, _P]),

@@ -686,3 +686,280 @@ extern "C" int sg_ctc_beam_decode(sg_ctx* ctx, const float* probs, int b, int t_
   SG_POST_LAUNCH(ctx);
   return SG_OK;
 }
+
+// ---------------------------------------------------------------------------------------------------
+// Lexicon (closed-vocabulary) decoding: the CTC log-likelihood of every (sample, word) pair, and each sample's best words.
+//   scores[b, v] = log p(lexicon[v] | x_b) with x_t = log-softmax(log(p_t + 1e-7)) over the C classes, as in
+//   k_ctc_beam_decode: minus K.ctc_batch_cost of the pair [TF-SEMANTICS].  Forward (alpha) recursion in the log domain with
+//   lse2 / lse3, no beta and no gradient.  One CTA per (sample, tile of LEX_WORDS words): the sample's frame table x[T_b, C]
+//   is built in shared memory once and read by every word of the tile; one warp per word, extended-label state s on lane s
+//   and lane s - 32, states s - 1 and s - 2 by warp shuffles.  A word that cannot fit in T_b frames (L + adjacent repeats >
+//   T_b) or holds a symbol outside [0, C - 1) scores -inf without running the recursion; with T_b = 0 the empty word
+//   scores 0.  Each score is one warp's fixed sequence of operations: bit-reproducible.
+//   dynamic smem: x[Tmax * C] (float)
+// ---------------------------------------------------------------------------------------------------
+#define LEX_THREADS 256
+#define LEX_WORDS 64
+#define LEX_MAX_L 31
+#define LEX_MAX_C 128
+#define LEX_MAX_TOPK 128
+#define LEX_MAX_SMEM (200 * 1024)
+
+__global__ void __launch_bounds__(LEX_THREADS) k_ctc_lexicon_scores(const float* __restrict__ probs, int Tmax, int C,
+                                                                    const int* __restrict__ input_len,
+                                                                    const int* __restrict__ lexicon,
+                                                                    const int* __restrict__ lex_len, int V, int Lmax,
+                                                                    int tiles, float* __restrict__ scores) {
+  extern __shared__ float x[];
+  const int b = blockIdx.x / tiles, tile = blockIdx.x - b * tiles;
+  const int tid = threadIdx.x, lane = tid & 31, warp = tid >> 5, nwarps = LEX_THREADS / 32;
+  const unsigned int full = 0xffffffffu;
+  int T = input_len ? input_len[b] : Tmax;
+  T = T < 0 ? 0 : (T > Tmax ? Tmax : T);
+  const float* p = probs + (long long)b * Tmax * C;
+  const int blank = C - 1;
+
+  for (int t = warp; t < T; t += nwarps) {            // the frame table, one warp per frame (C <= 128)
+    float lp[LEX_MAX_C / 32];
+    float m = NEG_INF;
+#pragma unroll
+    for (int j = 0; j < LEX_MAX_C / 32; ++j) {
+      const int k = lane + 32 * j;
+      lp[j] = k < C ? logf(p[(long long)t * C + k] + CTC_EPS) : NEG_INF;
+      m = fmaxf(m, lp[j]);
+    }
+    m = sg_warp_max(m);
+    float s = 0.f;
+#pragma unroll
+    for (int j = 0; j < LEX_MAX_C / 32; ++j)
+      if (lane + 32 * j < C) s += expf(lp[j] - m);
+    const float ls = logf(sg_warp_sum(s));
+#pragma unroll
+    for (int j = 0; j < LEX_MAX_C / 32; ++j)
+      if (lane + 32 * j < C) x[t * C + lane + 32 * j] = (lp[j] - m) - ls;
+  }
+  __syncthreads();
+
+  const int v_end = min(V, (tile + 1) * LEX_WORDS);
+  for (int v = tile * LEX_WORDS + warp; v < v_end; v += nwarps) {
+    int L = lex_len[v];
+    L = L < 0 ? 0 : (L > Lmax ? Lmax : L);
+    const int sym = lane < L ? lexicon[(long long)v * Lmax + lane] : blank;      // letter j on lane j (L <= 31)
+    const int before = __shfl_up_sync(full, sym, 1);
+    const unsigned int rep = __ballot_sync(full, lane >= 1 && lane < L && sym == before);
+    const unsigned int bad = __ballot_sync(full, lane < L && (sym < 0 || sym >= blank));
+    float* out = scores + (long long)b * V + v;
+    if (bad || L + __popc(rep) > T) {                 // no alignment: exactly -inf
+      if (lane == 0) *out = NEG_INF;
+      continue;
+    }
+    if (T == 0) {                                     // the empty word (L = 0 here) over no frames
+      if (lane == 0) *out = 0.f;
+      continue;
+    }
+    // state s: blank for even s, letter (s - 1) / 2 for odd s; lane holds s = lane (lo) and s = lane + 32 (hi).  The skip
+    // s - 2 -> s is allowed for a letter that differs from the letter before it: letter j = (s - 1) / 2 >= 1, bit j of rep clear.
+    const int S = 2 * L + 1;
+    const int odd = lane & 1, j_lo = lane >> 1, j_hi = 16 + (lane >> 1);
+    const int l_lo = __shfl_sync(full, sym, j_lo), l_hi = __shfl_sync(full, sym, j_hi);
+    const int e_lo = odd ? l_lo : blank, e_hi = odd ? l_hi : blank;
+    const bool in_lo = lane < S, in_hi = lane + 32 < S;
+    const bool skip_lo = odd && j_lo >= 1 && !((rep >> j_lo) & 1u), skip_hi = odd && !((rep >> j_hi) & 1u);
+    float a_lo = (lane < 2 && in_lo) ? x[e_lo] : NEG_INF, a_hi = NEG_INF;
+    if (S <= 32) {                                    // warp-uniform: words of up to 15 letters use the lo half only
+      for (int t = 1; t < T; ++t) {
+        const float u1 = __shfl_up_sync(full, a_lo, 1), u2 = __shfl_up_sync(full, a_lo, 2);
+        const float v3 = lse3(a_lo, lane >= 1 ? u1 : NEG_INF, skip_lo ? u2 : NEG_INF);
+        a_lo = (in_lo && v3 != NEG_INF) ? v3 + x[t * C + e_lo] : NEG_INF;
+      }
+    } else {
+      for (int t = 1; t < T; ++t) {
+        const float u1 = __shfl_up_sync(full, a_lo, 1), u2 = __shfl_up_sync(full, a_lo, 2);
+        const float h1 = __shfl_up_sync(full, a_hi, 1), h2 = __shfl_up_sync(full, a_hi, 2);
+        const float w1 = __shfl_sync(full, a_lo, 31), w2 = __shfl_sync(full, a_lo, 30 + (lane & 1));   // states 31 and 30/31
+        const float n_lo = lse3(a_lo, lane >= 1 ? u1 : NEG_INF, skip_lo ? u2 : NEG_INF);
+        const float n_hi = lse3(a_hi, lane >= 1 ? h1 : w1, skip_hi ? (lane >= 2 ? h2 : w2) : NEG_INF);
+        const float* xt = x + t * C;
+        a_lo = (in_lo && n_lo != NEG_INF) ? n_lo + xt[e_lo] : NEG_INF;
+        a_hi = (in_hi && n_hi != NEG_INF) ? n_hi + xt[e_hi] : NEG_INF;
+      }
+    }
+    // log p = lse2(alpha[S - 1], alpha[S - 2]) at the last frame, in k_ctc's order
+    const int s1 = S - 1, s2 = S - 2 < 0 ? 0 : S - 2;
+    const float f1 = __shfl_sync(full, s1 < 32 ? a_lo : a_hi, s1 & 31);
+    const float f2 = __shfl_sync(full, s2 < 32 ? a_lo : a_hi, s2 & 31);
+    if (lane == 0) *out = lse2(f1, S >= 2 ? f2 : NEG_INF);
+  }
+}
+
+// Top-k words of every sample, one CTA per row of V scores: radix select of the k largest orderable 32-bit keys (four 8-bit
+// digits, integer histogram counters in shared memory, warp-aggregated), then the keys above the threshold and the first
+// tied keys in index order are compacted with a block scan, and the <= 128 survivors are ranked by counting.  Equal scores go
+// to the lower word index; -inf is ranked like any other score (-0 and +0 are equal).  The chosen words are gathered from
+// the lexicon in the same launch.
+__device__ __forceinline__ unsigned int lex_key(float s) {
+  const unsigned int u = __float_as_uint(s == 0.f ? 0.f : s);
+  return (u & 0x80000000u) ? ~u : (u | 0x80000000u);        // larger float -> larger unsigned
+}
+
+__global__ void __launch_bounds__(LEX_THREADS) k_ctc_lexicon_topk(const float* __restrict__ scores, int V,
+                                                                  const int* __restrict__ lexicon,
+                                                                  const int* __restrict__ lex_len, int Lmax, int K,
+                                                                  int* __restrict__ decoded, int* __restrict__ decoded_len,
+                                                                  float* __restrict__ log_prob, int* __restrict__ index) {
+  __shared__ int s_hist[256];
+  __shared__ int s_digit, s_above, s_count;
+  __shared__ int s_wcnt[2][LEX_THREADS / 32];
+  __shared__ unsigned int s_key[LEX_MAX_TOPK];
+  __shared__ int s_idx[LEX_MAX_TOPK], s_order[LEX_MAX_TOPK];
+  const int b = blockIdx.x, tid = threadIdx.x, lane = tid & 31, warp = tid >> 5, nwarps = LEX_THREADS / 32;
+  const unsigned int full = 0xffffffffu, below = (1u << lane) - 1u;
+  const float* row = scores + (long long)b * V;
+
+  // the K-th largest key: after pass p its top 8(p + 1) bits are `prefix`; need = how many keys with that prefix are kept
+  unsigned int prefix = 0u, mask = 0u;
+  int need = K;
+  for (int pass = 0; pass < 4; ++pass) {
+    const int sh = 24 - 8 * pass;
+    for (int i = tid; i < 256; i += LEX_THREADS) s_hist[i] = 0;
+    __syncthreads();
+    for (int i0 = 0; i0 < V; i0 += LEX_THREADS) {
+      const int i = i0 + tid;
+      const unsigned int key = i < V ? lex_key(row[i]) : 0u;
+      const int bin = (i < V && (key & mask) == prefix) ? (int)((key >> sh) & 0xFFu) : 256;
+      const unsigned int peers = __match_any_sync(full, bin);
+      if (bin < 256 && lane == __ffs(peers) - 1) atomicAdd(&s_hist[bin], __popc(peers));
+    }
+    __syncthreads();
+    if (warp == 0) {                                  // lane l owns bins 255 - 8l .. 248 - 8l, scanned from the top
+      int cnt[8], sum = 0;
+#pragma unroll
+      for (int j = 0; j < 8; ++j) {
+        cnt[j] = s_hist[255 - 8 * lane - j];
+        sum += cnt[j];
+      }
+      int inc = sum;
+#pragma unroll
+      for (int o = 1; o < 32; o <<= 1) {
+        const int v = __shfl_up_sync(full, inc, o);
+        if (lane >= o) inc += v;
+      }
+      const int exc = inc - sum;
+      const unsigned int hit = __ballot_sync(full, exc < need && need <= inc);
+      if (hit && lane == __ffs(hit) - 1) {
+        int above = exc, sel = -1, count = 0;
+#pragma unroll
+        for (int j = 0; j < 8; ++j) {
+          if (sel >= 0) continue;
+          if (above + cnt[j] >= need) {
+            sel = j;
+            count = cnt[j];
+          } else {
+            above += cnt[j];
+          }
+        }
+        s_digit = 255 - 8 * lane - sel;
+        s_above = above;
+        s_count = count;
+      }
+    }
+    __syncthreads();
+    need -= s_above;
+    prefix |= (unsigned int)s_digit << sh;
+    mask |= 0xFFu << sh;
+    if (s_count == need) break;                       // every key with this prefix is kept
+  }
+
+  // compaction in index order: keys whose prefix is above, and the first `need` keys with the prefix
+  int base_eq = 0, base_sel = 0;
+  for (int i0 = 0; i0 < V && base_sel < K; i0 += LEX_THREADS) {
+    const int i = i0 + tid;
+    const unsigned int key = i < V ? lex_key(row[i]) : 0u;
+    const bool gt = i < V && (key & mask) > prefix, eq = i < V && (key & mask) == prefix;
+    const unsigned int beq = __ballot_sync(full, eq);
+    if (lane == 0) s_wcnt[0][warp] = __popc(beq);
+    __syncthreads();
+    int eq_before = base_eq + __popc(beq & below), eq_chunk = 0;
+    for (int w = 0; w < nwarps; ++w) {
+      if (w < warp) eq_before += s_wcnt[0][w];
+      eq_chunk += s_wcnt[0][w];
+    }
+    const bool take = gt || (eq && eq_before < need);
+    const unsigned int bt = __ballot_sync(full, take);
+    if (lane == 0) s_wcnt[1][warp] = __popc(bt);
+    __syncthreads();
+    int off = base_sel + __popc(bt & below), chunk = 0;
+    for (int w = 0; w < nwarps; ++w) {
+      if (w < warp) off += s_wcnt[1][w];
+      chunk += s_wcnt[1][w];
+    }
+    if (take) {
+      s_key[off] = key;
+      s_idx[off] = i;
+    }
+    base_eq += eq_chunk;
+    base_sel += chunk;
+    __syncthreads();                                  // s_wcnt is rewritten by the next chunk
+  }
+  for (int k = tid; k < K; k += LEX_THREADS) {        // rank = larger keys + equal keys of lower index (kept in index order)
+    const unsigned int key = s_key[k];
+    int rank = 0;
+    for (int j = 0; j < K; ++j) rank += s_key[j] > key || (s_key[j] == key && j < k);
+    s_order[rank] = k;
+  }
+  __syncthreads();
+  for (int k = warp; k < K; k += nwarps) {            // path k: one warp gathers the word
+    const int v = s_idx[s_order[k]];
+    int L = lex_len[v];
+    L = L < 0 ? 0 : (L > Lmax ? Lmax : L);
+    const long long o = (long long)k * gridDim.x + b;
+    int* out = decoded + o * Lmax;
+    for (int i = lane; i < Lmax; i += 32) out[i] = i < L ? lexicon[(long long)v * Lmax + i] : -1;
+    if (lane == 0) {
+      decoded_len[o] = L;
+      log_prob[(long long)b * K + k] = row[v];
+      index[(long long)b * K + k] = v;
+    }
+  }
+}
+
+extern "C" int sg_ctc_lexicon_scores(sg_ctx* ctx, const float* probs, int b, int t_max, int c, const int* input_len,
+                                     const int* lexicon, const int* lex_len, int v, int l_max, float* scores) {
+  SG_REQUIRE(ctx, "sg_ctc_lexicon_scores: NULL context");
+  SG_REQUIRE(b >= 0 && t_max >= 1 && v >= 0, "sg_ctc_lexicon_scores: bad sizes (b %d, t_max %d, v %d)", b, t_max, v);
+  SG_REQUIRE(c >= 2 && c <= LEX_MAX_C, "sg_ctc_lexicon_scores: c %d not in [2, %d]", c, LEX_MAX_C);
+  SG_REQUIRE(l_max >= 0 && l_max <= LEX_MAX_L, "sg_ctc_lexicon_scores: words of up to %d symbols (got rows of %d)", LEX_MAX_L,
+             l_max);
+  const size_t smem = (size_t)t_max * c * sizeof(float);
+  SG_REQUIRE(smem <= LEX_MAX_SMEM, "sg_ctc_lexicon_scores: t_max %d x c %d frame table (%zu bytes) exceeds %d bytes of shared "
+             "memory", t_max, c, smem, LEX_MAX_SMEM);
+  if (b == 0 || v == 0) return SG_OK;                            // nothing to read or write
+  SG_REQUIRE(probs && lex_len && scores && (lexicon || l_max == 0), "sg_ctc_lexicon_scores: NULL");
+  const long long tiles = (v + LEX_WORDS - 1) / LEX_WORDS;
+  SG_REQUIRE((long long)b * tiles <= 0x7fffffffLL, "sg_ctc_lexicon_scores: %d samples x %lld word tiles", b, tiles);
+  static std::atomic<unsigned long long> attr_set{0};           // allow the largest frame table once per device
+  const unsigned long long bit = ctx->device < 64 ? 1ull << ctx->device : 0ull;
+  if (!bit || !(attr_set.load() & bit)) {
+    SG_CHECK_CUDA(cudaFuncSetAttribute(k_ctc_lexicon_scores, cudaFuncAttributeMaxDynamicSharedMemorySize, LEX_MAX_SMEM));
+    attr_set.fetch_or(bit);
+  }
+  sg_launch(ctx, k_ctc_lexicon_scores, (unsigned int)(b * tiles), LEX_THREADS, smem, probs, t_max, c, input_len, lexicon, lex_len,
+            v, l_max, (int)tiles, scores);
+  SG_POST_LAUNCH(ctx);
+  return SG_OK;
+}
+
+extern "C" int sg_ctc_lexicon_topk(sg_ctx* ctx, const float* scores, int b, int v, const int* lexicon, const int* lex_len,
+                                   int l_max, int top_paths, int* decoded, int* decoded_len, float* log_prob, int* index) {
+  SG_REQUIRE(ctx, "sg_ctc_lexicon_topk: NULL context");
+  SG_REQUIRE(b >= 0 && v >= 0 && l_max >= 0, "sg_ctc_lexicon_topk: bad sizes (b %d, v %d, l_max %d)", b, v, l_max);
+  SG_REQUIRE(top_paths >= 1 && top_paths <= v && top_paths <= LEX_MAX_TOPK,
+             "sg_ctc_lexicon_topk: top_paths %d not in [1, min(v %d, %d)]", top_paths, v, LEX_MAX_TOPK);
+  if (b == 0) return SG_OK;
+  SG_REQUIRE(scores && lex_len && decoded_len && log_prob && index && (l_max == 0 || (lexicon && decoded)),
+             "sg_ctc_lexicon_topk: NULL");
+  sg_launch(ctx, k_ctc_lexicon_topk, b, LEX_THREADS, 0, scores, v, lexicon, lex_len, l_max, top_paths, decoded, decoded_len,
+            log_prob, index);
+  SG_POST_LAUNCH(ctx);
+  return SG_OK;
+}

@@ -1,16 +1,18 @@
-"""Reading words back with the recogniser: greedy and beam-search CTC decoding, edit distance, and the character error rate
-(CER) / word accuracy of R on real word images or on the generator's own words.
+"""Reading words back with the recogniser: greedy, beam-search and lexicon CTC decoding, edit distance, and the character
+error rate (CER) / word accuracy of R on real word images or on the generator's own words.
 
 Conventions (those of the CTC loss, csrc/ctc.cu): the blank is the LAST class (C - 1); decoded words and label matrices are
 int32 rows padded with -1 on the right; the decoding score is Keras' log_prob, the NEGATIVE sum over frames of
 log(max_c p + 1e-7) [TF-SEMANTICS: K.ctc_decode feeds log(y_pred + 1e-7) to tf.nn.ctc_greedy_decoder, whose score is the
 negated sum of the per-frame maxima].  The beam decoder's log_prob is the log probability of the decoded beam (prefix
-beam search, csrc/ctc.cu k_ctc_beam_decode).
+beam search, csrc/ctc.cu k_ctc_beam_decode).  The lexicon decoder reads every image as the word of a closed vocabulary with
+the highest CTC likelihood; its log_prob is that likelihood, minus K.ctc_batch_cost of the pair (k_ctc_lexicon_scores).
 
 The probabilities, argmax, decoding and distances are libsgan kernels; torch only allocates and copies.  There is no host
 fallback: without a GPU every call raises SganError."""
 from __future__ import annotations
 
+import numpy as np
 import torch
 
 from . import ops
@@ -46,6 +48,73 @@ def ctc_beam_decode(y_pred, input_length, beam_width=100, top_paths=1, merge_rep
     return list(decoded.unbind(0)), log_prob
 
 
+MAX_LEXICON_WORD = 31            # letters per lexicon word: the extended label of a word fits one warp (csrc/ctc.cu)
+
+
+def encode_words(words, char_vector=None):
+    """Host helper: a lexicon as the (V, Lmax) int32 matrix of class indices padded with -1 that the lexicon decoder takes,
+    Lmax = the longest word (at least 1).  words: strings, mapped through char_vector (class i = char_vector[i]), or
+    sequences of int class indices such as the words of `random_words` (flattened over its buckets).  Raises ValueError on
+    a character or index outside char_vector (any negative index), on a string without char_vector, and on a word longer
+    than 31 letters."""
+    index = None if char_vector is None else {ch: i for i, ch in enumerate(char_vector)}
+    rows = []
+    for w in words:
+        if isinstance(w, str):
+            if index is None:
+                raise ValueError("encode_words: the string {!r} needs a char_vector".format(w))
+            unknown = [ch for ch in w if ch not in index]
+            if unknown:
+                raise ValueError("encode_words: {!r} has characters outside char_vector: {!r}".format(w, "".join(unknown)))
+            row = [index[ch] for ch in w]
+        else:
+            row = [int(c) for c in (w.tolist() if hasattr(w, "tolist") else w)]
+            bad = [c for c in row if c < 0 or (char_vector is not None and c >= len(char_vector))]
+            if bad:
+                raise ValueError("encode_words: {} has class indices outside char_vector: {}".format(row, bad))
+        if len(row) > MAX_LEXICON_WORD:
+            raise ValueError("encode_words: {!r} has {} letters; lexicon words have at most {}".format(w, len(row),
+                                                                                                     MAX_LEXICON_WORD))
+        rows.append(row)
+    out = np.full((len(rows), max([1] + [len(r) for r in rows])), -1, np.int32)
+    for i, r in enumerate(rows):
+        out[i, :len(r)] = r
+    return out
+
+
+def _lexicon(rt, lexicon):
+    """The lexicon matrix on the device and its word lengths (ops.label_lengths: the run of leading entries >= 0)."""
+    lex = to_device_i32(rt, lexicon)
+    return lex, ops.label_lengths(rt, lex)
+
+
+def ctc_lexicon_scores(y_pred, input_length, lexicon):
+    """log p(word | image) of every (sample, lexicon word) pair, i.e. -K.ctc_batch_cost of the pair, without building the
+    replicated batch: (B, V) fp32 on the device.  y_pred: (B, T, C) softmax probabilities (C <= 128, T * C <= 51 200);
+    input_length: (B,) frames per sample or None for all T; lexicon: (V, Lmax <= 31) int32 padded with -1 (encode_words).
+    A word that cannot fit in a sample's frames scores -inf.  The scores give posteriors over the lexicon, or can be
+    combined with word priors; ops.ctc_lexicon_topk ranks any such (B, V) rows."""
+    rt = get_runtime()
+    probs = to_device_f32(rt, y_pred)
+    il = None if input_length is None else to_device_i32(rt, input_length).reshape(-1)
+    lex, lens = _lexicon(rt, lexicon)
+    return ops.ctc_lexicon_scores(rt, probs, il, lex, lens)
+
+
+def ctc_lexicon_decode(y_pred, input_length, lexicon, top_paths=1):
+    """Closed-vocabulary decoding: every sample reads as the lexicon words of highest CTC likelihood.  Arguments as in
+    ctc_lexicon_scores; 1 <= top_paths <= min(V, 128).  Returns ([decoded_0, ..., decoded_{top_paths-1}], log_prob, index):
+    decoded_k (B, Lmax) int32 on the device, the k-th best word padded with -1; log_prob (B, top_paths) fp32, its score;
+    index (B, top_paths) int32, its row in the lexicon.  Equal scores go to the lower row."""
+    rt = get_runtime()
+    probs = to_device_f32(rt, y_pred)
+    il = None if input_length is None else to_device_i32(rt, input_length).reshape(-1)
+    lex, lens = _lexicon(rt, lexicon)
+    decoded, _, log_prob, index = ops.ctc_lexicon_topk(rt, ops.ctc_lexicon_scores(rt, probs, il, lex, lens), lex, lens,
+                                                       top_paths)
+    return list(decoded.unbind(0)), log_prob, index
+
+
 def edit_distance(hyp, ref, hyp_length=None, ref_length=None):
     """Levenshtein distance between the rows of hyp (B, Lh) and ref (B, Lr <= 64), int32 (B,) on the device
     (tf.edit_distance with normalize=False).  Without a length, a row ends at its first negative entry."""
@@ -56,11 +125,15 @@ def edit_distance(hyp, ref, hyp_length=None, ref_length=None):
     return ops.edit_distance(rt, h, r, hl, rl)
 
 
-def _read(rt, recognizer, images, labels, input_length, label_length, totals, beam_width=None):
-    """R's reading of a batch (greedy, or path 0 of a beam search of beam_width), its distances to the labels added to the
-    device totals; returns the decoded words."""
+def _read(rt, recognizer, images, labels, input_length, label_length, totals, beam_width=None, lexicon=None):
+    """R's reading of a batch (greedy, path 0 of a beam search of beam_width, or the best word of `lexicon` = (matrix,
+    lengths) on the device), its distances to the labels added to the device totals; returns the decoded words."""
     probs = recognizer.frame_probs(images)
-    if beam_width is None:
+    if lexicon is not None:
+        lex, lens = lexicon
+        decoded, dlen, _, _ = ops.ctc_lexicon_topk(rt, ops.ctc_lexicon_scores(rt, probs, input_length, lex, lens), lex, lens)
+        decoded, dlen = decoded[0], dlen[0]
+    elif beam_width is None:
         decoded, dlen, _ = ops.ctc_greedy_decode(rt, probs, input_length)
     else:
         decoded, dlen, _ = ops.ctc_beam_decode(rt, probs, input_length, beam_width)
@@ -75,26 +148,36 @@ def _scores(totals) -> dict:
             "words": words, "chars": chars}
 
 
-def evaluate_recognizer(recognizer, batches, beam_width=None) -> dict:
+def _check_reader(beam_width, lexicon):
+    if lexicon is not None and beam_width is not None:
+        raise ValueError("pass either beam_width (open-vocabulary beam search) or lexicon (closed vocabulary), not both")
+
+
+def evaluate_recognizer(recognizer, batches, beam_width=None, lexicon=None) -> dict:
     """CER (sum of edit distances / sum of reference lengths) and word accuracy of R over `batches`, which yields
     (images, labels) like load_prepare_data -- one length bucket per batch, T = W/4 - 1 frames -- or ragged
     (images, labels, input_length, label_length).  The totals stay on the device: one device-to-host copy at the end.
-    beam_width: None reads greedily; an integer reads path 0 of a beam search that wide.
-    Returns {"cer", "word_accuracy", "words", "chars"}."""
+    beam_width: None reads greedily; an integer reads path 0 of a beam search that wide.  lexicon: a (V, Lmax <= 31) word
+    matrix padded with -1 (encode_words): every image reads as its most likely lexicon word (closed vocabulary); it
+    excludes beam_width.  Returns {"cer", "word_accuracy", "words", "chars"}."""
+    _check_reader(beam_width, lexicon)
     rt = recognizer.rt
+    lex = None if lexicon is None else _lexicon(rt, lexicon)
     totals = torch.zeros(4, device=rt.device, dtype=torch.int64)
     for batch in batches:
         images, labels = batch[0], batch[1]
         il = to_device_i32(rt, batch[2]).reshape(-1) if len(batch) > 2 and batch[2] is not None else None
         ll = to_device_i32(rt, batch[3]).reshape(-1) if len(batch) > 3 and batch[3] is not None else None
-        _read(rt, recognizer, images, to_device_i32(rt, labels), il, ll, totals, beam_width)
+        _read(rt, recognizer, images, to_device_i32(rt, labels), il, ll, totals, beam_width, lex)
     return _scores(totals)
 
 
-def evaluate_generated_words(generator, recognizer, labels, noise=None, beam_width=None) -> dict:
+def evaluate_generated_words(generator, recognizer, labels, noise=None, beam_width=None, lexicon=None) -> dict:
     """Generate the words `labels` ((B, L_max) padded with -1) in ONE ragged inference call of G, and let R read them back
     with input_length = 4 len - 1 (the reference R's interface).  noise: z (B, latent_dim), or None to draw it with
-    ops.random_.  beam_width as in evaluate_recognizer.  Returns evaluate_recognizer's dict plus "decoded", R's words (B, 4 L_max - 1) int32 padded with -1."""
+    ops.random_.  beam_width and lexicon as in evaluate_recognizer.  Returns evaluate_recognizer's dict plus "decoded", R's
+    words (B, 4 L_max - 1) int32 padded with -1 -- (B, Lmax) of the lexicon with a lexicon."""
+    _check_reader(beam_width, lexicon)
     rt = generator.rt
     y = to_device_i32(rt, labels)
     if noise is None:
@@ -106,7 +189,8 @@ def evaluate_generated_words(generator, recognizer, labels, noise=None, beam_wid
     images = generator([z, y], training=False, ragged=True)
     lens = ops.label_lengths(rt, y)
     totals = torch.zeros(4, device=rt.device, dtype=torch.int64)
-    decoded = _read(rt, recognizer, images, y, 4 * lens - 1, lens, totals, beam_width)
+    lex = None if lexicon is None else _lexicon(rt, lexicon)
+    decoded = _read(rt, recognizer, images, y, 4 * lens - 1, lens, totals, beam_width, lex)
     out = _scores(totals)
     out["decoded"] = decoded
     return out

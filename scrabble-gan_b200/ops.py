@@ -634,6 +634,31 @@ def ctc_beam_decode(rt, probs, input_length=None, beam_width=100, top_paths=1, m
     return decoded, dlen, log_prob
 
 
+def ctc_lexicon_scores(rt, probs, input_length, lexicon, lexicon_length):
+    """-K.ctc_batch_cost of every (sample, word) pair: scores (B, V) fp32 = log p(lexicon[v] | probs[b]).  probs (B, T, C),
+    input_length (B,) int32 device tensor or None (all T frames), lexicon (V, Lmax <= 31) int32 padded with -1,
+    lexicon_length (V,) int32."""
+    b, t, c = probs.shape
+    v, l = lexicon.shape
+    scores = rt.empty((b, v), SG_F32)
+    call.sg_ctc_lexicon_scores(rt.ctx, _p(probs), b, t, c, _p(input_length), _p(lexicon), _p(lexicon_length), v, l, _p(scores))
+    return scores
+
+
+def ctc_lexicon_topk(rt, scores, lexicon, lexicon_length, top_paths=1):
+    """The top_paths best words of every row of scores (B, V), ties to the lower index: decoded (top_paths, B, Lmax) int32
+    padded with -1, decoded_len (top_paths, B) int32, log_prob (B, top_paths) fp32, index (B, top_paths) int32."""
+    b, v = scores.shape
+    l = lexicon.shape[1]
+    decoded = torch.empty((top_paths, b, l), device=rt.device, dtype=torch.int32)
+    dlen = torch.empty((top_paths, b), device=rt.device, dtype=torch.int32)
+    log_prob = rt.empty((b, top_paths), SG_F32)
+    index = torch.empty((b, top_paths), device=rt.device, dtype=torch.int32)
+    call.sg_ctc_lexicon_topk(rt.ctx, _p(scores), b, v, _p(lexicon), _p(lexicon_length), l, int(top_paths), _p(decoded), _p(dlen),
+                             _p(log_prob), _p(index))
+    return decoded, dlen, log_prob, index
+
+
 def edit_distance(rt, hyp, ref, hyp_length=None, ref_length=None, totals=None):
     """Levenshtein distance (B,) int32 between the rows of hyp (B, Lh) and ref (B, Lr <= 64); without a length tensor a row
     ends at its first negative entry.  totals: int64 (4,) device tensor that is ADDED to (sum dist, sum ref length, exact
