@@ -325,6 +325,19 @@ int sg_ctc_lexicon_topk(sg_ctx* ctx, const float* scores, int b, int v, const in
 int sg_edit_distance(sg_ctx* ctx, const int* hyp, const int* hyp_len, int hyp_stride, const int* ref, const int* ref_len,
                      int ref_stride, int b, int* dist, long long* totals);
 
+/* ---- word augmentation for training R on its own -- replaces nothing in the reference: the HTR augmentation of the paper's
+ * HTR experiments (random affine warp + thin / thick strokes).  src, dst [n, h, w] fp32 (NHWC, C = 1), out of place; h = 32.
+ * widths [n] (NULL: all w) = each word's columns; dst columns >= widths[b] are copied from src bit for bit.  u [n, 7] in
+ * [-1, 1) (sg_random, normal = 0) sets word b's parameters: rotation u0 * rot_deg degrees, horizontal shear u1 * shear,
+ * scales 1 + u2 * scale and 1 + u3 * scale, translation (u4, u5) * translate_px; a 3x3 grey minimum if u6 < -1 + 2 p_morph,
+ * a 3x3 grey maximum if u6 > 1 - 2 p_morph.  The inverse map about the word's centre (widths[b] / 2, h / 2) is sampled
+ * bilinearly, coordinates clamped to the word (border replicate); the min / max leaves neighbours outside the word out.
+ * Ranges >= 0, scale < 1, p_morph <= 0.5; all ranges zero copy src bit for bit.  widths live in device memory, where the
+ * entry point cannot read them without a synchronisation: a width outside [1, w] makes that word's output NaN.  Draws no
+ * random numbers; deterministic. */
+int sg_word_augment(sg_ctx* ctx, const float* src, float* dst, int n, int h, int w, const int* widths, const float* u,
+                    float rot_deg, float shear, float scale, float translate_px, float p_morph);
+
 /* ---- GAN losses + gradient balancing (K16, K17) -- net_loss.py:4-54; data_utils.py:418-442,476-490 --
  * sums is double[SG_LOSS_NSUMS]; all-reduce it across replicas between the two calls. */
 #define SG_LOSS_NSUMS 16

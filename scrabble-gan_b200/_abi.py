@@ -134,6 +134,7 @@ _PROTOS = {
     "sg_ctc_beam_decode": (_I, [_P, _P, _I, _I, _I, _P, _I, _I, _I, _P, _P, _P, _P, _Z]),
     "sg_ctc_lexicon_scores": (_I, [_P, _P, _I, _I, _I, _P, _P, _P, _I, _I, _P]),
     "sg_ctc_lexicon_topk": (_I, [_P, _P, _I, _I, _P, _P, _I, _I, _P, _P, _P, _P]),
+    "sg_word_augment": (_I, [_P, _P, _P, _I, _I, _I, _P, _P, _F, _F, _F, _F, _F]),
     "sg_edit_distance": (_I, [_P, _P, _P, _I, _P, _P, _I, _I, _P, _P]),
     "sg_loss_sums": (_I, [_P, _I, _I, _P, _P, _P, _P, _P, _P, _P, _I, _P]),
     "sg_loss_finish": (_I, [_P, _I, _I, _I, _F, _P, _P, _P, _P, _P, _P, _I, _P, _P, _P, _P, _P, _P, _P, _P, _P, _P]),

@@ -14,7 +14,7 @@ HERE = os.path.dirname(os.path.abspath(__file__))
 CSRC = os.path.join(HERE, "csrc")
 BUILD = os.path.join(HERE, "csrc", "build")
 LIB = os.path.join(HERE, "libsgan.so")
-SOURCES = ["ctx.cu", "ew.cu", "bn.cu", "gemm.cu", "filterbank.cu", "attention.cu", "attention_tc.cu", "nonlocal.cu", "ctc.cu", "loss.cu", "optim.cu", "peer.cu",
+SOURCES = ["ctx.cu", "ew.cu", "bn.cu", "gemm.cu", "filterbank.cu", "attention.cu", "attention_tc.cu", "nonlocal.cu", "ctc.cu", "augment.cu", "loss.cu", "optim.cu", "peer.cu",
            "conv_simt.cu", "conv_tc.cu"]
 NVCC_FLAGS = ["-gencode", "arch=compute_100a,code=sm_100a", "-lineinfo", "-O3", "-std=c++17", "-Xcompiler", "-fPIC"]
 

@@ -670,6 +670,24 @@ def edit_distance(rt, hyp, ref, hyp_length=None, ref_length=None, totals=None):
     return dist
 
 
+def word_augment(rt, x, u, widths=None, rotation=0.0, shear=0.0, scale=0.0, translate=0.0, p_morph=0.0, out=None):
+    """sg_word_augment: x (n, 32, w[, 1]) fp32 word images -> augmented copy (same shape).  u (n, 7) fp32 in [-1, 1): each word's
+    parameters (rotation u0 * rotation degrees, shear u1 * shear, scales 1 + u2 / u3 * scale, translation u4 / u5 * translate
+    pixels, 3x3 min / max by u6 against p_morph).  widths: (n,) int32 device tensor of word columns, or None for all w."""
+    if x.dim() not in (3, 4) or (x.dim() == 4 and x.shape[3] != 1) or x.dtype != torch.float32 or not x.is_contiguous():
+        raise _abi.SganError("word_augment: x must be contiguous fp32 (n, h, w[, 1]), got {} {}".format(tuple(x.shape), x.dtype))
+    n, h, w = x.shape[0], x.shape[1], x.shape[2]
+    if tuple(u.shape) != (n, 7) or u.dtype != torch.float32 or not u.is_contiguous():
+        raise _abi.SganError("word_augment: u must be contiguous fp32 ({}, 7), got {} {}".format(n, tuple(u.shape), u.dtype))
+    if widths is not None and (tuple(widths.shape) != (n,) or widths.dtype != torch.int32):
+        raise _abi.SganError("word_augment: widths must be int32 ({},), got {} {}".format(n, tuple(widths.shape), widths.dtype))
+    if out is None:
+        out = rt.empty(x.shape, SG_F32)
+    call.sg_word_augment(rt.ctx, _p(x), _p(out), n, h, w, _p(widths), _p(u), float(rotation), float(shear), float(scale),
+                         float(translate), float(p_morph))
+    return out
+
+
 def random_(rt, out, normal: bool = True, seed: Optional[int] = None):
     """Fill `out` (fp32) with N(0,1) (or U[-1,1)) numbers from the runtime's Philox stream; the stream position lives on the
     device (rt.rng_state), so the launch can be captured in a CUDA graph and still draw fresh numbers on every replay."""
