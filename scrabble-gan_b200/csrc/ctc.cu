@@ -26,6 +26,25 @@ __device__ __forceinline__ float lse3(float a, float b, float c) {
   return m + log1pf(s);
 }
 
+// frame count of sample b: input_len[b] (all Tmax frames without input_len) clamped to [lo, Tmax]
+static __device__ __forceinline__ int sample_frames(const int* input_len, int b, int lo, int Tmax) {
+  const int T = input_len ? input_len[b] : Tmax;
+  return T < lo ? lo : (T > Tmax ? Tmax : T);
+}
+
+// softmax of one row z[0, C), one warp: max-subtracted exp and an fp32 sum; store(k, p_k) for every class
+template <class Store>
+static __device__ __forceinline__ void warp_softmax_row(const float* z, int C, int lane, Store store) {
+  float mx = NEG_INF;
+  for (int k = lane; k < C; k += 32) mx = fmaxf(mx, z[k]);
+  mx = sg_warp_max(mx);
+  float sum = 0.f;
+  for (int k = lane; k < C; k += 32) sum += expf(z[k] - mx);
+  sum = sg_warp_sum(sum);
+  const float inv = 1.f / sum;
+  for (int k = lane; k < C; k += 32) store(k, expf(z[k] - mx) * inv);
+}
+
 // dynamic smem: logq[T*C] | alpha[T*S] | beta[T*S] | occ[C] | ext[S] (int)
 // Ragged batches (K.ctc_batch_cost's own interface: per-sample input_length / label_length, net_architecture.py:57-72):
 // input_len / label_len, when given, hold every sample's frame count T_b <= Tmax and label count L_b <= Lmax; logits / labels
@@ -35,8 +54,8 @@ __global__ void k_ctc(const float* __restrict__ logits, const int* __restrict__ 
                       float* __restrict__ grad) {
   extern __shared__ float sm[];
   const int b = blockIdx.x;
-  int T = input_len ? input_len[b] : Tmax, L = label_len ? label_len[b] : Lmax;
-  T = T < 1 ? 1 : (T > Tmax ? Tmax : T);
+  const int T = sample_frames(input_len, b, 1, Tmax);
+  int L = label_len ? label_len[b] : Lmax;
   L = L < 0 ? 0 : (L > Lmax ? Lmax : L);
   const int S = 2 * L + 1, Smax = 2 * Lmax + 1;
   float* logq = sm;
@@ -54,19 +73,8 @@ __global__ void k_ctc(const float* __restrict__ logits, const int* __restrict__ 
 
   // per-frame effective log-probabilities: one warp per frame
   const float log_norm = logf(1.f + (float)C * CTC_EPS);
-  for (int t = warp; t < T; t += nwarps) {
-    float mx = NEG_INF;
-    for (int k = lane; k < C; k += 32) mx = fmaxf(mx, z[t * C + k]);
-    mx = sg_warp_max(mx);
-    float sum = 0.f;
-    for (int k = lane; k < C; k += 32) sum += expf(z[t * C + k] - mx);
-    sum = sg_warp_sum(sum);
-    float inv = 1.f / sum;
-    for (int k = lane; k < C; k += 32) {
-      float p = expf(z[t * C + k] - mx) * inv;
-      logq[t * C + k] = logf(p + CTC_EPS) - log_norm;
-    }
-  }
+  for (int t = warp; t < T; t += nwarps)
+    warp_softmax_row(z + t * C, C, lane, [&](int k, float p) { logq[t * C + k] = logf(p + CTC_EPS) - log_norm; });
   __syncthreads();
 
   // alpha recursion
@@ -154,6 +162,18 @@ __global__ void k_ctc(const float* __restrict__ logits, const int* __restrict__ 
   }
 }
 
+// Allow Kernel `cap` bytes of dynamic shared memory, once per device: the attribute is a cap (a launch asks for what it uses),
+// so it is not set again on every launch.  Devices >= 64 are not cached and set it every time.
+template <auto Kernel>
+static cudaError_t allow_dynamic_smem(const sg_ctx* ctx, int cap) {
+  static std::atomic<unsigned long long> done{0};
+  const unsigned long long bit = ctx->device < 64 ? 1ull << ctx->device : 0ull;
+  if (bit && (done.load() & bit)) return cudaSuccess;
+  const cudaError_t e = cudaFuncSetAttribute(Kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, cap);
+  if (e == cudaSuccess) done.fetch_or(bit);
+  return e;
+}
+
 static int ctc_launch(sg_ctx* ctx, const float* logits, const int* labels, int b, int t, int c, int l, const int* input_len,
                       const int* label_len, float* loss, float* grad_logits, const char* who) {
   SG_REQUIRE(ctx && logits && labels && loss, "%s: NULL", who);
@@ -163,7 +183,7 @@ static int ctc_launch(sg_ctx* ctx, const float* logits, const int* labels, int b
   int S = 2 * l + 1;
   size_t smem = sizeof(float) * ((size_t)t * c + 2 * (size_t)t * S + c) + sizeof(int) * S;
   SG_REQUIRE(smem <= 200 * 1024, "%s: T*C too large for shared memory (%zu bytes)", who, smem);
-  if (smem > 48 * 1024) SG_CHECK_CUDA(cudaFuncSetAttribute(k_ctc, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
+  if (smem > 48 * 1024) SG_CHECK_CUDA(allow_dynamic_smem<k_ctc>(ctx, 200 * 1024));
   sg_launch(ctx, k_ctc, b, 128, smem, logits, labels, t, c, l, input_len, label_len, loss, grad_logits);
   SG_POST_LAUNCH(ctx);
   return SG_OK;
@@ -188,20 +208,28 @@ extern "C" int sg_ctc_ragged(sg_ctx* ctx, const float* logits, const int* labels
 #define SOFTMAX_ROWS_PER_BLOCK 8
 
 // y = softmax(x) over rows of C fp32 values (the reference's Dense(activation='softmax'), net_architecture.py:55); one warp
-// per row, max-subtracted exp and an fp32 sum -- the first stage of k_ctc
+// per row (warp_softmax_row, the first stage of k_ctc)
 __global__ void k_softmax_rows(const float* __restrict__ x, long long rows, int C, float* __restrict__ y) {
   const int lane = threadIdx.x & 31;
   const long long r = (long long)blockIdx.x * SOFTMAX_ROWS_PER_BLOCK + (threadIdx.x >> 5);
   if (r >= rows) return;
-  const float* z = x + r * C;
-  float mx = NEG_INF;
-  for (int k = lane; k < C; k += 32) mx = fmaxf(mx, z[k]);
-  mx = sg_warp_max(mx);
-  float sum = 0.f;
-  for (int k = lane; k < C; k += 32) sum += expf(z[k] - mx);
-  sum = sg_warp_sum(sum);
-  const float inv = 1.f / sum;
-  for (int k = lane; k < C; k += 32) y[r * C + k] = expf(z[k] - mx) * inv;
+  warp_softmax_row(x + r * C, C, lane, [&](int k, float p) { y[r * C + k] = p; });
+}
+
+// One chunk of a block-scan compaction: the exclusive offset of this thread among the block's flagged threads (warps in
+// order, then lanes) and the chunk's total.  cnt[nwarps] holds the per-warp counts; one __syncthreads after they are
+// written, and the caller syncs before the next chunk rewrites them.
+static __device__ __forceinline__ int block_exclusive_offset(bool flag, int* cnt, int lane, int warp, int nwarps, int* chunk) {
+  const unsigned int bal = __ballot_sync(0xffffffffu, flag);
+  if (lane == 0) cnt[warp] = __popc(bal);
+  __syncthreads();
+  int off = __popc(bal & ((1u << lane) - 1u)), total = 0;
+  for (int w = 0; w < nwarps; ++w) {
+    if (w < warp) off += cnt[w];
+    total += cnt[w];
+  }
+  *chunk = total;
+  return off;
 }
 
 // Greedy decoding of one sample per CTA: best class of every frame t < T_b (ties -> lowest index), repeats merged, blanks
@@ -217,8 +245,7 @@ __global__ void __launch_bounds__(DECODE_THREADS) k_ctc_greedy_decode(const floa
   __shared__ int warp_cnt[DECODE_THREADS / 32];
   __shared__ float red[32];
   const int b = blockIdx.x, tid = threadIdx.x, lane = tid & 31, warp = tid >> 5, nwarps = DECODE_THREADS / 32;
-  int T = input_len ? input_len[b] : Tmax;
-  T = T < 0 ? 0 : (T > Tmax ? Tmax : T);
+  const int T = sample_frames(input_len, b, 0, Tmax);
   const float* p = probs + (long long)b * Tmax * C;
   const int blank = C - 1;
 
@@ -255,15 +282,9 @@ __global__ void __launch_bounds__(DECODE_THREADS) k_ctc_greedy_decode(const floa
     const int t = t0 + tid;
     const int a = t < T ? best[t] : blank;
     const bool emit = t < T && a != blank && (t == 0 || best[t - 1] != a);
-    const unsigned int bal = __ballot_sync(0xffffffffu, emit);
-    if (lane == 0) warp_cnt[warp] = __popc(bal);
-    __syncthreads();
-    int off = base, chunk = 0;
-    for (int w = 0; w < nwarps; ++w) {
-      if (w < warp) off += warp_cnt[w];
-      chunk += warp_cnt[w];
-    }
-    if (emit) out[off + __popc(bal & ((1u << lane) - 1u))] = a;
+    int chunk;
+    const int off = block_exclusive_offset(emit, warp_cnt, lane, warp, nwarps, &chunk);
+    if (emit) out[base + off] = a;
     base += chunk;
     __syncthreads();                   // warp_cnt is rewritten by the next chunk
   }
@@ -363,8 +384,7 @@ extern "C" int sg_ctc_greedy_decode(sg_ctx* ctx, const float* probs, int b, int 
   const size_t smem = (size_t)t_max * (sizeof(int) + sizeof(float));
   SG_REQUIRE(smem <= 200 * 1024, "sg_ctc_greedy_decode: t_max %d too large for shared memory", t_max);
   if (b == 0) return SG_OK;
-  if (smem > 48 * 1024)
-    SG_CHECK_CUDA(cudaFuncSetAttribute(k_ctc_greedy_decode, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
+  if (smem > 48 * 1024) SG_CHECK_CUDA(allow_dynamic_smem<k_ctc_greedy_decode>(ctx, 200 * 1024));
   sg_launch(ctx, k_ctc_greedy_decode, b, DECODE_THREADS, smem, probs, t_max, c, input_len, decoded, decoded_len, neg_sum_log);
   SG_POST_LAUNCH(ctx);
   return SG_OK;
@@ -405,10 +425,72 @@ extern "C" int sg_edit_distance(sg_ctx* ctx, const int* hyp, const int* hyp_len,
 #define BEAM_MAX_C 128
 #define BEAM_NO_SYMBOL 0xFF
 
-__device__ __forceinline__ unsigned long long beam_key(float s, int pos) {
+// the bits of s as an unsigned whose order is the float order: larger float -> larger unsigned
+static __device__ __forceinline__ unsigned int ordered_bits(float s) {
   const unsigned int u = __float_as_uint(s);
-  const unsigned int ord = (u & 0x80000000u) ? ~u : (u | 0x80000000u);          // larger float -> larger unsigned
-  return ((unsigned long long)ord << 32) | (unsigned long long)(0xFFFFFFFFu - (unsigned int)pos);   // then lower index
+  return (u & 0x80000000u) ? ~u : (u | 0x80000000u);
+}
+
+__device__ __forceinline__ unsigned long long beam_key(float s, int pos) {             // larger total, then lower index
+  return ((unsigned long long)ordered_bits(s) << 32) | (unsigned long long)(0xFFFFFFFFu - (unsigned int)pos);
+}
+
+// x[k] = log-softmax(log(p[k] + eps)) over the C <= 128 classes of one frame, one warp, the row in registers
+static __device__ __forceinline__ void frame_log_softmax(const float* p, int C, int lane, float* x) {
+  float lp[BEAM_MAX_C / 32];
+  float m = NEG_INF;
+#pragma unroll
+  for (int j = 0; j < BEAM_MAX_C / 32; ++j) {
+    const int k = lane + 32 * j;
+    lp[j] = k < C ? logf(p[k] + CTC_EPS) : NEG_INF;
+    m = fmaxf(m, lp[j]);
+  }
+  m = sg_warp_max(m);
+  float s = 0.f;
+#pragma unroll
+  for (int j = 0; j < BEAM_MAX_C / 32; ++j)
+    if (lane + 32 * j < C) s += expf(lp[j] - m);
+  const float ls = logf(sg_warp_sum(s));
+#pragma unroll
+  for (int j = 0; j < BEAM_MAX_C / 32; ++j)
+    if (lane + 32 * j < C) x[lane + 32 * j] = (lp[j] - m) - ls;
+}
+
+// One digit of a radix select, warp 0: scan the 256-bin histogram from the top for the bin that holds the need-th largest
+// key (lane l owns bins 255 - 8l .. 248 - 8l).  One lane writes that bin's digit, the number of keys in the bins above it and
+// the bin's count.  Returns the lane's inclusive count: the histogram's total on lane 31.
+static __device__ __forceinline__ int radix_pick_digit(const int* hist, int need, int lane, int* digit, int* above, int* count) {
+  int cnt[8], sum = 0;
+#pragma unroll
+  for (int j = 0; j < 8; ++j) {
+    cnt[j] = hist[255 - 8 * lane - j];
+    sum += cnt[j];
+  }
+  int inc = sum;
+#pragma unroll
+  for (int o = 1; o < 32; o <<= 1) {
+    const int v = __shfl_up_sync(0xffffffffu, inc, o);
+    if (lane >= o) inc += v;
+  }
+  const int exc = inc - sum;
+  const unsigned int hit = __ballot_sync(0xffffffffu, exc < need && need <= inc);
+  if (hit && lane == __ffs(hit) - 1) {
+    int ab = exc, sel = -1, c = 0;
+#pragma unroll
+    for (int j = 0; j < 8; ++j) {                     // unrolled: cnt stays in registers
+      if (sel >= 0) continue;
+      if (ab + cnt[j] >= need) {
+        sel = j;
+        c = cnt[j];
+      } else {
+        ab += cnt[j];
+      }
+    }
+    *digit = 255 - 8 * lane - sel;
+    *above = ab;
+    *count = c;
+  }
+  return inc;
 }
 
 __global__ void __launch_bounds__(BEAM_THREADS) k_ctc_beam_decode(const float* __restrict__ probs, int Tmax, int C,
@@ -428,8 +510,7 @@ __global__ void __launch_bounds__(BEAM_THREADS) k_ctc_beam_decode(const float* _
   __shared__ int s_hist[256];
   __shared__ int s_nsel, s_digit, s_above, s_count, s_total;
   const int b = blockIdx.x, tid = threadIdx.x, lane = tid & 31, warp = tid >> 5;
-  int T = input_len ? input_len[b] : Tmax;
-  T = T < 0 ? 0 : (T > Tmax ? Tmax : T);
+  const int T = sample_frames(input_len, b, 0, Tmax);
   const float* p = probs + (long long)b * Tmax * C;
   unsigned short* bpb = bp + (long long)b * Tmax * W;
   const int blank = C - 1;
@@ -443,25 +524,7 @@ __global__ void __launch_bounds__(BEAM_THREADS) k_ctc_beam_decode(const float* _
 
   for (int t = 0; t < T; ++t) {
     const int nxt = cur ^ 1;
-    if (warp == 0) {                                  // the frame's log-probabilities, one warp (C <= 128)
-      float lp[BEAM_MAX_C / 32];
-      float m = NEG_INF;
-#pragma unroll
-      for (int j = 0; j < BEAM_MAX_C / 32; ++j) {
-        const int k = lane + 32 * j;
-        lp[j] = k < C ? logf(p[(long long)t * C + k] + CTC_EPS) : NEG_INF;
-        m = fmaxf(m, lp[j]);
-      }
-      m = sg_warp_max(m);
-      float s = 0.f;
-#pragma unroll
-      for (int j = 0; j < BEAM_MAX_C / 32; ++j)
-        if (lane + 32 * j < C) s += expf(lp[j] - m);
-      const float ls = logf(sg_warp_sum(s));
-#pragma unroll
-      for (int j = 0; j < BEAM_MAX_C / 32; ++j)
-        if (lane + 32 * j < C) s_x[lane + 32 * j] = (lp[j] - m) - ls;
-    }
+    if (warp == 0) frame_log_softmax(p + (long long)t * C, C, lane, s_x);   // the frame's log-probabilities
     __syncthreads();
 
     // candidates: cand[r C + c] = total of the extension of beam r by c, or of r's continuation at c = blank
@@ -513,37 +576,8 @@ __global__ void __launch_bounds__(BEAM_THREADS) k_ctc_beam_decode(const float* _
         if ((key & mask) == prefix) atomicAdd(&s_hist[(int)((key >> sh) & 0xFFull)], 1);
       }
       __syncthreads();
-      if (warp == 0) {                                // lane l owns bins 255 - 8l .. 248 - 8l, scanned from the top
-        int cnt[8], sum = 0;
-#pragma unroll
-        for (int j = 0; j < 8; ++j) {
-          cnt[j] = s_hist[255 - 8 * lane - j];
-          sum += cnt[j];
-        }
-        int inc = sum;
-#pragma unroll
-        for (int o = 1; o < 32; o <<= 1) {
-          const int v = __shfl_up_sync(0xffffffffu, inc, o);
-          if (lane >= o) inc += v;
-        }
-        const int exc = inc - sum;
-        const unsigned int hit = __ballot_sync(0xffffffffu, exc < need && need <= inc);
-        if (hit && lane == __ffs(hit) - 1) {
-          int above = exc, sel = -1, count = 0;
-#pragma unroll
-          for (int j = 0; j < 8; ++j) {               // unrolled: cnt stays in registers
-            if (sel >= 0) continue;
-            if (above + cnt[j] >= need) {
-              sel = j;
-              count = cnt[j];
-            } else {
-              above += cnt[j];
-            }
-          }
-          s_digit = 255 - 8 * lane - sel;
-          s_above = above;
-          s_count = count;
-        }
+      if (warp == 0) {
+        const int inc = radix_pick_digit(s_hist, need, lane, &s_digit, &s_above, &s_count);
         if (lane == 31) s_total = inc;
       }
       __syncthreads();
@@ -672,15 +706,8 @@ extern "C" int sg_ctc_beam_decode(sg_ctx* ctx, const float* probs, int b, int t_
   SG_REQUIRE(scratch && scratch_bytes >= need, "sg_ctc_beam_decode: scratch of %zu bytes for %d x %d back-pointers, got %zu", need,
              b, t_max, scratch_bytes);
   const size_t smem = (size_t)beam_width * c * (sizeof(float) + 1);
-  // the kernel's ~11 KB of static shared memory counts against the 48 KB default too: allow the largest dynamic size once per
-  // device (the attribute is a cap, the launch asks for what it uses), not on every launch
-  static std::atomic<unsigned long long> attr_set{0};
-  const unsigned long long bit = ctx->device < 64 ? 1ull << ctx->device : 0ull;     // 0: no cache, set every time
-  if (!bit || !(attr_set.load() & bit)) {
-    SG_CHECK_CUDA(cudaFuncSetAttribute(k_ctc_beam_decode, cudaFuncAttributeMaxDynamicSharedMemorySize,
-                                       (int)((size_t)BEAM_MAX_W * BEAM_MAX_C * (sizeof(float) + 1))));
-    attr_set.fetch_or(bit);
-  }
+  // the kernel's ~11 KB of static shared memory counts against the 48 KB default too: allow the largest dynamic size
+  SG_CHECK_CUDA(allow_dynamic_smem<k_ctc_beam_decode>(ctx, (int)((size_t)BEAM_MAX_W * BEAM_MAX_C * (sizeof(float) + 1))));
   sg_launch(ctx, k_ctc_beam_decode, b, BEAM_THREADS, smem, probs, t_max, c, input_len, beam_width, top_paths, merge_repeated,
             decoded, decoded_len, log_prob, (unsigned short*)scratch);
   SG_POST_LAUNCH(ctx);
@@ -704,6 +731,7 @@ extern "C" int sg_ctc_beam_decode(sg_ctx* ctx, const float* probs, int b, int t_
 #define LEX_MAX_C 128
 #define LEX_MAX_TOPK 128
 #define LEX_MAX_SMEM (200 * 1024)
+static_assert(LEX_MAX_C <= BEAM_MAX_C, "frame_log_softmax holds up to BEAM_MAX_C classes");
 
 __global__ void __launch_bounds__(LEX_THREADS) k_ctc_lexicon_scores(const float* __restrict__ probs, int Tmax, int C,
                                                                     const int* __restrict__ input_len,
@@ -714,30 +742,12 @@ __global__ void __launch_bounds__(LEX_THREADS) k_ctc_lexicon_scores(const float*
   const int b = blockIdx.x / tiles, tile = blockIdx.x - b * tiles;
   const int tid = threadIdx.x, lane = tid & 31, warp = tid >> 5, nwarps = LEX_THREADS / 32;
   const unsigned int full = 0xffffffffu;
-  int T = input_len ? input_len[b] : Tmax;
-  T = T < 0 ? 0 : (T > Tmax ? Tmax : T);
+  const int T = sample_frames(input_len, b, 0, Tmax);
   const float* p = probs + (long long)b * Tmax * C;
   const int blank = C - 1;
 
-  for (int t = warp; t < T; t += nwarps) {            // the frame table, one warp per frame (C <= 128)
-    float lp[LEX_MAX_C / 32];
-    float m = NEG_INF;
-#pragma unroll
-    for (int j = 0; j < LEX_MAX_C / 32; ++j) {
-      const int k = lane + 32 * j;
-      lp[j] = k < C ? logf(p[(long long)t * C + k] + CTC_EPS) : NEG_INF;
-      m = fmaxf(m, lp[j]);
-    }
-    m = sg_warp_max(m);
-    float s = 0.f;
-#pragma unroll
-    for (int j = 0; j < LEX_MAX_C / 32; ++j)
-      if (lane + 32 * j < C) s += expf(lp[j] - m);
-    const float ls = logf(sg_warp_sum(s));
-#pragma unroll
-    for (int j = 0; j < LEX_MAX_C / 32; ++j)
-      if (lane + 32 * j < C) x[t * C + lane + 32 * j] = (lp[j] - m) - ls;
-  }
+  for (int t = warp; t < T; t += nwarps)              // the frame table, one warp per frame
+    frame_log_softmax(p + (long long)t * C, C, lane, x + t * C);
   __syncthreads();
 
   const int v_end = min(V, (tile + 1) * LEX_WORDS);
@@ -797,10 +807,7 @@ __global__ void __launch_bounds__(LEX_THREADS) k_ctc_lexicon_scores(const float*
 // tied keys in index order are compacted with a block scan, and the <= 128 survivors are ranked by counting.  Equal scores go
 // to the lower word index; -inf is ranked like any other score (-0 and +0 are equal).  The chosen words are gathered from
 // the lexicon in the same launch.
-__device__ __forceinline__ unsigned int lex_key(float s) {
-  const unsigned int u = __float_as_uint(s == 0.f ? 0.f : s);
-  return (u & 0x80000000u) ? ~u : (u | 0x80000000u);        // larger float -> larger unsigned
-}
+__device__ __forceinline__ unsigned int lex_key(float s) { return ordered_bits(s == 0.f ? 0.f : s); }
 
 __global__ void __launch_bounds__(LEX_THREADS) k_ctc_lexicon_topk(const float* __restrict__ scores, int V,
                                                                   const int* __restrict__ lexicon,
@@ -813,7 +820,7 @@ __global__ void __launch_bounds__(LEX_THREADS) k_ctc_lexicon_topk(const float* _
   __shared__ unsigned int s_key[LEX_MAX_TOPK];
   __shared__ int s_idx[LEX_MAX_TOPK], s_order[LEX_MAX_TOPK];
   const int b = blockIdx.x, tid = threadIdx.x, lane = tid & 31, warp = tid >> 5, nwarps = LEX_THREADS / 32;
-  const unsigned int full = 0xffffffffu, below = (1u << lane) - 1u;
+  const unsigned int full = 0xffffffffu;
   const float* row = scores + (long long)b * V;
 
   // the K-th largest key: after pass p its top 8(p + 1) bits are `prefix`; need = how many keys with that prefix are kept
@@ -831,38 +838,7 @@ __global__ void __launch_bounds__(LEX_THREADS) k_ctc_lexicon_topk(const float* _
       if (bin < 256 && lane == __ffs(peers) - 1) atomicAdd(&s_hist[bin], __popc(peers));
     }
     __syncthreads();
-    if (warp == 0) {                                  // lane l owns bins 255 - 8l .. 248 - 8l, scanned from the top
-      int cnt[8], sum = 0;
-#pragma unroll
-      for (int j = 0; j < 8; ++j) {
-        cnt[j] = s_hist[255 - 8 * lane - j];
-        sum += cnt[j];
-      }
-      int inc = sum;
-#pragma unroll
-      for (int o = 1; o < 32; o <<= 1) {
-        const int v = __shfl_up_sync(full, inc, o);
-        if (lane >= o) inc += v;
-      }
-      const int exc = inc - sum;
-      const unsigned int hit = __ballot_sync(full, exc < need && need <= inc);
-      if (hit && lane == __ffs(hit) - 1) {
-        int above = exc, sel = -1, count = 0;
-#pragma unroll
-        for (int j = 0; j < 8; ++j) {
-          if (sel >= 0) continue;
-          if (above + cnt[j] >= need) {
-            sel = j;
-            count = cnt[j];
-          } else {
-            above += cnt[j];
-          }
-        }
-        s_digit = 255 - 8 * lane - sel;
-        s_above = above;
-        s_count = count;
-      }
-    }
+    if (warp == 0) radix_pick_digit(s_hist, need, lane, &s_digit, &s_above, &s_count);
     __syncthreads();
     need -= s_above;
     prefix |= (unsigned int)s_digit << sh;
@@ -876,23 +852,10 @@ __global__ void __launch_bounds__(LEX_THREADS) k_ctc_lexicon_topk(const float* _
     const int i = i0 + tid;
     const unsigned int key = i < V ? lex_key(row[i]) : 0u;
     const bool gt = i < V && (key & mask) > prefix, eq = i < V && (key & mask) == prefix;
-    const unsigned int beq = __ballot_sync(full, eq);
-    if (lane == 0) s_wcnt[0][warp] = __popc(beq);
-    __syncthreads();
-    int eq_before = base_eq + __popc(beq & below), eq_chunk = 0;
-    for (int w = 0; w < nwarps; ++w) {
-      if (w < warp) eq_before += s_wcnt[0][w];
-      eq_chunk += s_wcnt[0][w];
-    }
+    int eq_chunk, chunk;
+    const int eq_before = base_eq + block_exclusive_offset(eq, s_wcnt[0], lane, warp, nwarps, &eq_chunk);
     const bool take = gt || (eq && eq_before < need);
-    const unsigned int bt = __ballot_sync(full, take);
-    if (lane == 0) s_wcnt[1][warp] = __popc(bt);
-    __syncthreads();
-    int off = base_sel + __popc(bt & below), chunk = 0;
-    for (int w = 0; w < nwarps; ++w) {
-      if (w < warp) off += s_wcnt[1][w];
-      chunk += s_wcnt[1][w];
-    }
+    const int off = base_sel + block_exclusive_offset(take, s_wcnt[1], lane, warp, nwarps, &chunk);
     if (take) {
       s_key[off] = key;
       s_idx[off] = i;
@@ -937,12 +900,7 @@ extern "C" int sg_ctc_lexicon_scores(sg_ctx* ctx, const float* probs, int b, int
   SG_REQUIRE(probs && lex_len && scores && (lexicon || l_max == 0), "sg_ctc_lexicon_scores: NULL");
   const long long tiles = (v + LEX_WORDS - 1) / LEX_WORDS;
   SG_REQUIRE((long long)b * tiles <= 0x7fffffffLL, "sg_ctc_lexicon_scores: %d samples x %lld word tiles", b, tiles);
-  static std::atomic<unsigned long long> attr_set{0};           // allow the largest frame table once per device
-  const unsigned long long bit = ctx->device < 64 ? 1ull << ctx->device : 0ull;
-  if (!bit || !(attr_set.load() & bit)) {
-    SG_CHECK_CUDA(cudaFuncSetAttribute(k_ctc_lexicon_scores, cudaFuncAttributeMaxDynamicSharedMemorySize, LEX_MAX_SMEM));
-    attr_set.fetch_or(bit);
-  }
+  SG_CHECK_CUDA(allow_dynamic_smem<k_ctc_lexicon_scores>(ctx, LEX_MAX_SMEM));    // the largest frame table
   sg_launch(ctx, k_ctc_lexicon_scores, (unsigned int)(b * tiles), LEX_THREADS, smem, probs, t_max, c, input_len, lexicon, lex_len,
             v, l_max, (int)tiles, scores);
   SG_POST_LAUNCH(ctx);

@@ -20,6 +20,12 @@ from .bigacgan.net_architecture import to_device_f32, to_device_i32
 from .runtime import get_runtime
 
 
+def _frame_inputs(y_pred, input_length):
+    """The runtime, and (y_pred, input_length) on its device: (B, T, C) fp32 probabilities, (B,) int32 frame counts or None."""
+    rt = get_runtime()
+    return rt, to_device_f32(rt, y_pred), None if input_length is None else to_device_i32(rt, input_length).reshape(-1)
+
+
 def ctc_decode(y_pred, input_length, greedy=True, beam_width=100, top_paths=1):
     """tf.keras.backend.ctc_decode.  y_pred: (B, T, C) softmax probabilities (torch tensor, host buffer or DLPack producer);
     input_length: (B,) frames per sample, or None for all T.  Returns ([decoded], log_prob): decoded (B, T) int32 on the
@@ -28,9 +34,7 @@ def ctc_decode(y_pred, input_length, greedy=True, beam_width=100, top_paths=1):
     the signature); beam search is ctc_beam_decode."""
     if not greedy:
         raise NotImplementedError("ctc_decode: greedy=False is not wired here; use decode.ctc_beam_decode for beam search")
-    rt = get_runtime()
-    probs = to_device_f32(rt, y_pred)
-    il = None if input_length is None else to_device_i32(rt, input_length).reshape(-1)
+    rt, probs, il = _frame_inputs(y_pred, input_length)
     decoded, _, score = ops.ctc_greedy_decode(rt, probs, il)
     return [decoded], score.view(-1, 1)
 
@@ -41,9 +45,7 @@ def ctc_beam_decode(y_pred, input_length, beam_width=100, top_paths=1, merge_rep
     Returns ([decoded_0, ..., decoded_{top_paths-1}], log_prob): decoded_k (B, T) int32 on the device, padded with -1, the
     k-th most probable beam; log_prob (B, top_paths) fp32, -inf where a sample has fewer live beams.  merge_repeated merges
     consecutive equal symbols of the written path, as TF v1 does [TF-SEMANTICS]."""
-    rt = get_runtime()
-    probs = to_device_f32(rt, y_pred)
-    il = None if input_length is None else to_device_i32(rt, input_length).reshape(-1)
+    rt, probs, il = _frame_inputs(y_pred, input_length)
     decoded, _, log_prob = ops.ctc_beam_decode(rt, probs, il, beam_width, top_paths, merge_repeated)
     return list(decoded.unbind(0)), log_prob
 
@@ -88,17 +90,19 @@ def _lexicon(rt, lexicon):
     return lex, ops.label_lengths(rt, lex)
 
 
+def _best_words(rt, probs, il, lexicon, top_paths=1):
+    """Every sample's top_paths most likely words of lexicon = (matrix, lengths) on the device (ops.ctc_lexicon_topk)."""
+    return ops.ctc_lexicon_topk(rt, ops.ctc_lexicon_scores(rt, probs, il, *lexicon), *lexicon, top_paths)
+
+
 def ctc_lexicon_scores(y_pred, input_length, lexicon):
     """log p(word | image) of every (sample, lexicon word) pair, i.e. -K.ctc_batch_cost of the pair, without building the
     replicated batch: (B, V) fp32 on the device.  y_pred: (B, T, C) softmax probabilities (C <= 128, T * C <= 51 200);
     input_length: (B,) frames per sample or None for all T; lexicon: (V, Lmax <= 31) int32 padded with -1 (encode_words).
     A word that cannot fit in a sample's frames scores -inf.  The scores give posteriors over the lexicon, or can be
     combined with word priors; ops.ctc_lexicon_topk ranks any such (B, V) rows."""
-    rt = get_runtime()
-    probs = to_device_f32(rt, y_pred)
-    il = None if input_length is None else to_device_i32(rt, input_length).reshape(-1)
-    lex, lens = _lexicon(rt, lexicon)
-    return ops.ctc_lexicon_scores(rt, probs, il, lex, lens)
+    rt, probs, il = _frame_inputs(y_pred, input_length)
+    return ops.ctc_lexicon_scores(rt, probs, il, *_lexicon(rt, lexicon))
 
 
 def ctc_lexicon_decode(y_pred, input_length, lexicon, top_paths=1):
@@ -106,12 +110,8 @@ def ctc_lexicon_decode(y_pred, input_length, lexicon, top_paths=1):
     ctc_lexicon_scores; 1 <= top_paths <= min(V, 128).  Returns ([decoded_0, ..., decoded_{top_paths-1}], log_prob, index):
     decoded_k (B, Lmax) int32 on the device, the k-th best word padded with -1; log_prob (B, top_paths) fp32, its score;
     index (B, top_paths) int32, its row in the lexicon.  Equal scores go to the lower row."""
-    rt = get_runtime()
-    probs = to_device_f32(rt, y_pred)
-    il = None if input_length is None else to_device_i32(rt, input_length).reshape(-1)
-    lex, lens = _lexicon(rt, lexicon)
-    decoded, _, log_prob, index = ops.ctc_lexicon_topk(rt, ops.ctc_lexicon_scores(rt, probs, il, lex, lens), lex, lens,
-                                                       top_paths)
+    rt, probs, il = _frame_inputs(y_pred, input_length)
+    decoded, _, log_prob, index = _best_words(rt, probs, il, _lexicon(rt, lexicon), top_paths)
     return list(decoded.unbind(0)), log_prob, index
 
 
@@ -130,8 +130,7 @@ def _read(rt, recognizer, images, labels, input_length, label_length, totals, be
     lengths) on the device), its distances to the labels added to the device totals; returns the decoded words."""
     probs = recognizer.frame_probs(images)
     if lexicon is not None:
-        lex, lens = lexicon
-        decoded, dlen, _, _ = ops.ctc_lexicon_topk(rt, ops.ctc_lexicon_scores(rt, probs, input_length, lex, lens), lex, lens)
+        decoded, dlen, _, _ = _best_words(rt, probs, input_length, lexicon)
         decoded, dlen = decoded[0], dlen[0]
     elif beam_width is None:
         decoded, dlen, _ = ops.ctc_greedy_decode(rt, probs, input_length)

@@ -13,6 +13,23 @@ import torch
 KERAS_EPS = 1e-7
 
 
+def _peaked_logits(seed, b, t, c):
+    """Logits of a planted path (letters held over several frames, blanks, repeats) plus N(0, 1.5^2) noise: peaked
+    probabilities with plausible competitors."""
+    g = torch.Generator().manual_seed(seed)
+    blank = c - 1
+    path = torch.empty(b, t, dtype=torch.long)
+    for i in range(b):
+        prev = blank
+        for s in range(t):
+            u = float(torch.rand(1, generator=g))
+            prev = prev if u < 0.45 else (blank if u < 0.7 else int(torch.randint(0, c, (1,), generator=g)))
+            path[i, s] = prev
+    z = torch.randn(b, t, c, generator=g) * 1.5
+    z.scatter_add_(2, path.unsqueeze(-1), torch.full((b, t, 1), 5.0))
+    return z
+
+
 def frame_log_probs(p):
     """log-softmax(log(p + 1e-7)) over the last axis, float64."""
     lp = np.log(np.asarray(p, np.float64) + KERAS_EPS)

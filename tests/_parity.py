@@ -134,6 +134,13 @@ def build_models(rt, P, style_encoder=False, r_classes=53):
     return G, D, R, W
 
 
+def _recognizer(rt, P, classes):
+    """A libsgan recogniser of `classes` outputs carrying the weights P."""
+    R = na.make_recognizer(IN_DIM, None, classes, vis_model=False, rt=rt, initialise=False)
+    R.load_state_dict(P)
+    return R
+
+
 def run_step(rt, G, D, R, W, images, labels, fake_labels, z, loss_name="hinge", balance=True, style=None, batch_idx=0):
     gan = na.make_gan(G, D, R, W, vis_model=False)
     g_opt, d_opt, r_opt, w_opt, loss_fn, disc_iters, agb = optim.setup_optimizer(2e-4, 2e-4, 2e-4, 2e-4, 0.0, 0.999, getattr(nl, loss_name), 1,

@@ -7,8 +7,8 @@ import pytest
 import torch
 
 import sgan_oracle as O
-from _beam_ref import ctc_beam_decode, frame_log_probs, labeling_log_probs
-from _parity import IN_DIM, na
+from _beam_ref import _peaked_logits, ctc_beam_decode, frame_log_probs, labeling_log_probs
+from _parity import IN_DIM, _recognizer, na
 
 pytestmark = pytest.mark.gpu
 ops = importlib.import_module("scrabble-gan_b200.ops")
@@ -17,23 +17,6 @@ decode = importlib.import_module("scrabble-gan_b200.decode")
 
 MARGIN = 1e-4          # nats: a pruning decision closer than this may go either way in fp32
 TOL_LOGP = 1e-4
-
-
-def _peaked_logits(seed, b, t, c):
-    """Logits of a planted path (letters held over several frames, blanks, repeats) plus N(0, 1.5^2) noise: peaked
-    probabilities with plausible competitors."""
-    g = torch.Generator().manual_seed(seed)
-    blank = c - 1
-    path = torch.empty(b, t, dtype=torch.long)
-    for i in range(b):
-        prev = blank
-        for s in range(t):
-            u = float(torch.rand(1, generator=g))
-            prev = prev if u < 0.45 else (blank if u < 0.7 else int(torch.randint(0, c, (1,), generator=g)))
-            path[i, s] = prev
-    z = torch.randn(b, t, c, generator=g) * 1.5
-    z.scatter_add_(2, path.unsqueeze(-1), torch.full((b, t, 1), 5.0))
-    return z
 
 
 def _run(rt, p, il, w, k, merge=True):
@@ -151,12 +134,6 @@ def test_beam_decode_limits(rt):
 # ----------------------------------------------------------------------------------------------------
 # with the recogniser
 # ----------------------------------------------------------------------------------------------------
-def _recognizer(rt, P, classes):
-    R = na.make_recognizer(IN_DIM, None, classes, vis_model=False, rt=rt, initialise=False)
-    R.load_state_dict(P)
-    return R
-
-
 def test_ctc_beam_decode_of_frame_probs(rt):
     rt.set_mode("fp32")
     b, l, classes = 64, 6, 53

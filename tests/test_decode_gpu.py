@@ -8,7 +8,7 @@ import torch
 
 import sgan_oracle as O
 from _decode_ref import ctc_greedy_decode, levenshtein
-from _parity import IN_DIM, na, rel_elementwise, rel_max
+from _parity import IN_DIM, _recognizer, na, rel_elementwise, rel_max
 
 pytestmark = pytest.mark.gpu
 ops = importlib.import_module("scrabble-gan_b200.ops")
@@ -138,12 +138,6 @@ def _oracle_probs(x, P, mode):
             return O.recognizer_probs(x, P)
     finally:
         O.set_operand_rounding(None)
-
-
-def _recognizer(rt, P, classes):
-    R = na.make_recognizer(IN_DIM, None, classes, vis_model=False, rt=rt, initialise=False)
-    R.load_state_dict(P)
-    return R
 
 
 @pytest.mark.parametrize("mode", ["fp32", "bf16"])

@@ -10,7 +10,7 @@ from scipy import ndimage
 
 import _htr_ref as H
 import sgan_oracle as O
-from _parity import IN_DIM, assert_grads, grad_profile, build_models, du, make_inputs, make_params, na, nl, optim, rel_elementwise, run_step
+from _parity import IN_DIM, _recognizer, assert_grads, grad_profile, build_models, du, make_inputs, make_params, na, nl, optim, rel_elementwise, run_step
 from test_models_gpu import check_dict
 from test_parity_benchpath_gpu import TOL, TOL_OUT
 
@@ -107,12 +107,6 @@ def _r_params(seed, classes, dt=torch.float64, bias_scale=0.1):
         P[k + ".gamma"] = (torch.rand(512, generator=g, dtype=torch.float64) + 0.5).to(dt)
         P[k + ".beta"] = (torch.randn(512, generator=g, dtype=torch.float64) * 0.1).to(dt)
     return P
-
-
-def _recognizer(rt, P, classes):
-    R = na.make_recognizer(IN_DIM, None, classes, vis_model=False, rt=rt, initialise=False)
-    R.load_state_dict(P)
-    return R
 
 
 def _r_opt(lr=1e-3, beta_1=0.5, rmsprop=0):

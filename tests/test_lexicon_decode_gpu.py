@@ -9,8 +9,9 @@ import torch
 from torch.profiler import ProfilerActivity, profile
 
 import sgan_oracle as O
+from _beam_ref import _peaked_logits
 from _lexicon_ref import lexicon_scores, word_lengths
-from _parity import IN_DIM, na
+from _parity import IN_DIM, _recognizer, na
 
 pytestmark = pytest.mark.gpu
 ops = importlib.import_module("scrabble-gan_b200.ops")
@@ -19,23 +20,6 @@ decode = importlib.import_module("scrabble-gan_b200.decode")
 
 TOL = 1e-4             # |got - ref| <= TOL * max(1, |ref|) on finite scores
 WORD_TILE = 64         # words per CTA of k_ctc_lexicon_scores (LEX_WORDS)
-
-
-def _peaked_logits(seed, b, t, c):
-    """Logits of a planted path (letters held over several frames, blanks, repeats) plus N(0, 1.5^2) noise, as in the beam
-    decoder's tests."""
-    g = torch.Generator().manual_seed(seed)
-    blank = c - 1
-    path = torch.empty(b, t, dtype=torch.long)
-    for i in range(b):
-        prev = blank
-        for s in range(t):
-            u = float(torch.rand(1, generator=g))
-            prev = prev if u < 0.45 else (blank if u < 0.7 else int(torch.randint(0, c, (1,), generator=g)))
-            path[i, s] = prev
-    z = torch.randn(b, t, c, generator=g) * 1.5
-    z.scatter_add_(2, path.unsqueeze(-1), torch.full((b, t, 1), 5.0))
-    return z
 
 
 def _lexicon(seed, v, letters, lo, hi, with_empty=True):
@@ -212,12 +196,6 @@ def test_beam_path_score_is_a_lower_bound(rt, b, t, c, w, exact):
 # ----------------------------------------------------------------------------------------------------
 # with the recogniser
 # ----------------------------------------------------------------------------------------------------
-def _recognizer(rt, P, classes):
-    R = na.make_recognizer(IN_DIM, None, classes, vis_model=False, rt=rt, initialise=False)
-    R.load_state_dict(P)
-    return R
-
-
 def test_ctc_lexicon_decode_of_frame_probs(rt):
     rt.set_mode("fp32")
     b, l, classes = 64, 6, 53

@@ -8,7 +8,6 @@ import argparse
 import importlib
 import json
 import os
-import subprocess
 import sys
 
 ROOT = os.path.dirname(os.path.dirname(os.path.abspath(__file__)))
@@ -16,31 +15,12 @@ sys.path.insert(0, ROOT)
 
 import torch  # noqa: E402
 
-from torch.profiler import ProfilerActivity, profile  # noqa: E402
-
 _abi = importlib.import_module("scrabble-gan_b200._abi")
 runtime = importlib.import_module("scrabble-gan_b200.runtime")
 ops = importlib.import_module("scrabble-gan_b200.ops")
 na = importlib.import_module("scrabble-gan_b200.bigacgan.net_architecture")
 
-
-def card():
-    q = subprocess.run(["nvidia-smi", "--query-gpu=name,power.limit,clocks.max.sm", "--format=csv,noheader"], capture_output=True,
-                       text=True)
-    return q.stdout.strip().splitlines()[0] if q.returncode == 0 and q.stdout.strip() else torch.cuda.get_device_name(0)
-
-
-def timed_ms(fn, iters, warmup=5):
-    for _ in range(warmup):
-        fn()
-    torch.cuda.synchronize()
-    a, b = torch.cuda.Event(enable_timing=True), torch.cuda.Event(enable_timing=True)
-    a.record()
-    for _ in range(iters):
-        fn()
-    b.record()
-    torch.cuda.synchronize()
-    return a.elapsed_time(b) / iters
+from _bench_util import card, device_us, r_forward_us, timed_ms  # noqa: E402
 
 
 def main():
@@ -72,42 +52,17 @@ def main():
         return lambda: _abi.call.sg_ctc_beam_decode(rt.ctx, ptr(p), n, t, c, ptr(lens), w, 1, 1, ptr(dec), ptr(dlen), ptr(lp),
                                                     ptr(scratch), nbytes)
 
-    def device_us(fn, name, calls=20):
-        """Device time of kernel `name` per call from torch.profiler (a pass of its own, after warm-up)."""
-        fn()
-        torch.cuda.synchronize()
-        with profile(activities=[ProfilerActivity.CUDA]) as prof:
-            for _ in range(calls):
-                fn()
-            torch.cuda.synchronize()
-        tot = 0.0
-        for e in prof.key_averages():
-            if name in e.key:
-                tot += getattr(e, "device_time_total", None) or getattr(e, "cuda_time_total", 0.0)
-        return tot / calls
-
     # CUDA events around back-to-back launches (host launch overhead included, as in r03's kernel legs), then the kernels'
     # own device time from the profiler
     res["R_forward_ms_host_included"] = timed_ms(lambda: R._logits(rt, x, False), args.iters)
     greedy = lambda: ops.ctc_greedy_decode(rt, probs, il)    # noqa: E731
     res["greedy_decode_us_host_included"] = 1e3 * timed_ms(greedy, args.iters * 4)
-    res["greedy_decode_us_device"] = device_us(greedy, "k_ctc_greedy_decode")
-    fwd_all = 0.0
-    R._logits(rt, x, False)
-    torch.cuda.synchronize()
-    with profile(activities=[ProfilerActivity.CUDA]) as prof:
-        for _ in range(10):
-            R._logits(rt, x, False)
-        torch.cuda.synchronize()
-    for e in prof.key_averages():
-        tt = getattr(e, "device_time_total", None) or getattr(e, "cuda_time_total", 0.0)
-        if not e.key.startswith(("Memcpy", "Memset")) and tt > 0:
-            fwd_all += tt
-    res["R_forward_us_device"] = fwd_all / 10
+    res["greedy_decode_us_device"] = device_us(greedy, ["k_ctc_greedy_decode"])["k_ctc_greedy_decode"]
+    res["R_forward_us_device"] = r_forward_us(R, rt, x)
     for w in (10, 100):
         fn = beam_launch(probs, il, w)
         res["beam%d_us_host_included" % w] = 1e3 * timed_ms(fn, args.iters)
-        dev = device_us(fn, "k_ctc_beam_decode")
+        dev = device_us(fn, ["k_ctc_beam_decode"])["k_ctc_beam_decode"]
         res["beam%d_us_device" % w] = dev
         res["beam%d_share_of_R_forward_device" % w] = dev / res["R_forward_us_device"]
         res["beam%d_over_greedy_device" % w] = dev / res["greedy_decode_us_device"]
@@ -116,7 +71,8 @@ def main():
     pb, ilb = probs.repeat(16, 1, 1), il.repeat(16)
     for w in (10, 100):
         res["beam%d_b256_us_per_sample_device" % w] = res["beam%d_us_device" % w] / b
-        res["beam%d_b4096_us_per_sample_device" % w] = device_us(beam_launch(pb, ilb, w), "k_ctc_beam_decode", 5) / (16 * b)
+        dev = device_us(beam_launch(pb, ilb, w), ["k_ctc_beam_decode"], 5)["k_ctc_beam_decode"]
+        res["beam%d_b4096_us_per_sample_device" % w] = dev / (16 * b)
     print(json.dumps(res, indent=1))
     if args.out:
         with open(args.out, "w") as f:

@@ -7,7 +7,6 @@ import argparse
 import importlib
 import json
 import os
-import subprocess
 import sys
 
 ROOT = os.path.dirname(os.path.dirname(os.path.abspath(__file__)))
@@ -20,24 +19,7 @@ ops = importlib.import_module("scrabble-gan_b200.ops")
 na = importlib.import_module("scrabble-gan_b200.bigacgan.net_architecture")
 decode = importlib.import_module("scrabble-gan_b200.decode")
 
-
-def card():
-    q = subprocess.run(["nvidia-smi", "--query-gpu=name,power.limit,clocks.max.sm", "--format=csv,noheader"], capture_output=True,
-                       text=True)
-    return q.stdout.strip().splitlines()[0] if q.returncode == 0 and q.stdout.strip() else torch.cuda.get_device_name(0)
-
-
-def timed_ms(fn, iters, warmup=5):
-    for _ in range(warmup):
-        fn()
-    torch.cuda.synchronize()
-    a, b = torch.cuda.Event(enable_timing=True), torch.cuda.Event(enable_timing=True)
-    a.record()
-    for _ in range(iters):
-        fn()
-    b.record()
-    torch.cuda.synchronize()
-    return a.elapsed_time(b) / iters
+from _bench_util import card, kernel_us, timed_ms  # noqa: E402
 
 
 def main():
@@ -78,19 +60,10 @@ def main():
     res["b_R_forward_ms"] = fwd_ms
     # device time of every kernel of one evaluate_recognizer pass (torch.profiler, a pass of its own): the three new kernels'
     # share, and their time against R's forward kernels (eager timing above includes the host's launch overhead)
-    from torch.profiler import ProfilerActivity, profile
-    with profile(activities=[ProfilerActivity.CUDA]) as prof:
-        decode.evaluate_recognizer(R, batches)
-        torch.cuda.synchronize()
+    per = kernel_us(lambda: decode.evaluate_recognizer(R, batches), 1)
     new = ("k_softmax_rows", "k_ctc_greedy_decode", "k_edit_distance")
-    t_new = t_all = 0.0
-    for e in prof.key_averages():
-        t = getattr(e, "device_time_total", None) or getattr(e, "cuda_time_total", 0.0)
-        if e.key.startswith(("Memcpy", "Memset")) or t <= 0:
-            continue
-        t_all += t
-        if any(k in e.key for k in new):
-            t_new += t
+    t_all = sum(per.values())
+    t_new = sum(t for k, t in per.items() if any(n in k for n in new))
     res["b_new_kernels_us_per_batch"] = t_new / nb
     res["b_all_kernels_us_per_batch"] = t_all / nb
     res["b_new_kernels_share_of_evaluate"] = t_new / t_all

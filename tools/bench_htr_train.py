@@ -9,7 +9,6 @@ import argparse
 import importlib
 import json
 import os
-import subprocess
 import sys
 import time
 
@@ -19,8 +18,6 @@ sys.path.insert(0, ROOT)
 import numpy as np  # noqa: E402
 import torch  # noqa: E402
 
-from torch.profiler import ProfilerActivity, profile  # noqa: E402
-
 runtime = importlib.import_module("scrabble-gan_b200.runtime")
 ops = importlib.import_module("scrabble-gan_b200.ops")
 optim = importlib.import_module("scrabble-gan_b200.optim")
@@ -29,27 +26,14 @@ na = importlib.import_module("scrabble-gan_b200.bigacgan.net_architecture")
 du = importlib.import_module("scrabble-gan_b200.bigacgan.data_utils")
 nl = importlib.import_module("scrabble-gan_b200.bigacgan.net_loss")
 
+from _bench_util import card, device_us, timed_ms  # noqa: E402
+
 AUG = dict(rotation=2.0, shear=0.3, scale=0.1, translate=2.0, p_morph=0.25)
-
-
-def card():
-    q = subprocess.run(["nvidia-smi", "--query-gpu=name,power.limit,clocks.max.sm", "--format=csv,noheader"], capture_output=True,
-                       text=True)
-    return q.stdout.strip().splitlines()[0] if q.returncode == 0 and q.stdout.strip() else torch.cuda.get_device_name(0)
 
 
 def timed(step, warmup, steps):
     """ms per step over `steps` steps after `warmup`, from CUDA events; and the host enqueue time of one more step."""
-    for _ in range(warmup):
-        step()
-    torch.cuda.synchronize()
-    e0, e1 = torch.cuda.Event(enable_timing=True), torch.cuda.Event(enable_timing=True)
-    e0.record()
-    for _ in range(steps):
-        step()
-    e1.record()
-    torch.cuda.synchronize()
-    ms = e0.elapsed_time(e1) / steps
+    ms = timed_ms(step, steps, warmup)
     t0 = time.perf_counter()
     step()
     enqueue_ms = (time.perf_counter() - t0) * 1e3
@@ -95,18 +79,7 @@ def main():
     u = ops.random_(rt, rt.empty((b, 7)), normal=False)
     out = rt.empty(x.shape)
     aug = lambda: ops.word_augment(rt, x, u, None, out=out, **AUG)  # noqa: E731
-    aug()
-    torch.cuda.synchronize()
-    calls = 50
-    with profile(activities=[ProfilerActivity.CUDA]) as prof:
-        for _ in range(calls):
-            aug()
-        torch.cuda.synchronize()
-    us = 0.0
-    for e in prof.key_averages():
-        if "k_word_augment" in e.key:
-            us += getattr(e, "device_time_total", None) or getattr(e, "cuda_time_total", 0.0)
-    us /= calls
+    us = device_us(aug, ["k_word_augment"], 50)["k_word_augment"]
     nbytes = 2 * x.numel() * 4                              # one read and one write of every pixel, the least it can move
     res["augment_kernel"] = {"us_device": us, "pixels": x.numel(), "min_bytes": nbytes,
                              "GB_per_s_min_bytes": nbytes / (us * 1e-6) / 1e9 if us > 0 else None}

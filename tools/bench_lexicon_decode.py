@@ -8,7 +8,6 @@ import argparse
 import importlib
 import json
 import os
-import subprocess
 import sys
 
 ROOT = os.path.dirname(os.path.dirname(os.path.abspath(__file__)))
@@ -17,35 +16,12 @@ sys.path.insert(0, ROOT)
 import numpy as np  # noqa: E402
 import torch  # noqa: E402
 
-from torch.profiler import ProfilerActivity, profile  # noqa: E402
-
 _abi = importlib.import_module("scrabble-gan_b200._abi")
 runtime = importlib.import_module("scrabble-gan_b200.runtime")
 ops = importlib.import_module("scrabble-gan_b200.ops")
 na = importlib.import_module("scrabble-gan_b200.bigacgan.net_architecture")
 
-
-def card():
-    q = subprocess.run(["nvidia-smi", "--query-gpu=name,power.limit,clocks.max.sm", "--format=csv,noheader"], capture_output=True,
-                       text=True)
-    return q.stdout.strip().splitlines()[0] if q.returncode == 0 and q.stdout.strip() else torch.cuda.get_device_name(0)
-
-
-def device_us(fn, names, calls=20):
-    """Device time per call of each kernel in `names` (substring match) from torch.profiler, in a pass of its own after
-    a warm-up call."""
-    fn()
-    torch.cuda.synchronize()
-    with profile(activities=[ProfilerActivity.CUDA]) as prof:
-        for _ in range(calls):
-            fn()
-        torch.cuda.synchronize()
-    out = {n: 0.0 for n in names}
-    for e in prof.key_averages():
-        for n in names:
-            if n in e.key:
-                out[n] += getattr(e, "device_time_total", None) or getattr(e, "cuda_time_total", 0.0)
-    return {n: v / calls for n, v in out.items()}
+from _bench_util import card, device_us, r_forward_us  # noqa: E402
 
 
 def main():
@@ -66,18 +42,7 @@ def main():
     il = torch.full((b,), t, device=rt.device, dtype=torch.int32)
     ptr = _abi.ptr
 
-    fwd_all = 0.0
-    R._logits(rt, x, False)
-    torch.cuda.synchronize()
-    with profile(activities=[ProfilerActivity.CUDA]) as prof:
-        for _ in range(10):
-            R._logits(rt, x, False)
-        torch.cuda.synchronize()
-    for e in prof.key_averages():
-        tt = getattr(e, "device_time_total", None) or getattr(e, "cuda_time_total", 0.0)
-        if not e.key.startswith(("Memcpy", "Memset")) and tt > 0:
-            fwd_all += tt
-    res["R_forward_us_device"] = fwd_all / 10
+    res["R_forward_us_device"] = r_forward_us(R, rt, x)
 
     w = 100
     dec = torch.empty((1, b, t), device=rt.device, dtype=torch.int32)
